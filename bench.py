@@ -2,7 +2,8 @@
 """bench.py — AMG-PCG solve of 3D 7-point Poisson 256^3 (BASELINE.json configs[2]) on N B200s.
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
-    python bench.py --impl reference --gpus N --steps K ...   # the reference's own CPU path on the box's host cores
+    python bench.py --impl reference --gpus N --steps K ...   # the reference's own CPU path on the host cores
+    python bench.py --steps K --dump-outputs DIR              # also write the last step's outputs to DIR (see --help)
 
 One "step" = one complete AMG-preconditioned CG solve (HEM hierarchy as shipped, V(7,7) Jacobi, omega = 0.66667) of the
 16.8M-row system to a RELATIVE residual of 1e-8 (north_star; the reference's absolute 1e-8 is unreachable at this size,
@@ -89,6 +90,23 @@ class ClockSampler:
 
 def problem_rhs(n):
     return np.ones(n)
+
+
+# --dump-outputs: solution vectors longer than this are written at one fixed, seeded sample of rows (2^21 doubles = 16 MB
+# per vector), so that the outputs of two builds at 256^3 can be compared entry for entry in well under 64 MB
+DUMP_ROWS = 1 << 21
+
+
+def dump_outputs(path, vectors, residual_history):
+    """write each vector of `vectors` (all of one length n) at the rows listed in x_index.npy, plus the residual history,
+    as float64 <path>/<name>.npy"""
+    n = len(next(iter(vectors.values())))
+    idx = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "x_index.npy"), idx.astype(np.float64))
+    for name, v in vectors.items():
+        np.save(os.path.join(path, f"{name}.npy"), np.ascontiguousarray(v[idx], dtype=np.float64))
+    np.save(os.path.join(path, "residual_history.npy"), np.asarray(residual_history, dtype=np.float64))
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -236,6 +254,7 @@ def run_ours(args):
     ev[1].synchronize()
     launches = sp.launch_count()
     solve_s = ev[0].elapsed_time(ev[1]) * 1e-3 / args.steps
+    x_device = dx.download() if args.dump_outputs else None  # before the e2e leg and the kernel timings reuse dx
 
     # e2e: host buffers in, host buffer out, copies inside the timed region
     # (each step is timed by itself: writing the initial guess x0 = 0 into the caller's buffer between two steps is the
@@ -261,6 +280,8 @@ def run_ours(args):
     if args.dump_hist:  # residual history of the solve, for the pin against the reference's own history (tools/)
         json.dump({"grid": grid, "iterations": int(it), "tol": tol, "history": [float(v) for v in hist]},
                   open(args.dump_hist, "w"))
+    if args.dump_outputs:  # what the caller of each timed path receives from its last step
+        dump_outputs(args.dump_outputs, {"x": x_device, "x_e2e": x_final}, hist)
 
     # roofline of the dominant kernel (fused Jacobi sweep on the finest level), timed alone on the same stream: the
     # kernel the solve really runs, then the same matrix forced to plain CSR (the kernel north_star's ">= 70 % of HBM
@@ -345,9 +366,17 @@ def main():
     ap.add_argument("--gpu-rap", action="store_true",
                     help="N=1: the Galerkin products of the (untimed) host setup run on the device (same hierarchy, bit for bit)")
     ap.add_argument("--dump-hist", default=None, help="N=1: write the PCG residual history of the solve to this JSON file")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="N=1: after the timed steps write the solution x of the last device-timed solve (x.npy), of the "
+                         "last e2e solve (x_e2e.npy) and the residual history (residual_history.npy) as float64 .npy "
+                         f"files to DIR; above {DUMP_ROWS} rows x is sampled at the fixed rows of x_index.npy")
     ap.add_argument("--profile", action="store_true",
                     help="for ncu: honour --warmup/--max-iter literally, do not insist on convergence")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.gpus > 1 or args.impl != "ours"):
+        ap.error("--dump-outputs is implemented for this repository's path on one GPU")
     if args.grid != 256:  # the headline metric is quoted at 256^3; other grids are named for what they are
         global METRIC
         METRIC = f"amg_pcg_solve_seconds_poisson3d_{args.grid}"

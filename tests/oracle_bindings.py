@@ -332,6 +332,53 @@ class OracleAmg:
         return x, hist[: k + 1]
 
 
+class OracleOps:
+    """the restatement's per-level primitives on hierarchy H, called the way RefAmg's are (by level index)"""
+
+    def __init__(self, oracle, H):
+        self.o, self.L = oracle, H.levels
+
+    def spmv(self, k, x):
+        return self.o.spmv(self.L[k]["A"], x)
+
+    def jacobi(self, k, b, x, iteration):
+        return self.o.jacobi(self.L[k]["A"], self.L[k]["diag"], b, x, 0.66667, iteration)
+
+    def store_residual(self, k, b, x):
+        return self.o.store_residual(self.L[k]["A"], b, x)
+
+    def residual(self, k, b, x):
+        return self.o.residual(self.L[k]["A"], b, x)
+
+    def transfer_residual(self, k, r):
+        return self.o.transfer_residual(self.L[k]["P"], r)
+
+    def transfer_solution(self, k, xc, xf):
+        return self.o.transfer_solution(self.L[k]["P"], xc, xf)
+
+    def coarse_solve(self, b):
+        return self.o.lu_solve(self.L[-1]["A"], b)
+
+
+def primitive_outputs(H, ops):
+    """{"<level>/<op>": output} of every per-level primitive of `ops` (OracleOps or RefAmg) on hierarchy H, from seeded
+    random inputs, plus "coarse_solve"; the residual norm as a 1-element array"""
+    rng = np.random.default_rng(11)
+    out = {}
+    for k, L in enumerate(H.levels):
+        x, b = rng.random(L["A"].nrow), rng.random(L["A"].nrow)
+        out[f"{k}/spmv"] = ops.spmv(k, x)
+        out[f"{k}/jacobi"] = ops.jacobi(k, b, x, 6)
+        out[f"{k}/store_residual"] = ops.store_residual(k, b, x)
+        out[f"{k}/residual"] = np.array([ops.residual(k, b, x)])
+        if L["P"] is not None:
+            xc = rng.random(L["P"].ncol)
+            out[f"{k}/transfer_residual"] = ops.transfer_residual(k, x)
+            out[f"{k}/transfer_solution"] = ops.transfer_solution(k, xc, x)
+    out["coarse_solve"] = ops.coarse_solve(rng.random(H.levels[-1]["A"].nrow))
+    return out
+
+
 def have_ref():
     return os.path.exists(REF_SO)
 

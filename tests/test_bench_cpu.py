@@ -45,6 +45,38 @@ def test_reference_arm_non_zero_ranks_do_nothing():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+@pytest.mark.parametrize("extra", [["--steps", "0"], ["--gpus", "2", "--dump-outputs", "out"],
+                                   ["--impl", "reference", "--dump-outputs", "out"]])
+def test_unsupported_arguments_are_refused(tmp_path, extra):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True,
+                         timeout=120, cwd=tmp_path)
+    assert out.returncode == 2 and "error:" in out.stderr
+    assert not os.path.exists(tmp_path / "out")
+
+
+def test_dump_outputs_samples_long_vectors(tmp_path):
+    """above DUMP_ROWS rows every vector is written at the same seeded rows, listed in x_index.npy; 256^3 stays < 64 MB"""
+    import numpy as np
+
+    import bench
+
+    n = bench.DUMP_ROWS + 1000
+    x = np.arange(n, dtype=np.float64)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"x": x, "x_e2e": -x}, [2.0, 1.0])
+    got = {f: np.load(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")}
+    assert set(got) == {"x.npy", "x_e2e.npy", "x_index.npy", "residual_history.npy"}
+    assert all(v.dtype == np.float64 for v in got.values())
+    idx = got["x_index.npy"]
+    assert len(idx) == bench.DUMP_ROWS and np.all(np.diff(idx) > 0) and idx[-1] < n
+    np.testing.assert_array_equal(got["x.npy"], idx)
+    np.testing.assert_array_equal(got["x_e2e.npy"], -idx)
+    np.testing.assert_array_equal(got["residual_history.npy"], [2.0, 1.0])
+    for f, v in got.items():
+        np.testing.assert_array_equal(np.load(tmp_path / "b" / f), v)
+    assert 3 * 8 * bench.DUMP_ROWS <= 64 << 20
+
+
 def test_product_arm_needs_a_gpu():
     try:
         import torch
