@@ -107,13 +107,6 @@ int sparsh_pattern_encode(int nrow, int ncol, int nnz, const int *h_rowptr, cons
  * patterns (0: no twin), table entries, escape rows, fraction of the rows that carry pattern 0 */
 int sparsh_matrix_pattern_stats(sparsh_matrix_t A, int *n_pat, int *n_ent, int *n_escape, double *cover0);
 
-/* x windows of the TMA-staged csr-pattern8 kernel (host-only helper, so the tiling arithmetic can be checked without a
- * GPU): a tile of *tile consecutive rows gathers x only from *nwin contiguous ranges [r0 + lo[w], r0 + lo[w] + len[w]),
- * one per group of table offsets that lie within a tile length of each other; win[k] names the window of table entry k,
- * *w0 the window that holds offset 0 (-1: none).  lo/len need 8 slots.  *nwin == 0: the variant does not apply. */
-int sparsh_pattern_windows(int n_ent, const int *ent_off, int *tile, int *nwin, int *lo, int *len, int *w0,
-                           unsigned char *win);
-
 /* ------------------------------------------------------------------ setup ------ */
 /* Galerkin product A_c = P^T (A P) on the device (SURVEY 8f.1): what parallel::coarsen_matrix does with two
  * mkl_sparse_spmm calls on the host (src/AMG_cycle_utilities.cpp:126-146).  Row-wise products with the host setup's

@@ -64,7 +64,6 @@ SIGNATURES = {
     "sparsh_matrix_pattern_stats": (_i, [_vp, c_int_p, c_int_p, c_int_p, c_dbl_p]),
     "sparsh_pattern_encode": (_i, [_i, _i, _i, c_int_p, c_int_p, c_dbl_p, c_dbl_p, _vp, c_dbl_p, c_int_p, c_int_p, c_int_p,
                                    c_int_p]),
-    "sparsh_pattern_windows": (_i, [_i, c_int_p, c_int_p, c_int_p, c_int_p, c_int_p, c_int_p, _vp]),
     "sparsh_dict_encode": (_i, [_i, _i, _i, c_int_p, c_int_p, c_dbl_p, _vp, c_dbl_p, c_int_p, c_int_p, c_int_p]),
     "sparsh_galerkin_rap": (_i, [_i, c_int_p, c_int_p, c_dbl_p, _i, c_int_p, c_int_p, c_dbl_p, _vpp, c_int_p]),
     "sparsh_galerkin_rap_next": (_i, [_vp, _i, c_int_p, c_int_p, c_dbl_p, _vpp, c_int_p]),

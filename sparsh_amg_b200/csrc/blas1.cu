@@ -79,37 +79,31 @@ __device__ __forceinline__ void reduce_finalize(double (&v)[NV], double *partial
 
 // ---- element-wise ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(BT) fill_kernel(double *x, size_t n, double v) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     for (size_t i = (size_t)blockIdx.x * BT + threadIdx.x; i < n; i += (size_t)gridDim.x * BT) x[i] = v;
 }
 __global__ void __launch_bounds__(BT) axpy_kernel(size_t n, double a, const double *__restrict__ x, double *y) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     for (size_t i = (size_t)blockIdx.x * BT + threadIdx.x; i < n; i += (size_t)gridDim.x * BT)
         y[i] = __dadd_rn(y[i], __dmul_rn(a, x[i]));
 }
 __global__ void __launch_bounds__(BT) axpby_kernel(size_t n, double a, const double *__restrict__ x, double b, double *y) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     for (size_t i = (size_t)blockIdx.x * BT + threadIdx.x; i < n; i += (size_t)gridDim.x * BT)
         y[i] = __dadd_rn(__dmul_rn(a, x[i]), __dmul_rn(b, y[i]));
 }
 // daxpbyc of src/AMG_main_solvers.cu:26-33: c = alpha*x + beta*y + gamma*c
 __global__ void __launch_bounds__(BT)
     axpbypcz_kernel(size_t n, double a, const double *__restrict__ x, double b, const double *__restrict__ y, double c, double *z) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     for (size_t i = (size_t)blockIdx.x * BT + threadIdx.x; i < n; i += (size_t)gridDim.x * BT)
         z[i] = __dadd_rn(__dadd_rn(__dmul_rn(a, x[i]), __dmul_rn(b, y[i])), __dmul_rn(c, z[i]));
 }
 // first Jacobi sweep from a zero guess: A*0 = 0, h = b - 0, x = 0 + (omega*h)/d   (src/AMG_smoothers.cpp:62-71)
 __global__ void __launch_bounds__(BT)
     jacobi_zero_kernel(size_t n, const double *__restrict__ b, const double *__restrict__ d, double omega, double *x) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     for (size_t i = (size_t)blockIdx.x * BT + threadIdx.x; i < n; i += (size_t)gridDim.x * BT)
         x[i] = __ddiv_rn(__dmul_rn(omega, b[i]), d[i]);
 }
 
 __global__ void __launch_bounds__(BT)
     dot_kernel(size_t n, const double *__restrict__ x, const double *__restrict__ y, double *partials, unsigned int *ticket, double *out) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     double v[1] = {0.0};
     for (size_t i = (size_t)blockIdx.x * BT + threadIdx.x; i < n; i += (size_t)gridDim.x * BT)
         v[0] = __dadd_rn(v[0], __dmul_rn(x[i], y[i]));
@@ -118,7 +112,6 @@ __global__ void __launch_bounds__(BT)
 __global__ void __launch_bounds__(BT)
     dot2_kernel(size_t n, const double *__restrict__ a, const double *__restrict__ b, const double *__restrict__ c, double *partials,
                 unsigned int *ticket, double *out) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     double v[2] = {0.0, 0.0};
     for (size_t i = (size_t)blockIdx.x * BT + threadIdx.x; i < n; i += (size_t)gridDim.x * BT) {
         const double ai = a[i];
@@ -133,7 +126,6 @@ __global__ void __launch_bounds__(BT)
 __global__ void __launch_bounds__(BT)
     mdot4_kernel(size_t n, const double *__restrict__ V, size_t ld, int cnt, const double *__restrict__ w, double *partials,
                  unsigned int *ticket, double *out) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     double v[4] = {0.0, 0.0, 0.0, 0.0};
     for (size_t i = (size_t)blockIdx.x * BT + threadIdx.x; i < n; i += (size_t)gridDim.x * BT) {
         const double wi = w[i];
@@ -146,7 +138,6 @@ __global__ void __launch_bounds__(BT)
 // w -= sum_q h[q] V_q  (q ascending; h in device memory)
 __global__ void __launch_bounds__(BT)
     maxpy_sub_kernel(size_t n, const double *__restrict__ V, size_t ld, int k, const double *__restrict__ h, double *w) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     extern __shared__ double sh[];
     for (int q = threadIdx.x; q < k; q += BT) sh[q] = h[q];
     __syncthreads();
@@ -159,7 +150,6 @@ __global__ void __launch_bounds__(BT)
 // out = sum_q y[q] V_q  (q ascending, from 0.0)
 __global__ void __launch_bounds__(BT)
     lincomb_kernel(size_t n, const double *__restrict__ V, size_t ld, int k, const double *__restrict__ y, double *out) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     extern __shared__ double sh[];
     for (int q = threadIdx.x; q < k; q += BT) sh[q] = y[q];
     __syncthreads();
@@ -172,7 +162,6 @@ __global__ void __launch_bounds__(BT)
 // out = in / sqrt(*nrm2)
 __global__ void __launch_bounds__(BT)
     scale_inv_sqrt_kernel(size_t n, const double *__restrict__ in, const double *nrm2, double *out) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     const double d = sqrt(*nrm2);
     for (size_t i = (size_t)blockIdx.x * BT + threadIdx.x; i < n; i += (size_t)gridDim.x * BT) out[i] = __ddiv_rn(in[i], d);
 }
@@ -182,7 +171,6 @@ __global__ void __launch_bounds__(BT)
 __global__ void __launch_bounds__(BT)
     pcg_update_xr_kernel(size_t n, const double *__restrict__ p, const double *__restrict__ Ap, double *x, double *r,
                          const double *rz, const double *pAp, double *partials, unsigned int *ticket, double *rr_out) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     const double alpha = *rz / *pAp;
     const double nalpha = -alpha;
     double v[1] = {0.0};
@@ -197,13 +185,11 @@ __global__ void __launch_bounds__(BT)
 // beta = rz_new/rz_old (:149); p = 1.0*z + beta*p (:150)
 __global__ void __launch_bounds__(BT)
     pcg_update_p_kernel(size_t n, const double *__restrict__ z, double *p, const double *rz_new, const double *rz_old) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     const double beta = *rz_new / *rz_old;
     for (size_t i = (size_t)blockIdx.x * BT + threadIdx.x; i < n; i += (size_t)gridDim.x * BT)
         p[i] = __dadd_rn(z[i], __dmul_rn(beta, p[i]));
 }
 __global__ void scalar_copy_kernel(double *dst, const double *src) {
-    pdl_prologue();
     *dst = *src;
 }
 
@@ -211,7 +197,6 @@ __global__ void scalar_copy_kernel(double *dst, const double *src) {
 // s = r - alpha*Ap, alpha = alpha1/apr0 (:406-411)
 __global__ void __launch_bounds__(BT)
     bicg_s_kernel(size_t n, const double *__restrict__ r, const double *__restrict__ Ap, double *s, const double *alpha1, const double *apr0) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     const double alpha = *alpha1 / *apr0;
     for (size_t i = (size_t)blockIdx.x * BT + threadIdx.x; i < n; i += (size_t)gridDim.x * BT)
         s[i] = __dsub_rn(r[i], __dmul_rn(alpha, Ap[i]));
@@ -222,7 +207,6 @@ __global__ void __launch_bounds__(BT)
     bicg_xr_kernel(size_t n, double *x, const double *__restrict__ ph, const double *__restrict__ sh, const double *__restrict__ s,
                    const double *__restrict__ As, double *r, const double *alpha1, const double *apr0, const double *ass,
                    const double *asas, const double *__restrict__ r0, double *partials, unsigned int *ticket, double *out2) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     const double alpha = *alpha1 / *apr0;
     const double omega1 = *ass / *asas;
     double v[2] = {0.0, 0.0};
@@ -238,7 +222,6 @@ __global__ void __launch_bounds__(BT)
 // sc[0]=alpha1 sc[1]=apr0 sc[2]=ass sc[3]=asas sc[4]=r.r0(new):  beta = (sc4/sc0)*(alpha/omega1) (:428-429);
 // p = r + beta*(p - omega1*Ap) (:434)
 __global__ void __launch_bounds__(BT) bicg_p_kernel(size_t n, const double *__restrict__ r, double *p, const double *__restrict__ Ap, const double *sc) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     const double alpha = sc[0] / sc[1];
     const double omega1 = sc[2] / sc[3];
     double beta = sc[4] / sc[0];
@@ -249,7 +232,6 @@ __global__ void __launch_bounds__(BT) bicg_p_kernel(size_t n, const double *__re
 // CG (src/AMG_main_solvers.cpp:82-83): beta = rr_new/rr_old; p = 1.0*r + beta*p
 __global__ void __launch_bounds__(BT)
     cg_update_p_kernel(size_t n, const double *__restrict__ r, double *p, const double *rr_new, const double *rr_old) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     const double beta = *rr_new / *rr_old;
     for (size_t i = (size_t)blockIdx.x * BT + threadIdx.x; i < n; i += (size_t)gridDim.x * BT)
         p[i] = __dadd_rn(r[i], __dmul_rn(beta, p[i]));
@@ -265,91 +247,91 @@ __global__ void __launch_bounds__(BT)
 
 int k_fill(double *x, size_t n, double v) {
     if (n == 0) return SPARSH_OK;
-    SP_CUDA(launch_k(fill_kernel, dim3(stream_grid(n)), dim3(BT), 0, ctx().stream, x, n, v));
+    fill_kernel<<<stream_grid(n), BT, 0, ctx().stream>>>(x, n, v);
     LAUNCH_CHECK();
 }
 int k_axpy(size_t n, double a, const double *x, double *y) {
     if (n == 0) return SPARSH_OK;
-    SP_CUDA(launch_k(axpy_kernel, dim3(stream_grid(n)), dim3(BT), 0, ctx().stream, n, a, x, y));
+    axpy_kernel<<<stream_grid(n), BT, 0, ctx().stream>>>(n, a, x, y);
     LAUNCH_CHECK();
 }
 int k_axpby(size_t n, double a, const double *x, double b, double *y) {
     if (n == 0) return SPARSH_OK;
-    SP_CUDA(launch_k(axpby_kernel, dim3(stream_grid(n)), dim3(BT), 0, ctx().stream, n, a, x, b, y));
+    axpby_kernel<<<stream_grid(n), BT, 0, ctx().stream>>>(n, a, x, b, y);
     LAUNCH_CHECK();
 }
 int k_axpbypcz(size_t n, double a, const double *x, double b, const double *y, double c, double *z) {
     if (n == 0) return SPARSH_OK;
-    SP_CUDA(launch_k(axpbypcz_kernel, dim3(stream_grid(n)), dim3(BT), 0, ctx().stream, n, a, x, b, y, c, z));
+    axpbypcz_kernel<<<stream_grid(n), BT, 0, ctx().stream>>>(n, a, x, b, y, c, z);
     LAUNCH_CHECK();
 }
 int k_jacobi_zero(size_t n, const double *b, const double *d, double omega, double *x) {
     if (n == 0) return SPARSH_OK;
-    SP_CUDA(launch_k(jacobi_zero_kernel, dim3(stream_grid(n)), dim3(BT), 0, ctx().stream, n, b, d, omega, x));
+    jacobi_zero_kernel<<<stream_grid(n), BT, 0, ctx().stream>>>(n, b, d, omega, x);
     LAUNCH_CHECK();
 }
 int k_dot(size_t n, const double *x, const double *y, double *d_out) {
     Context &c = ctx();
-    SP_CUDA(launch_k(dot_kernel, dim3(stream_grid(n)), dim3(BT), 0, c.stream, n, x, y, c.partials, c.ticket, d_out));
+    dot_kernel<<<stream_grid(n), BT, 0, c.stream>>>(n, x, y, c.partials, c.ticket, d_out);
     LAUNCH_CHECK();
 }
 int k_dot2(size_t n, const double *a, const double *b, const double *cc, double *d_out2) {
     Context &c = ctx();
-    SP_CUDA(launch_k(dot2_kernel, dim3(stream_grid(n)), dim3(BT), 0, c.stream, n, a, b, cc, c.partials, c.ticket, d_out2));
+    dot2_kernel<<<stream_grid(n), BT, 0, c.stream>>>(n, a, b, cc, c.partials, c.ticket, d_out2);
     LAUNCH_CHECK();
 }
 int k_mdot(size_t n, const double *V, size_t ld, int k, const double *w, double *d_out) {
     Context &c = ctx();
     for (int j0 = 0; j0 < k; j0 += 4) {  // d_out must have room for k rounded up to a multiple of 4
-        SP_CUDA(launch_k(mdot4_kernel, dim3(stream_grid(n)), dim3(BT), 0, c.stream, n, V + (size_t)j0 * ld, ld, k - j0 < 4 ? k - j0 : 4, w, c.partials, c.ticket, d_out + j0));
+        mdot4_kernel<<<stream_grid(n), BT, 0, c.stream>>>(n, V + (size_t)j0 * ld, ld, k - j0 < 4 ? k - j0 : 4, w, c.partials, c.ticket, d_out + j0);
         count_launch();
         SP_CUDA(cudaGetLastError());
     }
     return SPARSH_OK;
 }
 int k_maxpy_sub(size_t n, const double *V, size_t ld, int k, const double *d_h, double *w) {
-    SP_CUDA(launch_k(maxpy_sub_kernel, dim3(stream_grid(n)), dim3(BT), sizeof(double) * (size_t)k, ctx().stream, n, V, ld, k, d_h, w));
+    maxpy_sub_kernel<<<stream_grid(n), BT, sizeof(double) * (size_t)k, ctx().stream>>>(n, V, ld, k, d_h, w);
     LAUNCH_CHECK();
 }
 int k_lincomb(size_t n, const double *V, size_t ld, int k, const double *d_y, double *out) {
-    SP_CUDA(launch_k(lincomb_kernel, dim3(stream_grid(n)), dim3(BT), sizeof(double) * (size_t)k, ctx().stream, n, V, ld, k, d_y, out));
+    lincomb_kernel<<<stream_grid(n), BT, sizeof(double) * (size_t)k, ctx().stream>>>(n, V, ld, k, d_y, out);
     LAUNCH_CHECK();
 }
 int k_scale_inv_sqrt(size_t n, const double *in, const double *d_nrm2, double *out) {
-    SP_CUDA(launch_k(scale_inv_sqrt_kernel, dim3(stream_grid(n)), dim3(BT), 0, ctx().stream, n, in, d_nrm2, out));
+    scale_inv_sqrt_kernel<<<stream_grid(n), BT, 0, ctx().stream>>>(n, in, d_nrm2, out);
     LAUNCH_CHECK();
 }
 int k_pcg_update_xr(size_t n, const double *p, const double *Ap, double *x, double *r, const double *rz,
                     const double *pAp, double *rr_out) {
     Context &c = ctx();
-    SP_CUDA(launch_k(pcg_update_xr_kernel, dim3(stream_grid(n)), dim3(BT), 0, c.stream, n, p, Ap, x, r, rz, pAp, c.partials, c.ticket, rr_out));
+    pcg_update_xr_kernel<<<stream_grid(n), BT, 0, c.stream>>>(n, p, Ap, x, r, rz, pAp, c.partials, c.ticket, rr_out);
     LAUNCH_CHECK();
 }
 int k_pcg_update_p(size_t n, const double *z, double *p, const double *rz_new, const double *rz_old) {
-    SP_CUDA(launch_k(pcg_update_p_kernel, dim3(stream_grid(n)), dim3(BT), 0, ctx().stream, n, z, p, rz_new, rz_old));
+    pcg_update_p_kernel<<<stream_grid(n), BT, 0, ctx().stream>>>(n, z, p, rz_new, rz_old);
     LAUNCH_CHECK();
 }
 int k_scalar_copy(double *dst, const double *src) {
-    SP_CUDA(launch_k(scalar_copy_kernel, dim3(1), dim3(1), 0, ctx().stream, dst, src));
+    scalar_copy_kernel<<<1, 1, 0, ctx().stream>>>(dst, src);
     LAUNCH_CHECK();
 }
 int k_cg_update_p(size_t n, const double *r, double *p, const double *rr_new, const double *rr_old) {
-    SP_CUDA(launch_k(cg_update_p_kernel, dim3(stream_grid(n)), dim3(BT), 0, ctx().stream, n, r, p, rr_new, rr_old));
+    cg_update_p_kernel<<<stream_grid(n), BT, 0, ctx().stream>>>(n, r, p, rr_new, rr_old);
     LAUNCH_CHECK();
 }
 int k_bicg_s(size_t n, const double *r, const double *Ap, double *s, const double *alpha1, const double *apr0) {
-    SP_CUDA(launch_k(bicg_s_kernel, dim3(stream_grid(n)), dim3(BT), 0, ctx().stream, n, r, Ap, s, alpha1, apr0));
+    bicg_s_kernel<<<stream_grid(n), BT, 0, ctx().stream>>>(n, r, Ap, s, alpha1, apr0);
     LAUNCH_CHECK();
 }
 int k_bicg_xr(size_t n, double *x, const double *ph, const double *sh, const double *s, const double *As, double *r,
               const double *alpha1, const double *apr0, const double *ass, const double *asas, const double *r0,
               double *out2) {
     Context &c = ctx();
-    SP_CUDA(launch_k(bicg_xr_kernel, dim3(stream_grid(n)), dim3(BT), 0, c.stream, n, x, ph, sh, s, As, r, alpha1, apr0, ass, asas, r0, c.partials, c.ticket, out2));
+    bicg_xr_kernel<<<stream_grid(n), BT, 0, c.stream>>>(n, x, ph, sh, s, As, r, alpha1, apr0, ass, asas, r0, c.partials, c.ticket, out2);
     LAUNCH_CHECK();
 }
 int k_bicg_p(size_t n, const double *r, double *p, const double *Ap, const double *sc) {
-    SP_CUDA(launch_k(bicg_p_kernel, dim3(stream_grid(n)), dim3(BT), 0, ctx().stream, n, r, p, Ap, sc));
+    bicg_p_kernel<<<stream_grid(n), BT, 0, ctx().stream>>>(n, r, p, Ap, sc);
     LAUNCH_CHECK();
 }
 

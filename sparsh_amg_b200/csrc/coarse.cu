@@ -133,7 +133,6 @@ __global__ void __launch_bounds__(256) gj_unscramble_kernel(double *M, int n, co
 
 // x = Ainv b: one warp per row, fixed lane-strided accumulation + shuffle tree (deterministic)
 __global__ void __launch_bounds__(256) dense_gemv_kernel(const double *__restrict__ Minv, int n, const double *__restrict__ b, double *x) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     const int row = blockIdx.x * 8 + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (row >= n) return;
@@ -231,7 +230,7 @@ int coarse_build_inverse(int n, const int *rp, const int *ci, const double *v, C
 
 int coarse_apply(const CoarseInverse &ci, const double *b, double *x) {
     if (ci.n == 0) return SPARSH_OK;
-    SP_CUDA(launch_k(dense_gemv_kernel, dim3((ci.n + 7) / 8), dim3(256), 0, ctx().stream, ci.inv, ci.n, b, x));
+    dense_gemv_kernel<<<(ci.n + 7) / 8, 256, 0, ctx().stream>>>(ci.inv, ci.n, b, x);
     count_launch();
     SP_CUDA(cudaGetLastError());
     return SPARSH_OK;

@@ -14,8 +14,9 @@
 //     when done (fused compute + communication over peer memory).  Sequence counters live in device memory, so all of
 //     it replays inside a CUDA graph: no NCCL call, host round trip or staging copy sits on the exchange path;
 //   * halo_mode 0: pack kernel -> grouped ncclSend/ncclRecv into the halo tail on a communication stream (fallback);
-//     Boundary strips run beside the interior rows (auxiliary high-priority stream; or, SPARSH_DIST_MERGE=1, as the first
-//     CTAs of one grid): they wait for the flags and signal as soon as the last of them is done; interior rows never wait;
+//     Boundary strips run beside the interior rows (auxiliary high-priority stream; the fused reductions, which need one
+//     grid, as its first CTAs): they wait for the flags and signal as soon as the last of them is done; interior rows
+//     never wait;
 //   * Krylov scalars: local fixed-tree partial, then a one-warp kernel stores it into a slot of every peer's arena,
 //     waits for the peers' slots and adds them in rank order (deterministic, graph-replayable; ~one NVLink round trip).
 //     The handshake error flag rides along, so every rank learns of a failure in the same iteration;
@@ -489,8 +490,8 @@ int nccl_finish() {
     return SPARSH_OK;
 }
 
-// the auxiliary stream carries the generic halo pushes (and, with SPARSH_DIST_MERGE=0 — kept for A/B measurements — the
-// boundary strips as a launch of their own beside the interior rows); joined by events
+// the auxiliary stream carries the generic halo pushes and the boundary strips as a launch of their own beside the
+// interior rows; joined by events
 struct StreamSwap {
     cudaStream_t saved;
     explicit StreamSwap(cudaStream_t s) : saved(ctx().stream) { ctx().stream = s; }
@@ -508,17 +509,13 @@ int join_aux() {
     SP_CUDA(cudaStreamWaitEvent(ctx().stream, m.ev_done, 0));
     return SPARSH_OK;
 }
-bool env_on(const char *name, bool dflt) {
-    const char *e = getenv(name);
-    return e ? atoi(e) != 0 : dflt;
-}
 
 // y = epi(op x).  The rows that touch the halo (and, for the fused Jacobi, the rows a neighbour needs) form the two
 // boundary strips, everything else is interior.  Peer mode: a generic push first if the halo of x is not already on
 // its way, then the strips — their CTAs wait for the flags, compute, optionally store the new values into the
 // neighbours and signal as soon as the last of them is done — beside the interior rows, which never wait: as two
-// launches on two streams (default) or as one grid whose first CTAs are the strips.  `push_output`: y is the next
-// input of this same operator.
+// launches on two streams, or, for the fused reductions (one grid over all rows), as one grid whose first CTAs are the
+// strips.  `push_output`: y is the next input of this same operator.
 int apply(sparsh_dist_s *h, const DistOp &op, int epi, double *x, double *y, EpiArgs args, bool push_output = false) {
     if (!op.needs_exchange()) return launch_csr(op.M, epi, x, y, args, 0, op.nrow);
     const bool reduces = epi == EPI_SPMV_DOT || epi == EPI_RESNORM;
@@ -561,13 +558,12 @@ int apply(sparsh_dist_s *h, const DistOp &op, int epi, double *x, double *y, Epi
         hs.seq = h->seq + op.id;
         h->halo_ready[by] = op.id + 1;
     }
-    // Default: boundary strips (with the push in front of them) on the high-priority auxiliary stream, interior rows as a
-    // launch of their own on the main stream.  Measured on B200, 256^3 (profiles/r02i_n2_*.json, r02j_*.json): 0.1009 s
-    // against 0.1058 s for the single launch at N=2, 0.0815 / 0.0827 at N=4, 0.0727 / 0.0723 at N=8 — the fork/join
-    // costs nothing measurable inside a CUDA graph, the extra launch is hidden behind the interior rows, and the
-    // neighbours hear from the strips earlier.  SPARSH_DIST_MERGE=1 selects the single launch.
-    static const bool merge = env_on("SPARSH_DIST_MERGE", false);
-    if (!merge && split && !reduces) {
+    // Boundary strips (with the push in front of them) on the high-priority auxiliary stream, interior rows as a launch
+    // of their own on the main stream.  Measured on B200, 256^3 (profiles/r02i_n2_*.json, r02j_*.json): 0.1009 s against
+    // 0.1058 s for strips and interior rows as one grid at N=2, 0.0815 / 0.0827 at N=4, 0.0727 / 0.0723 at N=8 — the
+    // fork/join costs nothing measurable inside a CUDA graph, the extra launch is hidden behind the interior rows, and
+    // the neighbours hear from the strips earlier.
+    if (split && !reduces) {
         EpiArgs iargs = args;  // interior rows: nothing to send
         iargs.pm_ptr = nullptr;
         SP_TRY(fork_aux());
@@ -579,9 +575,10 @@ int apply(sparsh_dist_s *h, const DistOp &op, int epi, double *x, double *y, Epi
         SP_TRY(launch_csr(op.M, epi, x, y, iargs, op.ib, op.ie));
         return join_aux();
     }
-    // one launch: the generic push (if any) first — a consumer grid whose strip CTAs fill the GPU while they wait must
-    // never be in front of the push that the neighbours' strips are waiting for (that is a cross-GPU deadlock: measured
-    // at 512^3, where a strip has more CTAs than the GPU holds) — then strips + interior rows as one grid
+    // one launch (fused reductions, unsplit operators): the generic push (if any) first — a consumer grid whose strip
+    // CTAs fill the GPU while they wait must never be in front of the push that the neighbours' strips are waiting for
+    // (that is a cross-GPU deadlock: measured at 512^3, where a strip has more CTAs than the GPU holds) — then strips +
+    // interior rows as one grid
     if (need_push) SP_TRY(peer_push(h, op, x));
     if (!split) return launch_csr3(op.M, epi, x, y, args, 0, op.nrow, 0, 0, 0, 0, &hs);
     return launch_csr3(op.M, epi, x, y, args, 0, op.ib, op.ie, op.nrow, op.ib, op.ie, &hs);
@@ -601,8 +598,7 @@ PeerTab peer_tab(const sparsh_dist_s *h) {
 int allreduce_sum(sparsh_dist_s *h, double *d_vals, int count) {
     Comm &m = comm();
     if (m.nranks == 1) return SPARSH_OK;
-    static const bool peer_coll = env_on("SPARSH_PEER_COLL", true);
-    if (h->peer && peer_coll) {
+    if (h->peer) {
         SP_REQUIRE(count >= 1 && count < RED_SLOTS, "peer all-reduce handles up to 3 scalars");
         peer_allreduce_kernel<<<1, 32, 0, ctx().stream>>>(d_vals, count, peer_tab(h), h->coll_off, h->red_seq, h->d_err, h->timeout_ns);
         count_launch();
@@ -662,8 +658,7 @@ int enqueue_dist_vcycle(sparsh_dist_s *h, const double *b, double *x, bool x_is_
     // replicated tail: every rank contributes its part of the restricted right-hand side to all copies of the vector,
     // the levels below are solved redundantly, the owned rows of the correction are kept
     const int gblocks = std::max(1, std::min((h->n_own_tail0 + 255) / 256, 4 * c.sm_count));
-    static const bool peer_coll = env_on("SPARSH_PEER_COLL", true);
-    if (m.nranks > 1 && h->peer && peer_coll) {
+    if (m.nranks > 1 && h->peer) {
         tail_exchange_kernel<<<gblocks, 256, 0, c.stream>>>(h->btail_local, h->d_tail_rows, h->n_own_tail0, peer_tab(h), h->tailb_off,
                                                             h->coll_off, h->tail_seq, h->tail_ticket, h->d_err, h->timeout_ns);
         count_launch();
@@ -679,7 +674,7 @@ int enqueue_dist_vcycle(sparsh_dist_s *h, const double *b, double *x, bool x_is_
         count_launch();
     }
     SP_TRY(enqueue_vcycle(h->tail, h->tail_b, h->tail_x, true));
-    if (m.nranks > 1 && h->peer && peer_coll) {
+    if (m.nranks > 1 && h->peer) {
         tail_gather_ack_kernel<<<gblocks, 256, 0, c.stream>>>(h->tail_x, h->d_tail_rows, h->n_own_tail0, h->xtail_local, peer_tab(h),
                                                               h->coll_off, h->tail_seq);
         count_launch();
@@ -723,14 +718,6 @@ int dist_run_graphed(sparsh_dist_s *h, const void *k0, const void *k1, int tag, 
         cudaError_t e = cudaStreamEndCapture(c.stream, &graph);
         if (rc == SPARSH_OK && e == cudaSuccess) e = cudaGraphInstantiate(&ent->exec, graph, 0);
         if (graph) cudaGraphDestroy(graph);
-        if ((rc != SPARSH_OK || e != cudaSuccess) && h->tail && h->tail->tail_state == 1) {
-            // the cooperative kernel of the replicated levels (tail.cu) is not capturable here: classical launches instead
-            cudaGetLastError();
-            ent->exec = nullptr;
-            tail_free(h->tail);
-            h->tail->tail_state = 2;
-            return dist_run_graphed(h, k0, k1, tag, body);
-        }
         if (rc != SPARSH_OK) return rc;
         SP_CUDA(e);
         ent->kernels = c.captured;

@@ -70,10 +70,7 @@ int enqueue_vcycle(sparsh_hierarchy_s *h, const double *b, double *x, bool x_is_
         T[l] = h->lev[l].tbuf;
         B[l] = l == 0 ? b : h->lev[l].bbuf;
     }
-    // the levels from `fused` down run as one cooperative kernel (tail.cu); -1: every level launches its own kernels
-    const int fused = tail_level(h);
-    const int bottom = fused >= 0 ? fused : L;
-    for (int l = 0; l < bottom; l++) {
+    for (int l = 0; l < L; l++) {
         Level &F = h->lev[l];
         SP_TRY(smooth(h, F, B[l], X[l], T[l], h->prm.pre_sweeps, l > 0 || x_is_zero));
         EpiArgs a;
@@ -85,13 +82,8 @@ int enqueue_vcycle(sparsh_hierarchy_s *h, const double *b, double *x, bool x_is_
         set_error("hierarchy without a coarse solver");
         return SPARSH_ERR_INVALID;
     }
-    if (fused >= 0) {
-        SP_TRY(enqueue_tail(h));
-        X[fused] = h->tail_x;
-    } else {
-        SP_TRY(coarse_apply(h->coarse, B[L], X[L]));
-    }
-    for (int l = bottom; l > 0; l--) {
+    SP_TRY(coarse_apply(h->coarse, B[L], X[L]));
+    for (int l = L; l > 0; l--) {
         Level &F = h->lev[l - 1];
         SP_TRY(launch_csr(F.P, EPI_PROLONG, X[l], X[l - 1], EpiArgs(), 0, F.n));
         SP_TRY(smooth(h, F, B[l - 1], X[l - 1], T[l - 1], h->prm.post_sweeps, false));
@@ -187,7 +179,7 @@ int sparsh_hierarchy_create(int nlevels, const sparsh_level_desc *levels, const 
             total += csr_bytes((size_t)d.nrow, (size_t)d.nnz) + 4 * (8 * ((size_t)d.nrow + 2) + 256);
             if (l < nlevels - 1) total += csr_bytes((size_t)d.nrow, (size_t)d.p_nnz) + csr_bytes((size_t)d.p_ncol, (size_t)d.p_nnz);
         }
-        h->slab = slab_create(total);  // nullptr (SPARSH_SLAB=0, or no room for one block): individual allocations
+        h->slab = slab_create(total);  // nullptr (no room for one block): individual allocations
     }
     auto run_task = [&](const Task &t) -> int {
         const sparsh_level_desc &d = levels[t.level];
@@ -281,7 +273,6 @@ int sparsh_hierarchy_destroy(sparsh_hierarchy_t h) {
         dev_free(L.rbuf);
     }
     coarse_free(&h->coarse);
-    tail_free(h);
     for (int i = 0; i < 8; i++) cudaFree(h->kv[i]);
     cudaFree(h->d_sc);
     cudaFreeHost(h->h_sc);

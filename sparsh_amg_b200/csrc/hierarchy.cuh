@@ -43,10 +43,6 @@ struct sparsh_hierarchy_s {
     double *gm_V = nullptr, *gm_d = nullptr, *gm_h = nullptr;
     int gm_m = 0;
     std::vector<sparsh::GraphEntry> graphs;
-    // the small levels of the cycle as one cooperative kernel (tail.cu): 0 undecided, 1 in use, 2 not applicable / refused
-    int tail_state = 0, tail_first = -1, tail_grid = 0, tail_nops = 0;
-    void *tail_prog = nullptr;   // device array of operations
-    double *tail_x = nullptr;    // where the correction of level tail_first ends up
 };
 
 namespace sparsh {
@@ -57,10 +53,6 @@ int enqueue_vcycle(sparsh_hierarchy_s *h, const double *b, double *x, bool x_is_
 template <class F>
 int run_graphed(sparsh_hierarchy_s *h, const void *k0, const void *k1, int tag, F body);
 int krylov_workspace(sparsh_hierarchy_s *h, int nvec);
-// tail.cu: first level of the bottom of the cycle that runs as one cooperative kernel (-1: none), its launch, its teardown
-int tail_level(sparsh_hierarchy_s *h);
-int enqueue_tail(sparsh_hierarchy_s *h);
-void tail_free(sparsh_hierarchy_s *h);
 
 template <class F>
 int run_graphed(sparsh_hierarchy_s *h, const void *k0, const void *k1, int tag, F body) {
@@ -89,15 +81,6 @@ int run_graphed(sparsh_hierarchy_s *h, const void *k0, const void *k1, int tag, 
         cudaError_t e = cudaStreamEndCapture(c.stream, &graph);
         if (rc == SPARSH_OK && e == cudaSuccess) e = cudaGraphInstantiate(&ent->exec, graph, 0);
         if (graph) cudaGraphDestroy(graph);
-        if ((rc != SPARSH_OK || e != cudaSuccess) && h->tail_state == 1) {
-            // a cooperative launch that this driver will not capture: give the fused tail up for this hierarchy and
-            // capture the classical launches instead
-            cudaGetLastError();
-            ent->exec = nullptr;
-            tail_free(h);
-            h->tail_state = 2;
-            return run_graphed(h, k0, k1, tag, body);
-        }
         if (rc != SPARSH_OK) return rc;
         SP_CUDA(e);
         ent->kernels = c.captured;

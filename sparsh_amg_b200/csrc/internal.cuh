@@ -43,45 +43,6 @@ struct NvtxRange {
     NvtxRange &operator=(const NvtxRange &) = delete;
 };
 
-// ---- programmatic dependent launch (PDL) ------------------------------------------------------------------------------
-// An iteration is ~250 dependent kernels, most of them a few microseconds long on the small levels.  Launched with the
-// programmatic-stream-serialisation attribute, kernel k+1 is scheduled as soon as every CTA of kernel k has passed its
-// griddepcontrol.launch_dependents (the first thing our kernels do after their own griddepcontrol.wait; SASS: ACQBULK /
-// PREEXIT) and then blocks in griddepcontrol.wait until kernel k has completed and its memory operations are visible.
-// A kernel launched WITHOUT the attribute passes the wait at once, and a predecessor that never triggers releases its
-// dependents when it exits, so mixing is safe; CUDA graphs capture the attribute as programmatic dependency edges.
-// MEASURED (B200, 256^3, profiles/r02n_*): no gain — 0.1442 s against 0.1446 s on one GPU, 0.0991 s against 0.0961 s on
-// two (inside a CUDA graph the node-to-node gap is already small, and a dependent grid that is resident while it waits
-// takes SM slots from the strips of the other stream).  Hence OFF by default; SPARSH_PDL=1 turns it on.
-__device__ __forceinline__ void pdl_prologue() {
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-}
-bool pdl_enabled();
-void pdl_disable();  // a launch with the attribute was refused (old driver): everything is launched classically from then on
-template <class... KArgs, class... Args>
-inline cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args &&...args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    if (pdl_enabled()) {
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-        const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-        if (e != cudaErrorNotSupported) return e;
-        cudaGetLastError();
-        pdl_disable();
-        cfg.attrs = nullptr;
-        cfg.numAttrs = 0;
-    }
-    return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-
 // ---- runtime context --------------------------------------------------------------------------------
 struct Context {
     bool ready = false;
@@ -144,19 +105,6 @@ struct PatView {
     int far_off;    // largest positive offset of the table (0: none): the only x line of a row that rows swept earlier
                     // have not pulled into L2 yet — prefetched while the pattern byte is still on its way
 };
-// x windows of the TMA-staged pattern kernel: a tile of PAT_TILE consecutive rows gathers x only from a few contiguous
-// index ranges [r0 + lo_w, r0 + lo_w + len_w) — one per group of table offsets that lie within a tile length of each
-// other — which one thread fetches with bulk copies.  win[k] tells which window serves table entry k.
-constexpr int PAT_TILE = 512;
-constexpr int PAT_MAX_WIN = 8;
-constexpr int PAT_WIN_DOUBLES = 3072;  // sum of the window lengths that still leaves >= 6 tiles resident per SM
-struct PatWindows {
-    int nwin;
-    int lo[PAT_MAX_WIN], len[PAT_MAX_WIN];  // len is even
-    int total;                              // sum of (len + 2): doubles of shared memory
-    int w0;                                 // window that contains offset 0 (-1: none)
-    const unsigned char *__restrict__ win;  // n_ent
-};
 // Pattern 0 (the most frequent row: patterns are numbered by decreasing row count) travels BY VALUE in the kernel
 // parameters, so the lean kernel reads its offsets and values as constant-bank operands: no shared-memory look-up, no
 // register, and — because the offsets do not depend on anything loaded — every gather of a row can be issued before
@@ -212,9 +160,7 @@ struct sparsh_matrix_s {
     double *pat_diag = nullptr;
     int n_pat = 0, n_pent = 0, n_escape = 0, pat_far = 0;
     bool has_pat = false;
-    sparsh::Pat0 pat0;                    // len == 0: the lean (speculative-gather) variant does not apply
-    sparsh::PatWindows pat_windows = {};  // nwin == 0: the TMA-staged variant does not apply
-    unsigned char *pat_win = nullptr;
+    sparsh::Pat0 pat0;  // len == 0: the lean (speculative-gather) variant does not apply
     sparsh::PatView pattern(bool use_pdiag) const {
         return sparsh::PatView{pat, pat_ent, pat_start, pat_diag, n_pat, n_pent, use_pdiag ? 1 : 0, pat_far};
     }

@@ -412,41 +412,6 @@ bool pattern_encode(int n, const int *rp, const int *ci, const double *v, const 
     return n > 0 && !T.diag.empty() && (double)covered >= min_cover * (double)n;
 }
 
-// x windows of the TMA-staged pattern kernel (PatWindows, internal.cuh): distinct table offsets, ascending, merged while
-// the gap to the previous one is at most a tile.  false when more than PAT_MAX_WIN windows or too much shared memory
-// would be needed (the LSU variant then runs).  Host only.
-bool pattern_windows(const std::vector<int> &off, PatWindows &W, std::vector<unsigned char> &win) {
-    std::vector<int> offs(off.begin(), off.end());
-    std::sort(offs.begin(), offs.end());
-    offs.erase(std::unique(offs.begin(), offs.end()), offs.end());
-    W = PatWindows();
-    W.w0 = -1;
-    if (offs.empty()) return false;
-    std::vector<int> hi;  // largest offset of each window
-    for (int o : offs) {
-        if (W.nwin > 0 && (long long)o - hi.back() <= PAT_TILE) {
-            hi.back() = o;
-        } else if (W.nwin == PAT_MAX_WIN) {
-            return false;
-        } else {
-            W.lo[W.nwin++] = o;
-            hi.push_back(o);
-        }
-    }
-    for (int w = 0; w < W.nwin; w++) {
-        const long long len = (long long)hi[w] - W.lo[w] + PAT_TILE;
-        W.len[w] = (int)((len + 1) & ~1LL);
-        W.total += W.len[w] + 2;
-        if (W.lo[w] <= 0 && hi[w] >= 0) W.w0 = w;
-    }
-    if (W.total > PAT_WIN_DOUBLES) return false;
-    win.assign(off.size() + 1, 0);
-    for (size_t k = 0; k < off.size(); k++)
-        for (int w = 0; w < W.nwin; w++)
-            if (off[k] >= W.lo[w] && off[k] <= hi[w]) win[k] = (unsigned char)w;
-    return true;
-}
-
 // ---- csr-pattern8 encoder on the device -----------------------------------------------------------------------
 // The host encoder above (kept as the CPU-checkable statement of the format, sparsh_pattern_encode) walks every row
 // with a hash map on one core: 0.5 s for 3D Poisson 256^3, a quarter of the whole upload.  The matrix is on the device
@@ -679,17 +644,6 @@ bool build_pattern(sparsh_matrix_s *A, const int *rp, const int *ci, const doubl
         }
         A->pat0 = z;
     }
-    {  // x windows for the TMA-staged variant
-        PatWindows W = {};
-        std::vector<unsigned char> win;
-        if (pattern_windows(T.off, W, win) && dev_alloc(&A->pat_win, win.size()) == cudaSuccess &&
-            cudaMemcpy(A->pat_win, win.data(), win.size(), cudaMemcpyHostToDevice) == cudaSuccess) {
-            W.win = A->pat_win;
-            A->pat_windows = W;
-        } else {
-            cudaGetLastError();
-        }
-    }
     A->has_pat = true;
     kept = true;
     cleanup();
@@ -815,23 +769,6 @@ int sparsh_pattern_encode(int nrow, int ncol, int nnz, const int *rp, const int 
     return SPARSH_OK;
 }
 
-int sparsh_pattern_windows(int n_ent, const int *ent_off, int *tile, int *nwin, int *lo, int *len, int *w0,
-                           unsigned char *win) {
-    SP_REQUIRE(n_ent >= 0 && ent_off && tile && nwin && lo && len && w0 && win, "bad arguments");
-    PatWindows W;
-    std::vector<unsigned char> wv;
-    *tile = PAT_TILE;
-    *nwin = 0;
-    *w0 = -1;
-    if (!pattern_windows(std::vector<int>(ent_off, ent_off + n_ent), W, wv)) return SPARSH_OK;
-    *nwin = W.nwin;
-    *w0 = W.w0;
-    std::copy(W.lo, W.lo + W.nwin, lo);
-    std::copy(W.len, W.len + W.nwin, len);
-    std::copy(wv.begin(), wv.begin() + n_ent, win);
-    return SPARSH_OK;
-}
-
 int sparsh_matrix_create_transpose(int nrow, int ncol, int nnz, const int *rp, const int *ci, const double *v,
                                    sparsh_matrix_t *out) {
     SP_TRY(ensure_init());
@@ -865,7 +802,6 @@ int sparsh_matrix_destroy(sparsh_matrix_t A) {
     dev_free(A->pat_ent);
     dev_free(A->pat_start);
     dev_free(A->pat_diag);
-    dev_free(A->pat_win);
     delete A;
     return SPARSH_OK;
 }

@@ -3,7 +3,6 @@
 #include <atomic>
 #include <cmath>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 #include <vector>
@@ -25,16 +24,6 @@ Context &ctx() {
     static Context c;
     return c;
 }
-
-static int g_pdl = -1;  // -1: not decided yet
-bool pdl_enabled() {
-    if (g_pdl < 0) {
-        const char *e = getenv("SPARSH_PDL");
-        g_pdl = e ? (atoi(e) != 0 ? 1 : 0) : 0;
-    }
-    return g_pdl == 1;
-}
-void pdl_disable() { g_pdl = 0; }
 
 int ensure_init() {
     if (ctx().ready) return SPARSH_OK;
@@ -61,8 +50,7 @@ thread_local size_t t_scratch_bytes = 0;
 }  // namespace
 
 DevSlab *slab_create(size_t bytes) {
-    static const bool off = getenv("SPARSH_SLAB") && atoi(getenv("SPARSH_SLAB")) == 0;
-    if (off || bytes == 0) return nullptr;
+    if (bytes == 0) return nullptr;
     DevSlab *s = new DevSlab();
     if (cudaMalloc(&s->base, bytes) != cudaSuccess) {
         cudaGetLastError();

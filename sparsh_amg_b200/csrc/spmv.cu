@@ -16,8 +16,6 @@
 //    csr-pattern8: 1 B per row), for matrices whose entries / rows repeat (stencils and their Galerkin coarsenings).
 //  * SCALAR (<= 2.5 nnz/row: aggregation P and R): thread per row straight from global memory (already coalesced).
 //  * VECTOR (irregular / long rows): 2..32 lanes per row, shuffle-tree reduction (1e-12 parity, not bit-exact).
-#include <cstdlib>
-
 #include "spmv_common.cuh"
 
 namespace sparsh {
@@ -25,7 +23,6 @@ namespace sparsh {
 // stage 2: a single CTA adds the partials in index order (65536 per-block atomics on one ticket cost ~60 us on a
 // 256^3 SpMV; this kernel costs ~4 us and keeps the result independent of block scheduling)
 __global__ void __launch_bounds__(1024) finalize_partials_kernel(const double *__restrict__ partials, int count, double *out) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     __shared__ double sred[32];
     double acc = 0.0;
     for (int i = threadIdx.x; i < count; i += 1024) acc += partials[i];
@@ -40,7 +37,6 @@ template <int THREADS, int EPI, bool DIST>
 __global__ void __launch_bounds__(THREADS)
     csr_stream_kernel(CsrView A, const double *x, double *y, EpiArgs args, RowRange rr, int cap, double *partials,
                       HaloSync hs) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     extern __shared__ __align__(128) unsigned char smem_raw[];
     double *sval = reinterpret_cast<double *>(smem_raw);
     int *scol = reinterpret_cast<int *>(smem_raw + (size_t)cap * sizeof(double));
@@ -117,7 +113,6 @@ template <int THREADS, int RPT, int EPI, bool DIST>
 __global__ void __launch_bounds__(THREADS)
     csr_dict_kernel(CsrView A, DictView D, const double *x, double *y, EpiArgs args, RowRange rr, int cap,
                     double *partials, HaloSync hs) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     // One CTA owns THREADS*RPT consecutive rows, thread t the rows r0 + s*THREADS + t (s < RPT).  With 2 B/nnz a
     // 256-row tile is only ~4 KB of matrix: a CTA must own several tiles' worth of rows, or the fixed cost of a CTA
     // (row pointer fetch -> bulk copy -> wait) caps the bytes in flight per SM below what saturates HBM.
@@ -220,7 +215,6 @@ template <int THREADS, int RPT, int JB, int EPI, bool DIST>
 __global__ void __launch_bounds__(THREADS)
     csr_pattern_kernel(CsrView A, PatView P, const double *x, double *y, EpiArgs args, RowRange rr, double *partials,
                        HaloSync hs) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     constexpr bool NEEDS_D = (EPI == EPI_JACOBI || EPI == EPI_SOR);
     extern __shared__ __align__(128) unsigned char smem_raw[];
     double *sval = reinterpret_cast<double *>(smem_raw);   // n_ent values
@@ -320,126 +314,11 @@ __global__ void __launch_bounds__(THREADS)
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// PATTERN kernel, TMA-staged variant (opt-in inside the opt-in: SPARSH_PATTERN_TMA=1).  Everything a tile of
-// PAT_TILE rows reads from DRAM — its pattern bytes, its slice of b and the few contiguous x windows its table offsets
-// reach (PatWindows) — is fetched by ONE thread with bulk copies (cp.async.bulk -> mbarrier) into shared memory; the
-// threads then walk their rows entirely out of shared memory.  No register holds a load in flight, so the bytes in
-// flight per SM are (resident tiles) x (tile bytes) instead of (threads) x (loads per thread), and the dependent
-// pattern-byte -> gather round trip of the LSU variant disappears.  Same entries, same order: bit-identical.
-// Preconditions (checked by the launcher, else the LSU variant runs): x and b 16-byte aligned, nrow and ncol even
-// (bulk copies move multiples of 16 bytes).
-// ---------------------------------------------------------------------------------------------------------
-template <int THREADS, int EPI>
-__global__ void __launch_bounds__(THREADS)
-    csr_pattern_tma_kernel(CsrView A, PatView P, PatWindows W, const double *x, double *y, EpiArgs args, RowRange rr,
-                           double *partials) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
-    constexpr int RPT = PAT_TILE / THREADS;
-    constexpr bool NEEDS_B = (EPI == EPI_RESID || EPI == EPI_JACOBI || EPI == EPI_SOR || EPI == EPI_RESNORM);
-    constexpr bool NEEDS_D = (EPI == EPI_JACOBI || EPI == EPI_SOR);
-    // shared memory: the three bulk-copy targets first (each starts on a 16-byte boundary), then the table
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    double *xw = reinterpret_cast<double *>(smem_raw);                            // W.total doubles (even)
-    double *sb = xw + W.total;                                                    // PAT_TILE + 2 doubles
-    unsigned char *spat = reinterpret_cast<unsigned char *>(sb + PAT_TILE + 2);   // PAT_TILE + 16 bytes
-    double *sval = reinterpret_cast<double *>(spat + PAT_TILE + 16);              // n_ent
-    double *sdiag = sval + P.n_ent;                                               // n_pat
-    int *sidx = reinterpret_cast<int *>(sdiag + P.n_pat);  // n_ent: (shift of the entry's window) + offset
-    int *sstart = sidx + P.n_ent;                          // n_pat + 1
-    __shared__ __align__(8) uint64_t bar;
-    __shared__ int s_shift[PAT_MAX_WIN];  // index into xw of global column c served by window w = s_shift[w] + c
-
-    const int tid = threadIdx.x;
-    int r0, row_end;
-    block_rows(rr, PAT_TILE, r0, row_end);
-    const int nrows = min(PAT_TILE, row_end - r0);
-    const int b0 = r0 & ~1, p0 = r0 & ~15;
-
-    if (tid < W.nwin) {
-        int base = 0;
-        for (int w = 0; w < tid; w++) base += W.len[w] + 2;
-        s_shift[tid] = base - (max(r0 + W.lo[tid], 0) & ~1);
-    }
-    if (tid == 0) {
-        mbar_init(&bar, 1);
-        fence_barrier_init();
-    }
-    __syncthreads();  // shifts and the initialised barrier visible to everyone
-    if (tid == 0) {
-        // sizes first (the barrier must know the byte count before any copy can complete), then the copies
-        int a0[PAT_MAX_WIN], cnt[PAT_MAX_WIN];
-        uint32_t bytes = 0;
-        for (int w = 0; w < W.nwin; w++) {
-            const int lo = max(r0 + W.lo[w], 0);
-            const int hi = min(r0 + W.lo[w] + W.len[w] - (PAT_TILE - nrows), A.ncol);
-            a0[w] = lo & ~1;
-            cnt[w] = max(((hi + 1) & ~1) - a0[w], 0);
-            bytes += (uint32_t)cnt[w] * 8u;
-        }
-        const int bcnt = NEEDS_B ? ((r0 + nrows + 1) & ~1) - b0 : 0;
-        const int pcnt = ((r0 + nrows + 15) & ~15) - p0;  // pat is padded by 16 bytes (matrix.cu)
-        bytes += (uint32_t)bcnt * 8u + (uint32_t)pcnt;
-        mbar_arrive_expect_tx(&bar, bytes);
-        int base = 0;
-        for (int w = 0; w < W.nwin; w++) {
-            if (cnt[w] > 0) bulk_g2s(xw + base, x + a0[w], (uint32_t)cnt[w] * 8u, &bar);
-            base += W.len[w] + 2;
-        }
-        if (bcnt > 0) bulk_g2s(sb, args.b + b0, (uint32_t)bcnt * 8u, &bar);
-        bulk_g2s(spat, P.pat + p0, (uint32_t)pcnt, &bar);
-    }
-    // the table, while the copies are in flight
-    for (int i = tid; i < P.n_ent; i += THREADS) {
-        const int4 q = __ldg(reinterpret_cast<const int4 *>(P.ent) + i);
-        sval[i] = __hiloint2double(q.y, q.x);
-        sidx[i] = s_shift[W.win[i]] + q.z;
-    }
-    for (int i = tid; i < P.n_pat; i += THREADS) sdiag[i] = __ldg(P.pdiag + i);
-    for (int i = tid; i <= P.n_pat; i += THREADS) sstart[i] = __ldg(P.start + i);
-    __syncthreads();  // table in place
-    mbar_wait(&bar, 0);
-
-    const bool xi_from_window = W.w0 >= 0 && args.xi == x;
-    const int xi_shift = W.w0 >= 0 ? s_shift[W.w0] : 0;
-    double contrib = 0.0;
-#pragma unroll
-    for (int s = 0; s < RPT; s++) {
-        const int local = s * THREADS + tid;
-        if (local < nrows) {
-            const int row = r0 + local;
-            const int pid = spat[row - p0];
-            EpiRegs e;
-            e.b = NEEDS_B ? sb[row - b0] : 0.0;
-            e.xi = 0.0;
-            e.d = 1.0;
-            if (EPI == EPI_JACOBI || EPI == EPI_SPMV_DOT) e.xi = xi_from_window ? xw[xi_shift + row] : args.xi[row];
-            if (EPI == EPI_PROLONG || EPI == EPI_SOR) e.xi = y[row];
-            double sum = 0.0;
-            if (pid != PAT_ESCAPE) {
-                const int st = sstart[pid], en = sstart[pid + 1];
-                for (int k = st; k < en; k++) sum = __dadd_rn(sum, __dmul_rn(sval[k], xw[sidx[k] + row]));
-                if (NEEDS_D) e.d = P.use_pdiag ? sdiag[pid] : args.d[row];
-            } else {
-                const int lo = A.rowptr[row], hi = A.rowptr[row + 1];
-#pragma unroll 1
-                for (int k = lo; k < hi; k++)
-                    sum = __dadd_rn(sum, __dmul_rn(__ldg(A.val + k),
-                                                   load_x<EpiTraits<EPI>::coherent_x>(x, __ldg(A.col + k))));
-                if (NEEDS_D) e.d = args.d[row];
-            }
-            contrib = __dadd_rn(contrib, epi_store<EPI, false>(args, e, sum, y, row));
-        }
-    }
-    if (EpiTraits<EPI>::reduces) block_partial<THREADS>(contrib, partials);
-}
-
-// ---------------------------------------------------------------------------------------------------------
 // SCALAR kernel: thread per row, rows of 1-2 entries (aggregation P / R): global loads are already coalesced
 // ---------------------------------------------------------------------------------------------------------
 template <int THREADS, int EPI, bool DIST>
 __global__ void __launch_bounds__(THREADS)
     csr_scalar_kernel(CsrView A, const double *x, double *y, EpiArgs args, RowRange rr, double *partials, HaloSync hs) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     int r0, row_end;
     block_rows(rr, THREADS, r0, row_end);
     const int row = r0 + threadIdx.x;
@@ -466,7 +345,6 @@ __global__ void __launch_bounds__(THREADS)
 template <int LANES, int EPI, bool DIST>
 __global__ void __launch_bounds__(256)
     csr_vector_kernel(CsrView A, const double *x, double *y, EpiArgs args, RowRange rr, double *partials, HaloSync hs) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
     constexpr int ROWS_PER_CTA = 256 / LANES;
     const int lane = threadIdx.x % LANES;
     int r0, row_end;
@@ -500,7 +378,7 @@ __global__ void __launch_bounds__(256)
 // ---------------------------------------------------------------------------------------------------------
 int launch_finalize_partials(int count, double *out) {
     Context &c = ctx();
-    SP_CUDA(launch_k(finalize_partials_kernel, dim3(1), dim3(1024), 0, c.stream, c.partials, count, out));
+    finalize_partials_kernel<<<1, 1024, 0, c.stream>>>(c.partials, count, out);
     count_launch();
     SP_CUDA(cudaGetLastError());
     return SPARSH_OK;
@@ -534,9 +412,9 @@ static int launch_stream(const sparsh_matrix_s *A, const double *x, double *y, c
         return SPARSH_ERR_INVALID;
     }
     if (d.dist)
-        SP_CUDA(launch_k(csr_stream_kernel<THREADS, EPI, true>, dim3(grid), dim3(THREADS), smem, c.stream, A->view(), x, y, args, d.rr, cap, c.partials, d.hs));
+        csr_stream_kernel<THREADS, EPI, true><<<grid, THREADS, smem, c.stream>>>(A->view(), x, y, args, d.rr, cap, c.partials, d.hs);
     else
-        SP_CUDA(launch_k(csr_stream_kernel<THREADS, EPI, false>, dim3(grid), dim3(THREADS), smem, c.stream, A->view(), x, y, args, d.rr, cap, c.partials, d.hs));
+        csr_stream_kernel<THREADS, EPI, false><<<grid, THREADS, smem, c.stream>>>(A->view(), x, y, args, d.rr, cap, c.partials, d.hs);
     return finish_launch<EPI>(grid, args);
 }
 
@@ -562,9 +440,9 @@ static int launch_dict_rpt(const sparsh_matrix_s *A, const double *x, double *y,
         return SPARSH_ERR_INVALID;
     }
     if (d.dist)
-        SP_CUDA(launch_k(csr_dict_kernel<THREADS, RPT, EPI, true>, dim3(grid), dim3(THREADS), smem, c.stream, A->view(), A->dict(), x, y, args, d.rr, cap, c.partials, d.hs));
+        csr_dict_kernel<THREADS, RPT, EPI, true><<<grid, THREADS, smem, c.stream>>>(A->view(), A->dict(), x, y, args, d.rr, cap, c.partials, d.hs);
     else
-        SP_CUDA(launch_k(csr_dict_kernel<THREADS, RPT, EPI, false>, dim3(grid), dim3(THREADS), smem, c.stream, A->view(), A->dict(), x, y, args, d.rr, cap, c.partials, d.hs));
+        csr_dict_kernel<THREADS, RPT, EPI, false><<<grid, THREADS, smem, c.stream>>>(A->view(), A->dict(), x, y, args, d.rr, cap, c.partials, d.hs);
     return finish_launch<EPI>(grid, args);
 }
 
@@ -587,53 +465,19 @@ static int launch_pattern_cfg(const sparsh_matrix_s *A, const double *x, double 
     // a kernel may use without opting in
     const size_t smem = (size_t)A->n_pent * 12 + (size_t)A->n_pat * 8 + (size_t)(A->n_pat + 1) * 4;
     if (d.dist)
-        SP_CUDA(launch_k(csr_pattern_kernel<THREADS, RPT, JB, EPI, true>, dim3(grid), dim3(THREADS), smem, c.stream, A->view(), P, x, y, args, d.rr, c.partials, d.hs));
+        csr_pattern_kernel<THREADS, RPT, JB, EPI, true><<<grid, THREADS, smem, c.stream>>>(A->view(), P, x, y, args, d.rr, c.partials, d.hs);
     else
-        SP_CUDA(launch_k(csr_pattern_kernel<THREADS, RPT, JB, EPI, false>, dim3(grid), dim3(THREADS), smem, c.stream, A->view(), P, x, y, args, d.rr, c.partials, d.hs));
-    return finish_launch<EPI>(grid, args);
-}
-
-static bool pattern_tma() {
-    static const bool v = [] {
-        const char *e = getenv("SPARSH_PATTERN_TMA");
-        return e && atoi(e) == 1;
-    }();
-    return v;
-}
-
-template <int EPI>
-static int launch_pattern_tma(const sparsh_matrix_s *A, const double *x, double *y, const EpiArgs &args, LaunchDesc d) {
-    Context &c = ctx();
-    constexpr int THREADS = 256;
-    static bool attr_set = false;
-    if (!attr_set) {
-        SP_CUDA(cudaFuncSetAttribute(csr_pattern_tma_kernel<THREADS, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-        attr_set = true;
-    }
-    const PatWindows &W = A->pat_windows;
-    const size_t smem = (size_t)(W.total + PAT_TILE + 2) * 8 + (PAT_TILE + 16) + (size_t)(A->n_pent + A->n_pat) * 8 +
-                        (size_t)(A->n_pent + A->n_pat + 1) * 4;
-    const int grid = grid_for(d, PAT_TILE);
-    if (grid > RED_MAX_BLOCKS) {
-        set_error("matrix too large for the reduction workspace");
-        return SPARSH_ERR_INVALID;
-    }
-    const PatView P = A->pattern(args.d != nullptr && args.d == A->diag);
-    SP_CUDA(launch_k(csr_pattern_tma_kernel<THREADS, EPI>, dim3(grid), dim3(THREADS), smem, c.stream, A->view(), P, W, x, y, args, d.rr, c.partials));
+        csr_pattern_kernel<THREADS, RPT, JB, EPI, false><<<grid, THREADS, smem, c.stream>>>(A->view(), P, x, y, args, d.rr, c.partials, d.hs);
     return finish_launch<EPI>(grid, args);
 }
 
 template <int THREADS, int EPI>
 static int launch_pattern(const sparsh_matrix_s *A, const double *x, double *y, const EpiArgs &args, const LaunchDesc &d) {
-    // TMA-staged variant: single GPU only, bulk copies need 16-byte aligned vectors and even extents
-    constexpr bool needs_b = (EPI == EPI_RESID || EPI == EPI_JACOBI || EPI == EPI_SOR || EPI == EPI_RESNORM);
-    if (pattern_tma() && !d.dist && A->pat_windows.nwin > 0 && (A->nrow & 1) == 0 && (A->ncol & 1) == 0 &&
-        ((uintptr_t)x & 15) == 0 && (!needs_b || ((uintptr_t)args.b & 15) == 0))
-        return launch_pattern_tma<EPI>(A, x, y, args, d);
     // lean variant (spmv_pattern.cu): one dominant pattern, gathers issued before the pattern byte is known
-    if (!pattern_tma() && pattern_lean_applies(A)) return launch_pattern_lean(A, EPI, x, y, args, d);
-    // first csr-pattern8 kernel (table in shared memory), 4 rows x 2 entries in flight per thread: the best of the
-    // shapes swept in round 2 (profiles/r02_pattern_sweep_256cubed.log); reached when the lean variant does not apply
+    if (pattern_lean_applies(A)) return launch_pattern_lean(A, EPI, x, y, args, d);
+    // every other csr-pattern8 matrix (pattern 0 not 5 or 7 entries long, or carried by fewer than half the rows): the
+    // table kernel, 4 rows x 2 entries in flight per thread, the best of the shapes swept in round 2
+    // (profiles/r02_pattern_sweep_256cubed.log)
     return launch_pattern_cfg<THREADS, 4, 2, EPI>(A, x, y, args, d);
 }
 
@@ -646,9 +490,9 @@ static int launch_scalar(const sparsh_matrix_s *A, const double *x, double *y, c
         return SPARSH_ERR_INVALID;
     }
     if (d.dist)
-        SP_CUDA(launch_k(csr_scalar_kernel<256, EPI, true>, dim3(grid), dim3(256), 0, c.stream, A->view(), x, y, args, d.rr, c.partials, d.hs));
+        csr_scalar_kernel<256, EPI, true><<<grid, 256, 0, c.stream>>>(A->view(), x, y, args, d.rr, c.partials, d.hs);
     else
-        SP_CUDA(launch_k(csr_scalar_kernel<256, EPI, false>, dim3(grid), dim3(256), 0, c.stream, A->view(), x, y, args, d.rr, c.partials, d.hs));
+        csr_scalar_kernel<256, EPI, false><<<grid, 256, 0, c.stream>>>(A->view(), x, y, args, d.rr, c.partials, d.hs);
     return finish_launch<EPI>(grid, args);
 }
 
@@ -661,9 +505,9 @@ static int launch_vector(const sparsh_matrix_s *A, const double *x, double *y, c
         return SPARSH_ERR_INVALID;
     }
     if (d.dist)
-        SP_CUDA(launch_k(csr_vector_kernel<LANES, EPI, true>, dim3(grid), dim3(256), 0, c.stream, A->view(), x, y, args, d.rr, c.partials, d.hs));
+        csr_vector_kernel<LANES, EPI, true><<<grid, 256, 0, c.stream>>>(A->view(), x, y, args, d.rr, c.partials, d.hs);
     else
-        SP_CUDA(launch_k(csr_vector_kernel<LANES, EPI, false>, dim3(grid), dim3(256), 0, c.stream, A->view(), x, y, args, d.rr, c.partials, d.hs));
+        csr_vector_kernel<LANES, EPI, false><<<grid, 256, 0, c.stream>>>(A->view(), x, y, args, d.rr, c.partials, d.hs);
     return finish_launch<EPI>(grid, args);
 }
 

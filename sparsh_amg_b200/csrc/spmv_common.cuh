@@ -217,11 +217,6 @@ struct EpiTraits {
     static constexpr bool coherent_x = (EPI == EPI_SOR);
 };
 
-template <bool COHERENT>
-__device__ __forceinline__ double load_x(const double *x, int c) {
-    if (COHERENT) return x[c];
-    return __ldg(x + c);
-}
 // multi-GPU kernels: halo entries are written by peers over NVLink while the grid may already be resident, so the
 // non-coherent path (ld.global.nc: data must be read-only for the kernel's lifetime) is off limits for the gathered
 // vector.  Plain loads are ordered behind the flag acquire + CTA barrier of halo_wait, and a stale L1 line cannot exist:

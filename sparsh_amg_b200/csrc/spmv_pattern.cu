@@ -1,7 +1,8 @@
 // spmv_pattern.cu — csr-pattern8, lean variant: the row-sum kernel for matrices whose rows almost all repeat ONE pattern
 // (the interior stencil row: 97.7 % of the rows of 3D Poisson 256^3 and of every level of its HEM hierarchy).
 //
-// What the first pattern kernel (spmv.cu: csr_pattern_kernel) pays for and this one does not:
+// The table kernel (spmv.cu: csr_pattern_kernel) serves every other csr-pattern8 matrix.  What it pays for and this one
+// does not:
 //  * two dependent memory round trips per tile (pattern byte -> table look-up -> gathers).  Pattern 0 travels BY VALUE
 //    in the kernel parameters (Pat0, internal.cuh), so its offsets are constant-bank operands known before anything is
 //    loaded: every thread issues the pattern byte, b, x_i AND all gathers of pattern 0 for all its rows at once —
@@ -12,9 +13,6 @@
 //    address computation, one LDG, one DMUL and one DADD whose second operands come from the constant bank;
 //  * the table copy into shared memory: done only by CTAs that meet a row with another pattern.
 // Same entries, same order, same unfused arithmetic as the CSR kernels: results are bit-identical.
-#include <algorithm>
-#include <cstdlib>
-
 #include "spmv_common.cuh"
 
 namespace sparsh {
@@ -27,31 +25,10 @@ __device__ __forceinline__ double gather(const double *x, int c, int ncol, int h
     return load_xd<COHERENT, DIST>(x, c, halo_begin);
 }
 
-__device__ __forceinline__ void prefetch_l2_line(const void *p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
-
-// rows [first, first + count) of virtual block `blk` (the mapping of block_rows for an arbitrary block index)
-__device__ __forceinline__ void virtual_block_rows(const RowRange &rr, int blk, int rows_per_cta, int &first, int &end) {
-    first = rr.b1;
-    end = rr.e1;
-    if (blk >= rr.nblk1) {
-        blk -= rr.nblk1;
-        first = rr.b2;
-        end = rr.e2;
-        if (blk >= rr.nblk2) {
-            blk -= rr.nblk2;
-            first = rr.b3;
-            end = rr.e3;
-        }
-    }
-    first += blk * rows_per_cta;
-}
-
 template <int THREADS, int RPT, int LEN0, int EPI, bool DIST>
 __global__ void __launch_bounds__(THREADS)
     csr_pat2_kernel(CsrView A, PatView P, const __grid_constant__ Pat0 Z, const double *x, double *y, EpiArgs args,
-                    RowRange rr, double *partials, HaloSync hs, int pf_dist) {
-    pdl_prologue();  // PDL: wait for the predecessor grid, then let the successor be scheduled
-    constexpr bool NEEDS_B = (EPI == EPI_RESID || EPI == EPI_JACOBI || EPI == EPI_SOR || EPI == EPI_RESNORM);
+                    RowRange rr, double *partials, HaloSync hs) {
     constexpr bool NEEDS_D = (EPI == EPI_JACOBI || EPI == EPI_SOR);
     constexpr bool COH = EpiTraits<EPI>::coherent_x;
     constexpr int TILE = THREADS * RPT;
@@ -60,27 +37,6 @@ __global__ void __launch_bounds__(THREADS)
     int r0, row_end;
     block_rows(rr, TILE, r0, row_end);
     const int nrows = min(TILE, row_end - r0);
-
-    // DRAM latency is paid by somebody else: this CTA asks L2 for the lines of the tile that the CTA taking its place
-    // on the SM will work on (pf_dist = co-resident CTAs of the grid), so that tile's own loads are L2 hits.  What is
-    // new to L2 per tile: its slice of b, of x (offset 0), of the pattern bytes, and the x lines at the largest offset
-    // of pattern 0 (the next grid plane; smaller offsets were gathered by earlier tiles).  One line per thread.
-    if (pf_dist > 0 && (int)blockIdx.x + pf_dist < (int)gridDim.x) {
-        int p0, pend;
-        virtual_block_rows(rr, blockIdx.x + pf_dist, TILE, p0, pend);
-        const int pn = min(TILE, pend - p0);
-        constexpr int LPT = TILE / 16;  // 128-byte lines of doubles per tile
-        if (pn > 0) {
-            const int part = tid / LPT, line = tid % LPT;  // THREADS >= 4 * LPT for RPT <= 4
-            const int i = p0 + line * 16;
-            if (i < p0 + pn) {
-                if (part == 0) prefetch_l2_line(x + i);
-                if (part == 1 && Z.hi > 0 && i + Z.hi < A.ncol) prefetch_l2_line(x + i + Z.hi);
-                if (part == 2 && NEEDS_B) prefetch_l2_line(args.b + i);
-                if (part == 3 && (line & 7) == 0) prefetch_l2_line(P.pat + i);
-            }
-        }
-    }
 
     HaloTurn hs_turn;
     if (DIST) hs_turn = halo_wait(hs);  // multi-GPU: the halo slices have landed before any (speculative) gather
@@ -158,18 +114,10 @@ int launch_cfg(const sparsh_matrix_s *A, const double *x, double *y, const EpiAr
         return SPARSH_ERR_INVALID;
     }
     const PatView P = A->pattern(args.d != nullptr && args.d == A->diag);
-    // successor-tile L2 prefetch: OFF by default.  Measured (profiles/r02g_pattern_lean_v3_sweep.log, ncu source page in
-    // profiles/r02m_*): it buys 1.5 % of the sweep while its index arithmetic is 28 of the 182 instructions a warp
-    // executes in a kernel that ncu shows issue-bound (76 % issue-active, DRAM 41 %).  SPARSH_PAT2_PF=<tiles> enables it
-    // (a sensible distance is the number of co-resident CTAs, sm_count x 8).
-    static const int pf = [] {
-        const char *e = getenv("SPARSH_PAT2_PF");
-        return e ? atoi(e) : 0;
-    }();
     if (d.dist)
-        SP_CUDA(launch_k(csr_pat2_kernel<THREADS, RPT, LEN0, EPI, true>, dim3(grid), dim3(THREADS), 0, c.stream, A->view(), P, A->pat0, x, y, args, d.rr, c.partials, d.hs, pf));
+        csr_pat2_kernel<THREADS, RPT, LEN0, EPI, true><<<grid, THREADS, 0, c.stream>>>(A->view(), P, A->pat0, x, y, args, d.rr, c.partials, d.hs);
     else
-        SP_CUDA(launch_k(csr_pat2_kernel<THREADS, RPT, LEN0, EPI, false>, dim3(grid), dim3(THREADS), 0, c.stream, A->view(), P, A->pat0, x, y, args, d.rr, c.partials, d.hs, pf));
+        csr_pat2_kernel<THREADS, RPT, LEN0, EPI, false><<<grid, THREADS, 0, c.stream>>>(A->view(), P, A->pat0, x, y, args, d.rr, c.partials, d.hs);
     count_launch();
     SP_CUDA(cudaGetLastError());
     if (EpiTraits<EPI>::reduces) return launch_finalize_partials(grid, args.red_out);
@@ -200,14 +148,10 @@ int launch_epi(const sparsh_matrix_s *A, const double *x, double *y, const EpiAr
 }  // namespace
 
 // stencils whose interior row has 5 or 7 entries (2D/3D Poisson-like operators and their semi-coarsened Galerkin
-// levels), as long as that row is the majority; SPARSH_PAT2=0 keeps the first pattern kernel (A/B measurements)
+// levels), as long as that row is the majority
 bool pattern_lean_applies(const sparsh_matrix_s *A) {
-    static const bool enabled = [] {
-        const char *e = getenv("SPARSH_PAT2");
-        return !(e && atoi(e) == 0);
-    }();
     const int len = A->pat0.len;
-    return enabled && A->has_pat && (len == 5 || len == 7) && A->pat0.cover >= 0.5;
+    return A->has_pat && (len == 5 || len == 7) && A->pat0.cover >= 0.5;
 }
 
 int launch_pattern_lean(const sparsh_matrix_s *A, int epi, const double *x, double *y, const EpiArgs &args, LaunchDesc d) {

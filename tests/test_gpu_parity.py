@@ -576,10 +576,9 @@ def test_graph_and_direct_launch_agree_bitwise(sp, oracle, fixture_system):
     np.testing.assert_array_equal(out[0][2], out[1][2])
 
 
-def test_fused_tail_kernel_is_bit_identical(sp, oracle, monkeypatch):
-    """the small levels of the cycle as ONE kernel (csrc/tail.cu: cooperative grid, or one 16-CTA cluster) against the same
-    levels launched kernel by kernel: V-cycle, AMG-PCG and BiCGStab leave the same bits behind (HEM and Beck hierarchies, graph and direct mode),
-    and both agree with the oracle"""
+def test_graph_and_direct_solves_agree_bitwise_on_hem_and_beck(sp, oracle):
+    """V-cycle, AMG-PCG and BiCGStab leave the same bits behind with and without CUDA graphs (HEM and Beck hierarchies),
+    and agree with the oracle"""
     A = oracle.gen_poisson3d(40, 36, 32)
     b = np.ones(A.nrow)
     xr = np.random.default_rng(9).standard_normal(A.nrow)
@@ -588,19 +587,17 @@ def test_fused_tail_kernel_is_bit_identical(sp, oracle, monkeypatch):
         levels = amg.hierarchy().levels
         assert len(levels) >= 4
         out = {}
-        for mode in ("0", "1", "2"):  # per-kernel launches, cooperative grid, 16-CTA cluster
-            monkeypatch.setenv("SPARSH_TAIL_MODE", mode)
-            for graph in (True, False):
-                dH = sp.DeviceHierarchy(levels, use_graph=graph)
-                db = sp.DeviceVector(data=b)
-                v = dH.vcycle(db, sp.DeviceVector(data=xr), 2).download()
-                dx = sp.DeviceVector(A.nrow).fill(0.0)
-                it, hist, ok = dH.pcg(db, dx, 1e-8)
-                dy = sp.DeviceVector(A.nrow).fill(0.0)
-                itb, histb, okb = dH.pbicgstab(db, dy, 1e-8)
-                assert ok and okb
-                out[(mode, graph)] = (v, it, hist, dx.download(), itb, histb, dy.download())
-        ref = out[("0", True)]
+        for graph in (True, False):
+            dH = sp.DeviceHierarchy(levels, use_graph=graph)
+            db = sp.DeviceVector(data=b)
+            v = dH.vcycle(db, sp.DeviceVector(data=xr), 2).download()
+            dx = sp.DeviceVector(A.nrow).fill(0.0)
+            it, hist, ok = dH.pcg(db, dx, 1e-8)
+            dy = sp.DeviceVector(A.nrow).fill(0.0)
+            itb, histb, okb = dH.pbicgstab(db, dy, 1e-8)
+            assert ok and okb
+            out[graph] = (v, it, hist, dx.download(), itb, histb, dy.download())
+        ref = out[True]
         for key, got in out.items():
             np.testing.assert_array_equal(got[0], ref[0])
             assert got[1] == ref[1] and got[4] == ref[4]
@@ -611,7 +608,6 @@ def test_fused_tail_kernel_is_bit_identical(sp, oracle, monkeypatch):
         _, want = amg.pcg(b, np.zeros(A.nrow), 1e-8)
         assert ref[1] == len(want) - 1
         assert_hist(ref[2], want)
-    monkeypatch.delenv("SPARSH_TAIL_MODE")
 
 
 def test_sweep_count_and_zero_guess_semantics(sp, oracle, fixture_system):

@@ -537,93 +537,3 @@ def test_fused_aggregation_product_equals_the_two_general_products(host, fixture
         for M in mats:
             M.free()
 
-
-def _emulate_tma_tile_arithmetic(M, enc, row_begin=0, row_end=None):
-    """Replays, in numpy, the index arithmetic of csr_pattern_tma_kernel (spmv.cu) for every tile: which x ranges the
-    bulk copies fetch, where they land in shared memory, and which shared-memory slot each (row, entry) reads.
-    Returns y = A x computed ONLY through those slots, plus the largest shared-memory footprint seen."""
-    import ctypes as C
-    import sparsh_amg_b200 as sp
-
-    pat, ent_val, ent_off, start, n_pat, _ = enc
-    n_ent = int(start[n_pat])
-    lib = sp.capi.load()
-    tile, nwin, w0 = C.c_int(), C.c_int(), C.c_int()
-    lo, ln = np.zeros(8, dtype=np.int32), np.zeros(8, dtype=np.int32)
-    win = np.zeros(max(n_ent, 1), dtype=np.uint8)
-    offs = np.ascontiguousarray(ent_off[:n_ent])
-    assert lib.sparsh_pattern_windows(n_ent, sp.capi.ip(offs), C.byref(tile), C.byref(nwin), sp.capi.ip(lo),
-                                      sp.capi.ip(ln), C.byref(w0), win.ctypes.data_as(C.c_void_p)) == 0
-    T, W = tile.value, nwin.value
-    if W == 0:
-        return None
-    assert all(l % 2 == 0 for l in ln[:W])
-    row_end = M.nrow if row_end is None else row_end
-    rng = np.random.default_rng(3)
-    x = rng.standard_normal(M.ncol)
-    y = np.zeros(M.nrow)
-    total = int(sum(ln[:W] + 2))
-    for r0 in range(row_begin, row_end, T):
-        nrows = min(T, row_end - r0)
-        xw = np.full(total, np.nan)  # shared memory; NaN = never written by a copy
-        shift, base = [], 0
-        for w in range(W):
-            lo_c = max(r0 + lo[w], 0)
-            hi_c = min(r0 + lo[w] + ln[w] - (T - nrows), M.ncol)
-            a0 = lo_c & ~1
-            cnt = max(((hi_c + 1) & ~1) - a0, 0)
-            assert cnt <= ln[w] + 2 and a0 % 2 == 0 and cnt % 2 == 0 and base % 2 == 0
-            assert cnt == 0 or (0 <= a0 and a0 + cnt <= M.ncol)  # a window wholly outside the vector copies nothing
-            xw[base: base + cnt] = x[a0: a0 + cnt]
-            shift.append(base - a0)
-            base += ln[w] + 2
-        for row in range(r0, r0 + nrows):
-            p = pat[row]
-            if p == 255:
-                s = 0.0
-                for j in range(M.rowptr[row], M.rowptr[row + 1]):
-                    s += M.val[j] * x[M.colindex[j]]
-            else:
-                s = 0.0
-                for k in range(start[p], start[p + 1]):
-                    s += ent_val[k] * xw[shift[win[k]] + ent_off[k] + row]
-            y[row] = s
-        if w0.value >= 0:  # the row's own entry, as the Jacobi epilogue reads it
-            rows = np.arange(r0, r0 + nrows)
-            np.testing.assert_array_equal(xw[shift[w0.value] + rows], x[rows])
-    return x, y, total
-
-
-@pytest.mark.parametrize("case", ["p3", "p2", "coarse", "range"])
-def test_tma_pattern_tile_arithmetic(host, case):
-    """csr_pattern_tma_kernel cannot run here, but its tiling arithmetic can: every (row, entry) must find its x value in
-    the shared-memory slot the kernel computes, for full tiles, the ragged last tile, clipped windows at both ends of
-    the vector, and row-range launches that do not start on a tile boundary."""
-    if case == "p2":
-        Mh = host.HostMatrix.poisson2d(70, 38)  # offsets +-70: one merged window
-    else:
-        Mh = host.HostMatrix.poisson3d(34, 18, 6)  # plane 612 > tile: three windows; 3672 rows = 7 tiles + ragged
-    host.set_options(coarse_upper=300, coarse_lower=100, max_levels=4, print_setup=0)
-    try:
-        amg = host.HostAmg(Mh)
-        L = amg.levels()[1 if case == "coarse" else 0]
-        M, diag = L["A"], np.ascontiguousarray(L["diag"])
-        if M.nrow % 2:
-            pytest.skip("odd extent: the launcher keeps the LSU variant")
-        enc = _pattern_encode(M, diag)
-        rb, re = (130, M.nrow - 77) if case == "range" else (0, None)
-        out = _emulate_tma_tile_arithmetic(M, enc, rb, re)
-        assert out is not None
-        x, y, total = out
-        want = M.to_scipy() @ x if hasattr(M, "to_scipy") else None
-        if want is None:
-            import scipy.sparse as sps
-
-            want = sps.csr_matrix((M.val, M.colindex, M.rowptr), shape=(M.nrow, M.ncol)) @ x
-        re = M.nrow if re is None else re
-        np.testing.assert_allclose(y[rb:re], want[rb:re], rtol=1e-13, atol=1e-13)  # no NaN: every slot was filled
-        assert total <= 3072
-        amg.free()
-    finally:
-        host.set_options(coarse_upper=4000, coarse_lower=2000, max_levels=6, print_setup=1)
-    Mh.free()

@@ -3,8 +3,8 @@
 Times the SpMV-family kernels and BLAS-1 on synthetic Poisson matrices with CUDA events on the library's stream and
 prints achieved algorithmic GB/s (SURVEY §8d byte model) per kernel family.  Usage:
     python tools/perf_probe.py [--n 256] [--dim 3] [--reps 20] [--families all|default]
-The csr-pattern8 kernels are probed when the twin exists (default; SPARSH_PAT2=0 selects the first kernel instead of the
-lean one).  The dict families need SPARSH_DICT=2 (the dict twin is not built where csr-pattern8 is selected).
+The csr-pattern8 kernels are probed when the twin exists (default: the lean kernel where it applies, the table kernel
+elsewhere).  The dict families need SPARSH_DICT=2 (the dict twin is not built where csr-pattern8 is selected).
 """
 import argparse
 import json
