@@ -107,6 +107,18 @@ int sparsh_pattern_encode(int nrow, int ncol, int nnz, const int *h_rowptr, cons
  * patterns (0: no twin), table entries, escape rows, fraction of the rows that carry pattern 0 */
 int sparsh_matrix_pattern_stats(sparsh_matrix_t A, int *n_pat, int *n_ent, int *n_escape, double *cover0);
 
+/* The row-sum kernel for matrices that mostly repeat pattern 0 (csr_pat2_kernel) evaluates a row of another pattern as
+ * pattern 0 with terms left out when that pattern's (offset, value bits) list is an in-order subsequence of pattern
+ * 0's and its diagonal (first offset-0 entry, else 0) has pattern 0's bits: the Dirichlet boundary rows of a stencil
+ * and their Galerkin coarsenings.  Host-only helper (needs no GPU) over a table as sparsh_pattern_encode returns it:
+ * mask[256] receives, per pattern id, 0x80 | (bit k set when the pattern has entry k of pattern 0), or 0 when the
+ * pattern is not such a subsequence.  Pattern 0 has every bit set when it has at most 7 entries; otherwise, and for
+ * ids >= n_pat, every mask is 0. */
+int sparsh_pattern_masks(int n_pat, const int *start, const double *ent_val, const int *ent_off, unsigned char *mask);
+/* what the upload built: patterns other than pattern 0 that run as masked pattern 0, and the fraction of the rows that
+ * carry pattern 0 or one of those patterns */
+int sparsh_matrix_pattern_mask_stats(sparsh_matrix_t A, int *n_masked, double *cover_masked);
+
 /* ------------------------------------------------------------------ setup ------ */
 /* Galerkin product A_c = P^T (A P) on the device (SURVEY 8f.1): what parallel::coarsen_matrix does with two
  * mkl_sparse_spmm calls on the host (src/AMG_cycle_utilities.cpp:126-146).  Row-wise products with the host setup's

@@ -62,6 +62,8 @@ SIGNATURES = {
     "sparsh_matrix_force_kernel": (_i, [_vp, _i, _i]),
     "sparsh_matrix_kernel_name": (_i, [_vp, _i, C.c_char_p, _sz]),
     "sparsh_matrix_pattern_stats": (_i, [_vp, c_int_p, c_int_p, c_int_p, c_dbl_p]),
+    "sparsh_matrix_pattern_mask_stats": (_i, [_vp, c_int_p, c_dbl_p]),
+    "sparsh_pattern_masks": (_i, [_i, c_int_p, c_dbl_p, c_int_p, _vp]),
     "sparsh_pattern_encode": (_i, [_i, _i, _i, c_int_p, c_int_p, c_dbl_p, c_dbl_p, _vp, c_dbl_p, c_int_p, c_int_p, c_int_p,
                                    c_int_p]),
     "sparsh_dict_encode": (_i, [_i, _i, _i, c_int_p, c_int_p, c_dbl_p, _vp, c_dbl_p, c_int_p, c_int_p, c_int_p]),

@@ -110,14 +110,22 @@ struct PatView {
 // register, and — because the offsets do not depend on anything loaded — every gather of a row can be issued before
 // the row's pattern byte has arrived (csr_pat2_kernel in spmv.cu).
 constexpr int PAT0_MAX = 32;
+// mask[p] (pattern_masks in matrix.cu): PAT_MASK_VALID set when the row of pattern p is pattern 0's row with some terms
+// left out — its (offset, value bits) list is an in-order subsequence of pattern 0's and its tabulated diagonal has
+// pattern 0's bits (the Dirichlet boundary rows of a stencil and their Galerkin coarsenings).  Bit k (< PAT_MASK_BITS)
+// then says whether the row has entry k of pattern 0.  Pattern 0 itself has every bit; the escape id has none.
+constexpr int PAT_MASK_BITS = 7;
+constexpr unsigned PAT_MASK_VALID = 0x80u;
 struct Pat0 {
     int len = 0;      // entries of pattern 0 (0: the lean kernel does not apply)
     int kdiag = -1;   // index of its offset-0 entry (-1: none)
     int lo = 0, hi = 0;  // smallest / largest offset
     double diag = 0.0;   // the tabulated diagonal (pdiag[0])
     double cover = 0.0;  // fraction of the rows that carry pattern 0
+    double cover_masked = 0.0;  // fraction of the rows that carry pattern 0 or a pattern with a valid mask
     int off[PAT0_MAX] = {};
     double val[PAT0_MAX] = {};
+    unsigned char mask[256] = {};  // per pattern id, see PAT_MASK_VALID
 };
 constexpr int PAT_ESCAPE = 255;    // pattern id of an escape row
 constexpr int PAT_MAX_ENT = 2048;  // table entries over all patterns (32 KB)

@@ -412,6 +412,30 @@ bool pattern_encode(int n, const int *rp, const int *ci, const double *v, const 
     return n > 0 && !T.diag.empty() && (double)covered >= min_cover * (double)n;
 }
 
+// The lean kernel's masks (Pat0::mask in internal.cuh).  A pattern whose (offset, value bits) list is an in-order
+// subsequence of pattern 0's, with pattern 0's diagonal, is evaluated as pattern 0 with the missing terms skipped: the
+// same products added in the same order, so the same bits as the table walk and the CSR kernels.  Greedy leftmost
+// matching decides the subsequence; where pattern 0 repeats an (offset, value) pair, any match adds the same terms.
+void pattern_masks(const PatternTable &T, unsigned char mask[256]) {
+    std::fill(mask, mask + 256, (unsigned char)0);
+    const int n_pat = std::min((int)T.diag.size(), PAT_ESCAPE);
+    if (n_pat == 0) return;
+    const int len0 = T.start[1] - T.start[0];
+    if (len0 > PAT_MASK_BITS) return;
+    for (int p = 0; p < n_pat; p++) {
+        if (!same_bits(T.diag[p], T.diag[0])) continue;
+        unsigned m = 0;
+        int k = 0;
+        bool sub = true;
+        for (int j = T.start[p]; sub && j < T.start[p + 1]; j++) {
+            while (k < len0 && !(T.off[k] == T.off[j] && same_bits(T.val[k], T.val[j]))) k++;
+            sub = k < len0;
+            if (sub) m |= 1u << k++;
+        }
+        if (sub) mask[p] = (unsigned char)(PAT_MASK_VALID | m);
+    }
+}
+
 // ---- csr-pattern8 encoder on the device -----------------------------------------------------------------------
 // The host encoder above (kept as the CPU-checkable statement of the format, sparsh_pattern_encode) walks every row
 // with a hash map on one core: 0.5 s for 3D Poisson 256^3, a quarter of the whole upload.  The matrix is on the device
@@ -477,12 +501,12 @@ __global__ void __launch_bounds__(256)
 
 // pat[i] = id of row i's pattern if the row equals the tabulated pattern entry by entry (and, when `diag` is given, its
 // smoothing diagonal equals the tabulated one bit for bit), PAT_ESCAPE otherwise; counts[0] += covered rows, counts[1] += rows
-// of pattern 0
+// of pattern 0, counts[2] += rows of pattern 0 or of a pattern with a valid mask in Z
 __global__ void __launch_bounds__(256)
     pat_assign_kernel(int n, const int *__restrict__ rp, const int *__restrict__ ci, const double *__restrict__ v,
                       const double *__restrict__ diag, const int *__restrict__ slot_of, const int *__restrict__ id_of_slot,
                       const PatEntry *__restrict__ ent, const int *__restrict__ start, const double *__restrict__ pdiag,
-                      unsigned char *pat, unsigned long long *counts) {
+                      const __grid_constant__ Pat0 Z, unsigned char *pat, unsigned long long *counts) {
     const int row = blockIdx.x * 256 + threadIdx.x;
     int id = -1;
     if (row < n) {
@@ -499,9 +523,11 @@ __global__ void __launch_bounds__(256)
         pat[row] = (unsigned char)(id >= 0 ? id : PAT_ESCAPE);
     }
     const unsigned int covered = __ballot_sync(0xffffffffu, id >= 0), zero = __ballot_sync(0xffffffffu, id == 0);
+    const unsigned int masked = __ballot_sync(0xffffffffu, id == 0 || (id > 0 && (Z.mask[id] & PAT_MASK_VALID)));
     if ((threadIdx.x & 31) == 0) {
         if (covered) atomicAdd(&counts[0], (unsigned long long)__popc(covered));
         if (zero) atomicAdd(&counts[1], (unsigned long long)__popc(zero));
+        if (masked) atomicAdd(&counts[2], (unsigned long long)__popc(masked));
     }
 }
 
@@ -548,7 +574,7 @@ bool build_pattern(sparsh_matrix_s *A, const int *rp, const int *ci, const doubl
     std::vector<PatSlot> table(PAT_SLOTS, PatSlot{0ull, 0x7fffffff, 0});
     cudaMemcpyAsync(d_table, table.data(), sizeof(PatSlot) * PAT_SLOTS, cudaMemcpyHostToDevice, st);
     cudaMemsetAsync(d_overflow, 0, sizeof(int) * 2, st);
-    cudaMemsetAsync(d_counts, 0, sizeof(unsigned long long) * 2, st);
+    cudaMemsetAsync(d_counts, 0, sizeof(unsigned long long) * 3, st);
     const int grid = (n + 255) / 256;
     pat_hash_kernel<<<grid, 256, 0, st>>>(n, A->rowptr, A->col, A->val, d_table, d_slot_of, d_overflow);
     int overflow = 0;
@@ -601,10 +627,25 @@ bool build_pattern(sparsh_matrix_s *A, const int *rp, const int *ci, const doubl
     }
     std::vector<PatEntry> ent((size_t)n_ent + 8, PatEntry{0.0, 0, 0});
     for (int k = 0; k < n_ent; k++) ent[k] = PatEntry{T.val[k], T.off[k], 0};
+    Pat0 z;  // pattern 0 by value for the lean kernel (spmv_pattern.cu: csr_pat2_kernel)
+    const int len0 = T.start[1] - T.start[0];
+    if (len0 >= 1 && len0 <= PAT0_MAX) {
+        z.len = len0;
+        z.diag = T.diag[0];
+        z.lo = z.hi = T.off[0];
+        for (int k = 0; k < len0; k++) {
+            z.off[k] = T.off[k];
+            z.val[k] = T.val[k];
+            z.lo = std::min(z.lo, T.off[k]);
+            z.hi = std::max(z.hi, T.off[k]);
+            if (T.off[k] == 0 && z.kdiag < 0) z.kdiag = k;
+        }
+        pattern_masks(T, z.mask);
+    }
     ok = dev_alloc(&A->pat, (size_t)n + 16) == cudaSuccess && dev_alloc(&A->pat_ent, sizeof(PatEntry) * ent.size()) == cudaSuccess &&
          dev_alloc(&A->pat_start, sizeof(int) * ((size_t)n_pat + 1)) == cudaSuccess &&
          dev_alloc(&A->pat_diag, sizeof(double) * (size_t)n_pat) == cudaSuccess;
-    unsigned long long counts[2] = {0ull, 0ull};
+    unsigned long long counts[3] = {0ull, 0ull, 0ull};
     if (ok) {
         cudaMemsetAsync(A->pat, PAT_ESCAPE, (size_t)n + 16, st);
         cudaMemcpyAsync(A->pat_ent, ent.data(), sizeof(PatEntry) * ent.size(), cudaMemcpyHostToDevice, st);
@@ -613,7 +654,7 @@ bool build_pattern(sparsh_matrix_s *A, const int *rp, const int *ci, const doubl
         cudaMemcpyAsync(d_id_of, id_of.data(), sizeof(int) * PAT_SLOTS, cudaMemcpyHostToDevice, st);
         // rows whose smoothing diagonal (A->diag, uploaded from h_diag) differs from the tabulated one become escapes
         pat_assign_kernel<<<grid, 256, 0, st>>>(n, A->rowptr, A->col, A->val, h_diag ? A->diag : nullptr, d_slot_of, d_id_of, A->pat_ent,
-                                                A->pat_start, A->pat_diag, A->pat, d_counts);
+                                                A->pat_start, A->pat_diag, z, A->pat, d_counts);
         cudaMemcpyAsync(counts, d_counts, sizeof counts, cudaMemcpyDeviceToHost, st);
         ok = cudaStreamSynchronize(st) == cudaSuccess;
     }
@@ -626,24 +667,11 @@ bool build_pattern(sparsh_matrix_s *A, const int *rp, const int *ci, const doubl
     A->n_escape = n - (int)counts[0];
     A->pat_far = 0;
     for (int k = 0; k < n_ent; k++) A->pat_far = std::max(A->pat_far, T.off[k]);
-    {  // pattern 0 by value for the lean kernel (spmv.cu: csr_pat2_kernel)
-        Pat0 z;
-        const int len0 = T.start[1] - T.start[0];
-        if (len0 >= 1 && len0 <= PAT0_MAX) {
-            z.len = len0;
-            z.diag = T.diag[0];
-            z.cover = (double)counts[1] / (double)n;
-            z.lo = z.hi = T.off[0];
-            for (int k = 0; k < len0; k++) {
-                z.off[k] = T.off[k];
-                z.val[k] = T.val[k];
-                z.lo = std::min(z.lo, T.off[k]);
-                z.hi = std::max(z.hi, T.off[k]);
-                if (T.off[k] == 0 && z.kdiag < 0) z.kdiag = k;
-            }
-        }
-        A->pat0 = z;
+    if (z.len > 0) {
+        z.cover = (double)counts[1] / (double)n;
+        z.cover_masked = (double)counts[2] / (double)n;
     }
+    A->pat0 = z;
     A->has_pat = true;
     kept = true;
     cleanup();
@@ -769,6 +797,31 @@ int sparsh_pattern_encode(int nrow, int ncol, int nnz, const int *rp, const int 
     return SPARSH_OK;
 }
 
+int sparsh_pattern_masks(int n_pat, const int *start, const double *ent_val, const int *ent_off, unsigned char *mask) {
+    SP_REQUIRE(start && ent_val && ent_off && mask, "pointer is NULL");
+    SP_REQUIRE(n_pat >= 0 && n_pat <= PAT_ESCAPE, "n_pat out of range");  // ids 0..254; 255 is the escape
+    SP_REQUIRE(n_pat == 0 || start[0] == 0, "start[0] != 0");
+    for (int p = 0; p < n_pat; p++) SP_REQUIRE(start[p] <= start[p + 1], "start not monotone");
+    SP_REQUIRE(n_pat == 0 || start[n_pat] <= PAT_MAX_ENT, "more table entries than a pattern table holds");
+    PatternTable T;
+    if (n_pat > 0) {
+        T.start.assign(start, start + n_pat + 1);
+        T.val.assign(ent_val, ent_val + start[n_pat]);
+        T.off.assign(ent_off, ent_off + start[n_pat]);
+    }
+    for (int p = 0; p < n_pat; p++) {  // the tabulated diagonal: the pattern's first offset-0 entry, else 0
+        double d = 0.0;
+        for (int k = start[p]; k < start[p + 1]; k++)
+            if (ent_off[k] == 0) {
+                d = ent_val[k];
+                break;
+            }
+        T.diag.push_back(d);
+    }
+    pattern_masks(T, mask);
+    return SPARSH_OK;
+}
+
 int sparsh_matrix_create_transpose(int nrow, int ncol, int nnz, const int *rp, const int *ci, const double *v,
                                    sparsh_matrix_t *out) {
     SP_TRY(ensure_init());
@@ -831,6 +884,16 @@ int sparsh_matrix_pattern_stats(sparsh_matrix_t A, int *n_pat, int *n_ent, int *
     if (n_ent) *n_ent = A->has_pat ? A->n_pent : 0;
     if (n_escape) *n_escape = A->has_pat ? A->n_escape : A->nrow;
     if (cover0) *cover0 = A->has_pat ? A->pat0.cover : 0.0;
+    return SPARSH_OK;
+}
+
+int sparsh_matrix_pattern_mask_stats(sparsh_matrix_t A, int *n_masked, double *cover_masked) {
+    SP_REQUIRE(A != nullptr, "matrix is NULL");
+    int m = 0;
+    if (A->has_pat)
+        for (int p = 1; p < A->n_pat; p++) m += (A->pat0.mask[p] & PAT_MASK_VALID) != 0;
+    if (n_masked) *n_masked = m;
+    if (cover_masked) *cover_masked = A->has_pat ? A->pat0.cover_masked : 0.0;
     return SPARSH_OK;
 }
 

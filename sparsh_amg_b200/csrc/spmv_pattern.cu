@@ -6,8 +6,9 @@
 //  * two dependent memory round trips per tile (pattern byte -> table look-up -> gathers).  Pattern 0 travels BY VALUE
 //    in the kernel parameters (Pat0, internal.cuh), so its offsets are constant-bank operands known before anything is
 //    loaded: every thread issues the pattern byte, b, x_i AND all gathers of pattern 0 for all its rows at once —
-//    one round trip — and only looks at the pattern byte when the data is there.  Rows that turn out to carry another
-//    pattern (boundary rows, a few per cent) are redone from the table in global memory, escapes from the CSR arrays;
+//    one round trip — and only looks at the pattern byte when the data is there.  Rows whose pattern is pattern 0 with
+//    terms left out (boundary rows, a few per cent: Pat0::mask) reuse those gathers and skip the missing terms; rows of
+//    any other pattern are redone from the table in global memory, escapes from the CSR arrays;
 //  * ~250 instructions per row of predicated 8-wide steps, selects and shared-memory look-ups (ncu on the dict kernel:
 //    issue slots 65 % busy, ALU the top pipe).  The fast path is straight-line code: per entry one integer add, one
 //    address computation, one LDG, one DMUL and one DADD whose second operands come from the constant bank;
@@ -72,13 +73,26 @@ __global__ void __launch_bounds__(THREADS)
         if (pid[s] < 0) continue;
         const int row = r0 + s * THREADS + tid;
         double sum = 0.0;
+        unsigned m;
         if (pid[s] == 0) {
 #pragma unroll
             for (int k = 0; k < LEN0; k++) sum = __dadd_rn(sum, __dmul_rn(Z.val[k], g[s][k]));
             if (NEEDS_D && table_d) e[s].d = Z.diag;
+        } else if ((m = Z.mask[pid[s]]) & PAT_MASK_VALID) {
+            // pattern 0 with terms left out (Pat0::mask: boundary rows and their Galerkin coarsenings; a quarter of the
+            // warps of the finest 256^3 level and most warps of the coarse levels hold some): pattern 0's straight-line
+            // code over the gathers already in registers.  A missing term's sum is discarded (the compiler selects the
+            // old sum: DADD + FSEL, no branch), never its product zeroed, so an Inf, NaN or -0 in a skipped neighbour
+            // changes nothing, as in the CSR kernels.
+#pragma unroll
+            for (int k = 0; k < LEN0; k++) {
+                const double t = __dmul_rn(Z.val[k], g[s][k]);
+                if (m & (1u << k)) sum = __dadd_rn(sum, t);
+            }
+            if (NEEDS_D && table_d) e[s].d = Z.diag;
         } else if (pid[s] != PAT_ESCAPE) {
-            // another pattern (boundary rows, a few per cent): walked straight from the table in global memory — a
-            // couple of KB that live in L1/L2 — by the lanes concerned only: no shared-memory copy, no CTA barrier
+            // another pattern: walked straight from the table in global memory — a couple of KB that live in L1/L2 —
+            // by the lanes concerned only: no shared-memory copy, no CTA barrier
             const int st = __ldg(P.start + pid[s]), en = __ldg(P.start + pid[s] + 1);
 #pragma unroll 1  // rare path: small code, the instruction cache belongs to the fast path
             for (int k = st; k < en; k++) {

@@ -115,6 +115,13 @@ class DeviceMatrix:
         check(self.lib.sparsh_matrix_pattern_stats(self.h, C.byref(a), C.byref(b), C.byref(c), C.byref(d)))
         return a.value, b.value, c.value, d.value
 
+    def pattern_mask_stats(self):
+        """(patterns other than pattern 0 that the lean kernel runs as masked pattern 0, share of the rows that carry
+        pattern 0 or one of them)"""
+        a, b = C.c_int(), C.c_double()
+        check(self.lib.sparsh_matrix_pattern_mask_stats(self.h, C.byref(a), C.byref(b)))
+        return a.value, b.value
+
     def kernel_name(self, epilogue):
         """name of the kernel instantiation launched for `epilogue` ('spmv' | 'residual' | 'jacobi' | 'prolong' | 'sor' |
         'spmv_dot' | 'resnorm')"""
