@@ -119,6 +119,12 @@ int sparsh_pattern_masks(int n_pat, const int *start, const double *ent_val, con
  * carry pattern 0 or one of those patterns */
 int sparsh_matrix_pattern_mask_stats(sparsh_matrix_t A, int *n_masked, double *cover_masked);
 
+/* Grid-transfer structure found at upload: *one_per_row = 1 when every row stores exactly one entry (rowptr[i] == i),
+ * *uniform_val = 1 when every stored value has the same bit pattern, *value (0 otherwise).  HEM's P has both, its
+ * R = P^T uniform values only.  A scalar-family matrix with one entry per row runs SpMV and prolongation with the
+ * aggregation kernel (no rowptr read, no val read when uniform); forcing KIND_SCALAR selects the plain scalar kernel. */
+int sparsh_matrix_transfer_info(sparsh_matrix_t A, int *one_per_row, int *uniform_val, double *value);
+
 /* ------------------------------------------------------------------ setup ------ */
 /* Galerkin product A_c = P^T (A P) on the device (SURVEY 8f.1): what parallel::coarsen_matrix does with two
  * mkl_sparse_spmm calls on the host (src/AMG_cycle_utilities.cpp:126-146).  Row-wise products with the host setup's
@@ -153,6 +159,9 @@ int sparsh_residual_norm(sparsh_matrix_t A, const double *d_b, const double *d_x
  *                                          106-127; parallel::jacobi_smoother, src/AMG_smoothers.cpp:53-76
  * (the CPU reference runs smooth_iter+1 = 7 sweeps, the GPU reference 6: SURVEY F7 — the count is an argument) */
 int sparsh_jacobi(sparsh_matrix_t A, const double *d_b, double *d_x, double *d_tmp, double omega, int sweeps);
+/* K1 from x = 0: x = (omega*b)/d, d the matrix' smoothing diagonal (A x = 0 needs no matrix pass).  With the lean
+ * csr-pattern8 kernel d is read through the pattern twin (1 B per row); the same bits either way. */
+int sparsh_jacobi_zero(sparsh_matrix_t A, const double *d_b, double omega, double *d_x);
 /* K6  multicolour SOR on a colour-permuted matrix: for each colour k, rows h_color_count[k]..[k+1] updated in
  * place, x_l -= (omega*(sum_j a_lj x_j - b_l))/d_l.   parallel::sor_smoother, src/AMG_smoothers.cpp:78-102 (no GPU
  * version exists in the reference: "SOR ... to be defined", src/AMG_gpu_matrix.cu:129) */
@@ -164,6 +173,10 @@ int sparsh_restrict(sparsh_matrix_t R, const double *d_r, double *d_bc);
 /* K5  xf += P xc                            csrmv beta=1, src/AMG_gpu_phases_2.cu:210;
  *                                          parallel::transfer_solution, src/AMG_cycle_utilities.cpp:107-112 */
 int sparsh_prolong_add(sparsh_matrix_t P, const double *d_xc, double *d_xf);
+/* K2+K4  bc = R (b - A x), the V-cycle's residual and restriction.  One fused pass when A runs the lean csr-pattern8
+ * kernel and R's values are uniform (HEM): the residual is neither stored nor read back.  Otherwise sparsh_residual
+ * into a temporary followed by sparsh_restrict (synchronous).  Bit-identical to the two calls either way. */
+int sparsh_residual_restrict(sparsh_matrix_t A, sparsh_matrix_t R, const double *d_b, const double *d_x, double *d_bc);
 
 /* K8  BLAS-1 (replace cublasDdot/Dnrm2/Daxpy and the kernels daxpby/daxpbyc, src/AMG_main_solvers.cu:17-33).
  * Reductions are two-stage with a fixed tree: bit-reproducible run to run. */

@@ -63,6 +63,7 @@ SIGNATURES = {
     "sparsh_matrix_kernel_name": (_i, [_vp, _i, C.c_char_p, _sz]),
     "sparsh_matrix_pattern_stats": (_i, [_vp, c_int_p, c_int_p, c_int_p, c_dbl_p]),
     "sparsh_matrix_pattern_mask_stats": (_i, [_vp, c_int_p, c_dbl_p]),
+    "sparsh_matrix_transfer_info": (_i, [_vp, c_int_p, c_int_p, c_dbl_p]),
     "sparsh_pattern_masks": (_i, [_i, c_int_p, c_dbl_p, c_int_p, _vp]),
     "sparsh_pattern_encode": (_i, [_i, _i, _i, c_int_p, c_int_p, c_dbl_p, c_dbl_p, _vp, c_dbl_p, c_int_p, c_int_p, c_int_p,
                                    c_int_p]),
@@ -79,6 +80,8 @@ SIGNATURES = {
     "sparsh_mc_sor": (_i, [_vp, c_int_p, _i, _vp, _vp, _d, _i]),
     "sparsh_restrict": (_i, [_vp, _vp, _vp]),
     "sparsh_prolong_add": (_i, [_vp, _vp, _vp]),
+    "sparsh_residual_restrict": (_i, [_vp, _vp, _vp, _vp, _vp]),
+    "sparsh_jacobi_zero": (_i, [_vp, _vp, _d, _vp]),
     "sparsh_dot": (_i, [_sz, _vp, _vp, c_dbl_p]),
     "sparsh_nrm2": (_i, [_sz, _vp, c_dbl_p]),
     "sparsh_dot_device": (_i, [_sz, _vp, _vp, _vp]),

@@ -6,8 +6,9 @@
 //   down: Jacobi(A_l,B_l,X_l) -> R_l = B_l - A_l X_l -> B_{l+1} = P_l^T R_l -> X_{l+1} = 0
 //   bottom: X_L = A_L^{-1} B_L
 //   up:   X_{l-1} += P_{l-1} X_l -> Jacobi(A_{l-1},B_{l-1},X_{l-1})
-// One fused kernel per Jacobi sweep (out of place, ping-pong), one per residual, restriction and
-// prolongation-correction; the first sweep after "X = 0" needs no matrix pass at all (A*0 = 0 exactly).
+// One fused kernel per Jacobi sweep (out of place, ping-pong), one for residual + restriction (two where the fused
+// kernel does not apply: resid_restrict_applies), one per prolongation-correction; the first sweep after "X = 0" needs
+// no matrix pass at all (A*0 = 0 exactly).
 // The whole cycle is captured into a CUDA graph: a 14-level hierarchy is ~250 launches, most of them on levels too
 // small to hide launch latency otherwise.
 #include <algorithm>
@@ -45,7 +46,11 @@ static int smooth(sparsh_hierarchy_s *h, Level &L, const double *b, double *&cur
     }
     for (int s = 0; s < sweeps; s++) {
         if (s == 0 && zero_guess) {
-            SP_TRY(k_jacobi_zero((size_t)L.n, b, L.A->diag, h->prm.omega, other));
+            // A x = 0: x = (omega*b)/d, d read through the pattern twin when A has one (1 B per row instead of 8)
+            if (jacobi_zero_pat_applies(L.A))
+                SP_TRY(launch_jacobi_zero_pat(L.A, b, h->prm.omega, other));
+            else
+                SP_TRY(k_jacobi_zero((size_t)L.n, b, L.A->diag, h->prm.omega, other));
         } else {
             EpiArgs a;
             a.b = b;
@@ -73,10 +78,15 @@ int enqueue_vcycle(sparsh_hierarchy_s *h, const double *b, double *x, bool x_is_
     for (int l = 0; l < L; l++) {
         Level &F = h->lev[l];
         SP_TRY(smooth(h, F, B[l], X[l], T[l], h->prm.pre_sweeps, l > 0 || x_is_zero));
-        EpiArgs a;
-        a.b = B[l];
-        SP_TRY(launch_csr(F.A, EPI_RESID, X[l], F.rbuf, a, 0, F.n));
-        SP_TRY(launch_csr(F.R, EPI_SPMV, F.rbuf, h->lev[l + 1].bbuf, EpiArgs(), 0, F.R->nrow));
+        if (resid_restrict_applies(F.A, F.R)) {
+            // B_{l+1} = R (B_l - A X_l) in one pass: the residual is not stored (rbuf stays unwritten)
+            SP_TRY(launch_resid_restrict(F.A, F.R, B[l], X[l], h->lev[l + 1].bbuf));
+        } else {
+            EpiArgs a;
+            a.b = B[l];
+            SP_TRY(launch_csr(F.A, EPI_RESID, X[l], F.rbuf, a, 0, F.n));
+            SP_TRY(launch_csr(F.R, EPI_SPMV, F.rbuf, h->lev[l + 1].bbuf, EpiArgs(), 0, F.R->nrow));
+        }
     }
     if (L == 0 && h->coarse.n == 0) {
         set_error("hierarchy without a coarse solver");

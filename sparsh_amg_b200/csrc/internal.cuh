@@ -169,6 +169,11 @@ struct sparsh_matrix_s {
     int n_pat = 0, n_pent = 0, n_escape = 0, pat_far = 0;
     bool has_pat = false;
     sparsh::Pat0 pat0;  // len == 0: the lean (speculative-gather) variant does not apply
+    // grid-transfer structure, read from the host arrays at upload (HEM: P has both, R = P^T uniform values only)
+    bool one_per_row = false;  // rowptr[i] == i: exactly one stored entry per row
+    bool uniform_val = false;  // every stored value has the same bits, uval
+    double uval = 0.0;
+    bool agg = false;  // KIND_SCALAR runs SpMV / prolongation with csr_agg_kernel (one_per_row; cleared by force_kernel)
     sparsh::PatView pattern(bool use_pdiag) const {
         return sparsh::PatView{pat, pat_ent, pat_start, pat_diag, n_pat, n_pent, use_pdiag ? 1 : 0, pat_far};
     }
@@ -239,6 +244,15 @@ struct HaloSync {
 // rows [b1,e1) + [b2,e2) (strips: handshake CTAs when hs is given) + [b3,e3) (interior) in one launch
 int launch_csr3(const sparsh_matrix_s *A, int epi, const double *x, double *y, const EpiArgs &args, int b1, int e1,
                 int b2, int e2, int b3, int e3, const HaloSync *hs);
+// V-cycle grid transfers (spmv_pattern.cu).  bc = R (b - A x) in one pass, one thread per row of R, the residual never
+// stored: same operations in the same order as EPI_RESID followed by the restriction SpMV, so the same bits.  Applies
+// when A runs the lean csr-pattern8 kernel and R's stored values are all one value (aggregation).
+bool resid_restrict_applies(const sparsh_matrix_s *A, const sparsh_matrix_s *R);
+int launch_resid_restrict(const sparsh_matrix_s *A, const sparsh_matrix_s *R, const double *b, const double *x, double *bc);
+// x = (omega*b)/d with d = A->diag taken from A's csr-pattern8 twin (1 B per row instead of 8); applies with the lean kernel
+bool jacobi_zero_pat_applies(const sparsh_matrix_s *A);
+int launch_jacobi_zero_pat(const sparsh_matrix_s *A, const double *b, double omega, double *x);
+
 inline int launch_csr2(const sparsh_matrix_s *A, int epi, const double *x, double *y, const EpiArgs &args, int b1, int e1,
                        int b2, int e2, const HaloSync *hs) {
     return launch_csr3(A, epi, x, y, args, b1, e1, b2, e2, 0, 0, hs);

@@ -49,6 +49,27 @@ void choose_kernel(sparsh_matrix_s *A, const int *rp) {
     }
 }
 
+// Aggregation operators (HEM: P has one 1.0 per row, R = P^T rows of one or two 1.0) are recognised from the host
+// arrays: one entry per row, and / or one value (bit pattern) throughout.  Both scans stop at the first counterexample,
+// so on any other matrix they cost a few entries.  One entry per row selects csr_agg_kernel for SpMV and prolongation.
+void transfer_structure(sparsh_matrix_s *A, const int *rp, const double *v) {
+    const int n = A->nrow;
+    bool one = n > 0 && A->nnz == n;
+    for (int i = 1; one && i <= n; i++) one = rp[i] == i;
+    bool uni = A->nnz > 0;
+    uint64_t u0 = 0;
+    if (uni) std::memcpy(&u0, v, sizeof u0);
+    for (int k = 1; uni && k < A->nnz; k++) {
+        uint64_t u;
+        std::memcpy(&u, v + k, sizeof u);
+        uni = u == u0;
+    }
+    A->one_per_row = one;
+    A->uniform_val = uni;
+    std::memcpy(&A->uval, &u0, sizeof u0);
+    A->agg = one && A->kind == KIND_SCALAR;
+}
+
 // uploads run on the library's stream, or on the calling thread's own stream while sparsh_hierarchy_create builds the
 // levels with several host threads (set_upload_stream)
 thread_local cudaStream_t t_upload_stream = nullptr;
@@ -735,6 +756,7 @@ int sparsh_matrix_create(int nrow, int ncol, int nnz, const int *h_rowptr, const
     };
     lap("validated");
     choose_kernel(A, h_rowptr);
+    transfer_structure(A, h_rowptr, h_val);
     lap("row statistics");
     int rc = upload(A, h_rowptr, h_colindex, h_val, h_diag);
     if (rc != SPARSH_OK) {
@@ -897,6 +919,14 @@ int sparsh_matrix_pattern_mask_stats(sparsh_matrix_t A, int *n_masked, double *c
     return SPARSH_OK;
 }
 
+int sparsh_matrix_transfer_info(sparsh_matrix_t A, int *one_per_row, int *uniform_val, double *value) {
+    SP_REQUIRE(A != nullptr, "matrix is NULL");
+    if (one_per_row) *one_per_row = A->one_per_row ? 1 : 0;
+    if (uniform_val) *uniform_val = A->uniform_val ? 1 : 0;
+    if (value) *value = A->uniform_val ? A->uval : 0.0;
+    return SPARSH_OK;
+}
+
 // name of the kernel instantiation launch_csr picks for this matrix and epilogue (reports: bench.py's roofline / kernel
 // table must name what really ran)
 int sparsh_matrix_kernel_name(sparsh_matrix_t A, int epi, char *buf, size_t len) {
@@ -906,7 +936,10 @@ int sparsh_matrix_kernel_name(sparsh_matrix_t A, int epi, char *buf, size_t len)
     char tmp[160];
     switch (A->kind) {
         case KIND_SCALAR:
-            std::snprintf(tmp, sizeof tmp, "csr_scalar_kernel<256,%s>", epis[epi]);
+            if (A->agg && (epi == EPI_SPMV || epi == EPI_PROLONG))
+                std::snprintf(tmp, sizeof tmp, "csr_agg_kernel<%s,%s>", epis[epi], A->uniform_val ? "true" : "false");
+            else
+                std::snprintf(tmp, sizeof tmp, "csr_scalar_kernel<256,%s>", epis[epi]);
             break;
         case KIND_STREAM:
             std::snprintf(tmp, sizeof tmp, "csr_stream_kernel<%d,%s>", A->threads, epis[epi]);
@@ -932,6 +965,7 @@ int sparsh_matrix_kernel_name(sparsh_matrix_t A, int epi, char *buf, size_t len)
 
 int sparsh_matrix_force_kernel(sparsh_matrix_t A, int kind, int tl) {
     SP_REQUIRE(A != nullptr, "matrix is NULL");
+    A->agg = false;  // a forced kind runs that family's kernel: KIND_SCALAR is csr_scalar_kernel even for one entry per row
     if (kind == KIND_SCALAR) {
         A->kind = kind;
         A->threads = 256;
@@ -1015,6 +1049,12 @@ int sparsh_jacobi(sparsh_matrix_t A, const double *d_b, double *d_x, double *d_t
     return SPARSH_OK;
 }
 
+int sparsh_jacobi_zero(sparsh_matrix_t A, const double *d_b, double omega, double *d_x) {
+    SP_REQUIRE(A != nullptr && A->diag != nullptr, "jacobi needs a square matrix with a diagonal");
+    if (jacobi_zero_pat_applies(A)) return launch_jacobi_zero_pat(A, d_b, omega, d_x);
+    return k_jacobi_zero((size_t)A->nrow, d_b, A->diag, omega, d_x);
+}
+
 int sparsh_mc_sor(sparsh_matrix_t A, const int *h_color_count, int total_colors, const double *d_b, double *d_x,
                   double omega, int sweeps) {
     SP_REQUIRE(A != nullptr && A->diag != nullptr, "mc_sor needs a square matrix with a diagonal");
@@ -1034,6 +1074,24 @@ int sparsh_mc_sor(sparsh_matrix_t A, const int *h_color_count, int total_colors,
 int sparsh_restrict(sparsh_matrix_t R, const double *d_r, double *d_bc) {
     SP_REQUIRE(R != nullptr, "matrix is NULL");
     return launch_csr(R, EPI_SPMV, d_r, d_bc, EpiArgs(), 0, R->nrow);
+}
+
+int sparsh_residual_restrict(sparsh_matrix_t A, sparsh_matrix_t R, const double *d_b, const double *d_x, double *d_bc) {
+    SP_REQUIRE(A != nullptr && R != nullptr, "matrix is NULL");
+    SP_REQUIRE(R->ncol == A->nrow, "R's column count differs from A's row count");
+    if (resid_restrict_applies(A, R)) return launch_resid_restrict(A, R, d_b, d_x, d_bc);
+    // the two launches the fused kernel replaces, through a temporary residual
+    double *r = nullptr;
+    SP_CUDA(cudaMalloc(&r, sizeof(double) * ((size_t)A->nrow + 1)));
+    EpiArgs a;
+    a.b = d_b;
+    int rc = launch_csr(A, EPI_RESID, d_x, r, a, 0, A->nrow);
+    if (rc == SPARSH_OK) rc = launch_csr(R, EPI_SPMV, r, d_bc, EpiArgs(), 0, R->nrow);
+    const cudaError_t e = cudaStreamSynchronize(ctx().stream);
+    cudaFree(r);
+    SP_TRY(rc);
+    SP_CUDA(e);
+    return SPARSH_OK;
 }
 
 int sparsh_prolong_add(sparsh_matrix_t P, const double *d_xc, double *d_xf) {

@@ -340,6 +340,27 @@ __global__ void __launch_bounds__(THREADS)
 }
 
 // ---------------------------------------------------------------------------------------------------------
+// AGGREGATION kernel: SpMV / prolongation with an operator of exactly one entry per row (rowptr[i] == i: HEM's P).  The
+// scalar kernel's arithmetic in its order — s = 0 + v*x[col[i]] (the 0 + turns a -0 product into +0), then the epilogue
+// — without reading rowptr, and without val when every stored value is the same (v passed by value, UNIFORM).
+// ---------------------------------------------------------------------------------------------------------
+template <int EPI, bool UNIFORM>
+__global__ void __launch_bounds__(256)
+    csr_agg_kernel(const int *__restrict__ col, const double *__restrict__ val, double v, const double *__restrict__ x, double *y,
+                   RowRange rr) {
+    int r0, row_end;
+    block_rows(rr, 256, r0, row_end);
+    const int row = r0 + threadIdx.x;
+    if (row >= row_end) return;
+    const double a = UNIFORM ? v : __ldg(val + row);
+    const double s = __dadd_rn(0.0, __dmul_rn(a, __ldg(x + __ldg(col + row))));
+    if (EPI == EPI_PROLONG)
+        y[row] = __dadd_rn(s, y[row]);
+    else
+        y[row] = s;
+}
+
+// ---------------------------------------------------------------------------------------------------------
 // VECTOR kernel: LANES lanes per row, fixed shuffle tree
 // ---------------------------------------------------------------------------------------------------------
 template <int LANES, int EPI, bool DIST>
@@ -488,6 +509,17 @@ static int launch_scalar(const sparsh_matrix_s *A, const double *x, double *y, c
     if (grid > RED_MAX_BLOCKS) {
         set_error("matrix too large for the reduction workspace");
         return SPARSH_ERR_INVALID;
+    }
+    if constexpr (EPI == EPI_SPMV || EPI == EPI_PROLONG) {
+        // one entry per row (HEM's P): rowptr is not read, nor val when it holds one value.  Single-GPU launches only:
+        // the distributed operators keep the kernel with the halo handshake.
+        if (A->agg && !d.dist) {
+            if (A->uniform_val)
+                csr_agg_kernel<EPI, true><<<grid, 256, 0, c.stream>>>(A->col, A->val, A->uval, x, y, d.rr);
+            else
+                csr_agg_kernel<EPI, false><<<grid, 256, 0, c.stream>>>(A->col, A->val, 0.0, x, y, d.rr);
+            return finish_launch<EPI>(grid, args);
+        }
     }
     if (d.dist)
         csr_scalar_kernel<256, EPI, true><<<grid, 256, 0, c.stream>>>(A->view(), x, y, args, d.rr, c.partials, d.hs);

@@ -26,6 +26,51 @@ __device__ __forceinline__ double gather(const double *x, int c, int ncol, int h
     return load_xd<COHERENT, DIST>(x, c, halo_begin);
 }
 
+// One row of A as the lean kernel evaluates it, from the row's speculative pattern-0 gathers g (already in registers):
+// pattern 0 by value, pattern 0 with terms left out (mask), another pattern from the table, or an escape from the CSR
+// arrays.  NEEDS_D: d receives the row's diagonal, from the table when table_d, else (escapes always) dvec[row].
+template <int LEN0, bool COH, bool DIST, bool NEEDS_D>
+__device__ __forceinline__ double lean_row_sum(const CsrView &A, const PatView &P, const Pat0 &Z, const double *x, int row, int pid,
+                                               const double (&g)[LEN0], bool table_d, const double *dvec, int halo_begin,
+                                               double &d) {
+    double sum = 0.0;
+    unsigned m;
+    if (pid == 0) {
+#pragma unroll
+        for (int k = 0; k < LEN0; k++) sum = __dadd_rn(sum, __dmul_rn(Z.val[k], g[k]));
+        if (NEEDS_D && table_d) d = Z.diag;
+    } else if ((m = Z.mask[pid]) & PAT_MASK_VALID) {
+        // pattern 0 with terms left out (Pat0::mask: boundary rows and their Galerkin coarsenings; a quarter of the
+        // warps of the finest 256^3 level and most warps of the coarse levels hold some): pattern 0's straight-line
+        // code over the gathers already in registers.  A missing term's sum is discarded (the compiler selects the
+        // old sum: DADD + FSEL, no branch), never its product zeroed, so an Inf, NaN or -0 in a skipped neighbour
+        // changes nothing, as in the CSR kernels.
+#pragma unroll
+        for (int k = 0; k < LEN0; k++) {
+            const double t = __dmul_rn(Z.val[k], g[k]);
+            if (m & (1u << k)) sum = __dadd_rn(sum, t);
+        }
+        if (NEEDS_D && table_d) d = Z.diag;
+    } else if (pid != PAT_ESCAPE) {
+        // another pattern: walked straight from the table in global memory — a couple of KB that live in L1/L2 —
+        // by the lanes concerned only: no shared-memory copy, no CTA barrier
+        const int st = __ldg(P.start + pid), en = __ldg(P.start + pid + 1);
+#pragma unroll 1  // rare path: small code, the instruction cache belongs to the fast path
+        for (int k = st; k < en; k++) {
+            const int4 q = __ldg(reinterpret_cast<const int4 *>(P.ent) + k);
+            sum = __dadd_rn(sum, __dmul_rn(__hiloint2double(q.y, q.x), load_xd<COH, DIST>(x, row + q.z, halo_begin)));
+        }
+        if (NEEDS_D && table_d) d = __ldg(P.pdiag + pid);
+    } else {
+        const int lo = A.rowptr[row], hi = A.rowptr[row + 1];
+#pragma unroll 1
+        for (int k = lo; k < hi; k++)
+            sum = __dadd_rn(sum, __dmul_rn(__ldg(A.val + k), load_xd<COH, DIST>(x, __ldg(A.col + k), halo_begin)));
+        if (NEEDS_D) d = dvec[row];
+    }
+    return sum;
+}
+
 template <int THREADS, int RPT, int LEN0, int EPI, bool DIST>
 __global__ void __launch_bounds__(THREADS)
     csr_pat2_kernel(CsrView A, PatView P, const __grid_constant__ Pat0 Z, const double *x, double *y, EpiArgs args,
@@ -72,41 +117,7 @@ __global__ void __launch_bounds__(THREADS)
     for (int s = 0; s < RPT; s++) {
         if (pid[s] < 0) continue;
         const int row = r0 + s * THREADS + tid;
-        double sum = 0.0;
-        unsigned m;
-        if (pid[s] == 0) {
-#pragma unroll
-            for (int k = 0; k < LEN0; k++) sum = __dadd_rn(sum, __dmul_rn(Z.val[k], g[s][k]));
-            if (NEEDS_D && table_d) e[s].d = Z.diag;
-        } else if ((m = Z.mask[pid[s]]) & PAT_MASK_VALID) {
-            // pattern 0 with terms left out (Pat0::mask: boundary rows and their Galerkin coarsenings; a quarter of the
-            // warps of the finest 256^3 level and most warps of the coarse levels hold some): pattern 0's straight-line
-            // code over the gathers already in registers.  A missing term's sum is discarded (the compiler selects the
-            // old sum: DADD + FSEL, no branch), never its product zeroed, so an Inf, NaN or -0 in a skipped neighbour
-            // changes nothing, as in the CSR kernels.
-#pragma unroll
-            for (int k = 0; k < LEN0; k++) {
-                const double t = __dmul_rn(Z.val[k], g[s][k]);
-                if (m & (1u << k)) sum = __dadd_rn(sum, t);
-            }
-            if (NEEDS_D && table_d) e[s].d = Z.diag;
-        } else if (pid[s] != PAT_ESCAPE) {
-            // another pattern: walked straight from the table in global memory — a couple of KB that live in L1/L2 —
-            // by the lanes concerned only: no shared-memory copy, no CTA barrier
-            const int st = __ldg(P.start + pid[s]), en = __ldg(P.start + pid[s] + 1);
-#pragma unroll 1  // rare path: small code, the instruction cache belongs to the fast path
-            for (int k = st; k < en; k++) {
-                const int4 q = __ldg(reinterpret_cast<const int4 *>(P.ent) + k);
-                sum = __dadd_rn(sum, __dmul_rn(__hiloint2double(q.y, q.x), load_xd<COH, DIST>(x, row + q.z, hs.halo_begin)));
-            }
-            if (NEEDS_D && table_d) e[s].d = __ldg(P.pdiag + pid[s]);
-        } else {
-            const int lo = A.rowptr[row], hi = A.rowptr[row + 1];
-#pragma unroll 1
-            for (int k = lo; k < hi; k++)
-                sum = __dadd_rn(sum, __dmul_rn(__ldg(A.val + k), load_xd<COH, DIST>(x, __ldg(A.col + k), hs.halo_begin)));
-            if (NEEDS_D) e[s].d = args.d[row];
-        }
+        const double sum = lean_row_sum<LEN0, COH, DIST, NEEDS_D>(A, P, Z, x, row, pid[s], g[s], table_d, args.d, hs.halo_begin, e[s].d);
         // reduction contributions are added in row order within the thread: a fixed tree
         contrib = __dadd_rn(contrib, epi_store<EPI, DIST>(args, e[s], sum, y, row, strip_cta));
     }
@@ -159,6 +170,85 @@ int launch_epi(const sparsh_matrix_s *A, const double *x, double *y, const EpiAr
     }
 }
 
+// V-cycle, fused residual + restriction: bc[i] = sum over the entries k of R's row i (stored order) of vR * r_j,
+// r_j = b_j - (A x)_j, j = Rcol[k] — exactly what EPI_RESID followed by csr_scalar_kernel<EPI_SPMV> on R computes, with
+// the residual never stored nor read back.  One thread per coarse row; fine row j is evaluated as csr_pat2_kernel does
+// (lean_row_sum).  HEM's R has rows of two entries (pairs) and of one (singletons, numbered last): the loads of both
+// rows of a pair — pattern byte, b and the clamped speculative pattern-0 gathers — are issued before either is used,
+// so a pair costs one round trip after the Rcol load, as a row of the lean kernel does.
+// (minimum 4 CTAs per SM: without it ptxas picks 40 registers and spills 16-20 B of the pair's state; with it, 40 / 46
+// registers and no spill)
+template <int LEN0>
+__global__ void __launch_bounds__(256, 4)
+    resid_restrict_kernel(CsrView A, PatView P, const __grid_constant__ Pat0 Z, const int *__restrict__ Rrp,
+                          const int *__restrict__ Rcol, double vR, int nc, const double *__restrict__ b, const double *x,
+                          double *bc) {
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= nc) return;
+    const int lo = __ldg(Rrp + i), hi = __ldg(Rrp + i + 1);
+    double acc = 0.0, dd = 0.0;
+    if (hi - lo == 2) {
+        int j[2], pid[2];
+        double bj[2], g[2][LEN0];
+        j[0] = __ldg(Rcol + lo);
+        j[1] = __ldg(Rcol + lo + 1);
+#pragma unroll
+        for (int t = 0; t < 2; t++) {
+            pid[t] = __ldg(P.pat + j[t]);
+            bj[t] = __ldg(b + j[t]);
+#pragma unroll
+            for (int k = 0; k < LEN0; k++) g[t][k] = gather<false, false, false>(x, j[t] + Z.off[k], A.ncol, 0);
+        }
+#pragma unroll
+        for (int t = 0; t < 2; t++) {
+            const double s = lean_row_sum<LEN0, false, false, false>(A, P, Z, x, j[t], pid[t], g[t], false, nullptr, 0, dd);
+            acc = __dadd_rn(acc, __dmul_rn(vR, __dsub_rn(bj[t], s)));
+        }
+    } else {
+#pragma unroll 1
+        for (int k = lo; k < hi; k++) {
+            const int j = __ldg(Rcol + k);
+            const int pid = __ldg(P.pat + j);
+            const double bj = __ldg(b + j);
+            double g[LEN0];
+#pragma unroll
+            for (int q = 0; q < LEN0; q++) g[q] = gather<false, false, false>(x, j + Z.off[q], A.ncol, 0);
+            const double s = lean_row_sum<LEN0, false, false, false>(A, P, Z, x, j, pid, g, false, nullptr, 0, dd);
+            acc = __dadd_rn(acc, __dmul_rn(vR, __dsub_rn(bj, s)));
+        }
+    }
+    bc[i] = acc;
+}
+
+// First Jacobi sweep from x = 0: x = (omega*b)/d, d = A's diagonal read through the csr-pattern8 twin — pattern 0 by
+// value, other patterns from the tabulated diagonals (a pattern with a valid mask has pattern 0's diagonal bits), escape
+// rows from the diagonal array.  The upload makes every row whose diagonal differs from its pattern's an escape, so d
+// has the bits of A->diag on every row: 17 B per row moved instead of 24.
+__global__ void __launch_bounds__(256)
+    jacobi_zero_pat_kernel(int n, const unsigned char *__restrict__ pat, const double *__restrict__ pdiag, double diag0,
+                           const double *__restrict__ diag, const double *__restrict__ b, double omega, double *x) {
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= n) return;
+    const int p = __ldg(pat + i);
+    const double bi = __ldg(b + i);
+    double d = diag0;
+    if (p == PAT_ESCAPE)
+        d = __ldg(diag + i);
+    else if (p != 0)
+        d = __ldg(pdiag + p);
+    x[i] = __ddiv_rn(__dmul_rn(omega, bi), d);
+}
+
+template <int LEN0>
+int launch_rr(const sparsh_matrix_s *A, const sparsh_matrix_s *R, const double *b, const double *x, double *bc) {
+    const int nc = R->nrow;
+    resid_restrict_kernel<LEN0><<<(nc + 255) / 256, 256, 0, ctx().stream>>>(A->view(), A->pattern(false), A->pat0, R->rowptr, R->col,
+                                                                          R->uval, nc, b, x, bc);
+    count_launch();
+    SP_CUDA(cudaGetLastError());
+    return SPARSH_OK;
+}
+
 }  // namespace
 
 // stencils whose interior row has 5 or 7 entries (2D/3D Poisson-like operators and their semi-coarsened Galerkin
@@ -187,6 +277,29 @@ int launch_pattern_lean(const sparsh_matrix_s *A, int epi, const double *x, doub
     }
     set_error("unknown epilogue");
     return SPARSH_ERR_INVALID;
+}
+
+bool resid_restrict_applies(const sparsh_matrix_s *A, const sparsh_matrix_s *R) {
+    return A->kind == KIND_PATTERN && pattern_lean_applies(A) && R->uniform_val && R->ncol == A->nrow;
+}
+
+int launch_resid_restrict(const sparsh_matrix_s *A, const sparsh_matrix_s *R, const double *b, const double *x, double *bc) {
+    if (R->nrow == 0) return SPARSH_OK;
+    if (A->pat0.len == 5) return launch_rr<5>(A, R, b, x, bc);
+    return launch_rr<7>(A, R, b, x, bc);
+}
+
+bool jacobi_zero_pat_applies(const sparsh_matrix_s *A) {
+    return A->kind == KIND_PATTERN && pattern_lean_applies(A) && A->diag != nullptr;
+}
+
+int launch_jacobi_zero_pat(const sparsh_matrix_s *A, const double *b, double omega, double *x) {
+    const int n = A->nrow;
+    if (n == 0) return SPARSH_OK;
+    jacobi_zero_pat_kernel<<<(n + 255) / 256, 256, 0, ctx().stream>>>(n, A->pat, A->pat_diag, A->pat0.diag, A->diag, b, omega, x);
+    count_launch();
+    SP_CUDA(cudaGetLastError());
+    return SPARSH_OK;
 }
 
 }  // namespace sparsh

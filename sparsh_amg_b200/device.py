@@ -122,6 +122,12 @@ class DeviceMatrix:
         check(self.lib.sparsh_matrix_pattern_mask_stats(self.h, C.byref(a), C.byref(b)))
         return a.value, b.value
 
+    def transfer_info(self):
+        """(one entry per row, one value throughout, that value) as the upload found them: aggregation operators"""
+        a, b, v = C.c_int(), C.c_int(), C.c_double()
+        check(self.lib.sparsh_matrix_transfer_info(self.h, C.byref(a), C.byref(b), C.byref(v)))
+        return bool(a.value), bool(b.value), v.value
+
     def kernel_name(self, epilogue):
         """name of the kernel instantiation launched for `epilogue` ('spmv' | 'residual' | 'jacobi' | 'prolong' | 'sor' |
         'spmv_dot' | 'resnorm')"""
@@ -170,6 +176,18 @@ class DeviceMatrix:
         bc = bc or DeviceVector(self.nrow)
         check(self.lib.sparsh_restrict(self.h, r.ptr, bc.ptr))
         return bc
+
+    def residual_restrict(self, R, b, x, bc=None):
+        """bc = R (b - A x) (self is A): one fused pass where it applies, else residual + restriction"""
+        bc = bc or DeviceVector(R.nrow)
+        check(self.lib.sparsh_residual_restrict(self.h, R.h, b.ptr, x.ptr, bc.ptr))
+        return bc
+
+    def jacobi_zero(self, b, omega, x=None):
+        """x = (omega*b)/d: the first Jacobi sweep from x = 0, d the smoothing diagonal"""
+        x = x or DeviceVector(self.nrow)
+        check(self.lib.sparsh_jacobi_zero(self.h, b.ptr, float(omega), x.ptr))
+        return x
 
     def prolong_add(self, xc, xf):
         check(self.lib.sparsh_prolong_add(self.h, xc.ptr, xf.ptr))

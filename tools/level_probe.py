@@ -10,6 +10,13 @@ before the host has enqueued the next one, and the events then time the enqueue 
 that floor (a one-element fill per call) and marks every row within 1.5x of it `launch_bound`: its ms and GB/s are
 upper / lower bounds, not kernel figures.
     python tools/level_probe.py [--grid 256] [--out level_probe.json] [--census]
+On every level but the coarsest it also times the grid transfers of the V-cycle against the kernels they replace:
+resid_restrict (fused residual + restriction, sparsh_residual_restrict) against resid+restrict (sparsh_residual into a
+vector, then sparsh_restrict), prolong (the default: the aggregation kernel for HEM's P) against prolong_scalar (P forced
+to KIND_SCALAR), and zero_sweep (x = (omega*b)/d, sparsh_jacobi_zero: d through the pattern twin) against
+zero_sweep_diag (the same with A forced to the stream kernel, which reads the diagonal array; timed last on a level, as
+the forcing is not undone).  Their stored bytes count each array once: pattern byte 1, b / x / vectors 8, R / P column
+4, rowptr 4 per row, values 8 unless the operator passes its one value by value.
 --census adds, per level, what the csr-pattern8 encoder makes of the level (host encoder, no GPU time): patterns, rows
 of pattern 0, patterns the lean kernel runs as masked pattern 0, and the share of 32-row warps that mix pattern-0 rows with
 rows of other patterns.
@@ -85,6 +92,7 @@ def main():
     A = host.HostMatrix.poisson3d(args.grid, args.grid, args.grid)
     amg = host.HostAmg(A)
     dH = amg.upload()
+    host_levels = amg.levels()
     gpu = gpu_info()
     print(f"# {args.grid}^3 HEM hierarchy, {dH.nlevels} levels, built and uploaded in {time.time() - t0:.1f} s; {gpu}", flush=True)
     ck = sp.capi.check
@@ -94,8 +102,18 @@ def main():
     floor = benchutil.timed(torch, stream, fill, 2000)
     print(f"# enqueue floor: {floor * 1e6:.2f} us per launch (rows within 1.5x of it are marked launch-bound)", flush=True)
     rows = []
+    def timed_row(k, n, z, op, kernel, per_call, kernels, fn, nb):
+        once = benchutil.timed(torch, stream, fn, 3)
+        reps = max(args.min_reps, min(5000, int(args.target_ms * 1e-3 / max(once, 1e-7))))
+        sec = benchutil.timed(torch, stream, fn, reps) / per_call
+        row = {"level": k, "rows": n, "nnz": z, "op": op, "kernel": kernel, "launches": reps * per_call,
+               "ms": sec * 1e3, "stored_bytes": nb, "gbs": nb / sec / 1e9, "launch_bound": sec * per_call <= 1.5 * floor * kernels}
+        print(f"L{k:<2d} {n:>9d} rows  {op:15s} {row['kernel']:40s} {row['ms']:9.5f} ms  {row['gbs']:8.1f} GB/s  "
+              f"({row['launches']} launches){'  launch-bound' if row['launch_bound'] else ''}", flush=True)
+        return row
+
     for k in range(dH.nlevels):
-        Ak, _, _ = dH.level(k)
+        Ak, Pk, Rk = dH.level(k)
         n, m, z = Ak.nrow, Ak.ncol, Ak.nnz
         kind = Ak.kernel()[0]
         rng = np.random.default_rng(k)
@@ -106,15 +124,34 @@ def main():
                ("spmv", 1, 1, lambda: ck(lib.sparsh_spmv(Ak.h, x.ptr, y.ptr))),
                ("spmv_dot", 1, 2, lambda: ck(lib.sparsh_spmv_dot(Ak.h, x.ptr, y.ptr, dsc.ptr)))]
         for op, per_call, kernels, fn in ops:  # per_call: sweeps per call; kernels: launches per call (+ finalize)
-            once = benchutil.timed(torch, stream, fn, 3)
-            reps = max(args.min_reps, min(5000, int(args.target_ms * 1e-3 / max(once, 1e-7))))
-            sec = benchutil.timed(torch, stream, fn, reps) / per_call
-            nb = benchutil.stored_bytes(kind, op, n, m, z)
-            row = {"level": k, "rows": n, "nnz": z, "op": op, "kernel": Ak.kernel_name(op), "launches": reps * per_call,
-                   "ms": sec * 1e3, "stored_bytes": nb, "gbs": nb / sec / 1e9, "launch_bound": sec * per_call <= 1.5 * floor * kernels}
-            rows.append(row)
-            print(f"L{k:<2d} {n:>9d} rows  {op:9s} {row['kernel']:40s} {row['ms']:9.5f} ms  {row['gbs']:8.1f} GB/s  "
-                  f"({row['launches']} launches){'  launch-bound' if row['launch_bound'] else ''}", flush=True)
+            rows.append(timed_row(k, n, z, op, Ak.kernel_name(op), per_call, kernels, fn, benchutil.stored_bytes(kind, op, n, m, z)))
+        if Pk is None:
+            continue
+        mc = Pk.ncol
+        r, bc, xc = sp.DeviceVector(n), sp.DeviceVector(mc), sp.DeviceVector(data=rng.standard_normal(mc))
+        one, uni, _ = Pk.transfer_info()
+        hP = host_levels[k]["P"]  # a private copy of P on the plain scalar kernel
+        Pf = sp.DeviceMatrix(hP.nrow, hP.ncol, hP.rowptr, hP.colindex, hP.val).force_kernel(sp.capi.KIND_SCALAR, 256)
+        pair_nb = benchutil.stored_bytes(kind, "residual", n, m, z) + 4 * (mc + 1) + 12 * Pk.nnz + 8 * n + 8 * mc
+        fused_nb = n + 16 * n + 4 * (mc + 1) + 4 * Pk.nnz + 8 * mc + (0 if Rk.transfer_info()[1] else 8 * Pk.nnz)
+        xfer = [("resid+restrict", f"{Ak.kernel_name('residual')} + {Rk.kernel_name('spmv')}", 2,
+                 lambda: (ck(lib.sparsh_residual(Ak.h, b.ptr, x.ptr, r.ptr)), ck(lib.sparsh_restrict(Rk.h, r.ptr, bc.ptr))), pair_nb),
+                ("resid_restrict", "resid_restrict_kernel" if Ak.kernel_name("residual").startswith("csr_pat2") and Rk.transfer_info()[1]
+                 else "(two launches)", 1, lambda: ck(lib.sparsh_residual_restrict(Ak.h, Rk.h, b.ptr, x.ptr, bc.ptr)), fused_nb),
+                ("prolong_scalar", Pf.kernel_name("prolong"), 1, lambda: ck(lib.sparsh_prolong_add(Pf.h, xc.ptr, y.ptr)),
+                 4 * (n + 1) + 12 * Pk.nnz + 8 * mc + 16 * n),
+                ("prolong", Pk.kernel_name("prolong"), 1, lambda: ck(lib.sparsh_prolong_add(Pk.h, xc.ptr, y.ptr)),
+                 (4 * n + (0 if uni else 8 * n) if one else 4 * (n + 1) + 12 * Pk.nnz) + 8 * mc + 16 * n),
+                ("zero_sweep", "jacobi_zero_pat_kernel" if Ak.kernel_name("jacobi").startswith("csr_pat2") else "jacobi_zero_kernel", 1,
+                 lambda: ck(lib.sparsh_jacobi_zero(Ak.h, b.ptr, 0.66667, t.ptr)),
+                 17 * n if Ak.kernel_name("jacobi").startswith("csr_pat2") else 24 * n)]
+        for op, kname, kernels, fn, nb in xfer:
+            rows.append(timed_row(k, n, z, op, kname, 1, kernels, fn, nb))
+        if Ak.kernel()[0] == sp.capi.KIND_PATTERN:
+            Ak.force_kernel(sp.capi.KIND_STREAM, 128)  # not undone: nothing else runs on this level afterwards
+            rows.append(timed_row(k, n, z, "zero_sweep_diag", "jacobi_zero_kernel", 1, 1,
+                                  lambda: ck(lib.sparsh_jacobi_zero(Ak.h, b.ptr, 0.66667, t.ptr)), 24 * n))
+        Pf.free()
     out = {"grid": args.grid, "levels": dH.nlevels, "gpu": gpu, "enqueue_floor_ms": floor * 1e3, "timings": rows}
     if args.census:
         out["census"] = census(lib, amg.levels())
