@@ -65,6 +65,16 @@ int sparsh_fill(double *d_x, size_t n, double value);
  * h_diag may be NULL: the diagonal is then extracted like sp_matrix_fill_diagonal (src/AMG_cpu_matrix.cpp:35-51). */
 int sparsh_matrix_create(int nrow, int ncol, int nnz, const int *h_rowptr, const int *h_colindex,
                          const double *h_val, const double *h_diag, sparsh_matrix_t *out);
+/* New values for a matrix whose sparsity is unchanged.  d_val[nnz] is on the device, in the stored entry order.
+ * d_diag[nrow] may be NULL: the diagonal is then extracted like sp_matrix_fill_diagonal.  Every value-derived choice
+ * is made again exactly as sparsh_matrix_create makes it for the same arrays.  That covers the diagonal, the
+ * csr-pattern8 and csr-dict16 twins with Pat0 and its masks, the kernel family and the transfer flags, under every
+ * SPARSH_PATTERN / SPARSH_DICT setting.  A kernel forced with sparsh_matrix_force_kernel is forgotten.  The encoders'
+ * device scratch stays with the calling thread, so later updates of the same sizes allocate nothing. */
+int sparsh_matrix_update_values(sparsh_matrix_t A, const double *d_val, const double *d_diag);
+/* Copy a device matrix back to the host.  Any pointer may be NULL (that array is skipped).
+ * Sizes: rowptr[nrow+1], colindex[nnz], val[nnz], diag[nrow]. */
+int sparsh_matrix_fetch(sparsh_matrix_t A, int *h_rowptr, int *h_colindex, double *h_val, double *h_diag);
 /* explicit R = P^T (stable: each R row lists fine rows ascending), built once; replaces the transposed csrmv of
  * src/AMG_gpu_phases_2.cu:125,186 / src/AMG_gpu_phases.cu:512 with a deterministic gather */
 int sparsh_matrix_create_transpose(int nrow, int ncol, int nnz, const int *h_rowptr, const int *h_colindex,
@@ -225,6 +235,16 @@ void sparsh_params_default(sparsh_params *p);
  * factor the coarsest level (Direct_Solver_Pardiso ctor, src/AMG_coarse_level_solver.cpp:9-62, done on the device). */
 int sparsh_hierarchy_create(int nlevels, const sparsh_level_desc *levels, const sparsh_params *params,
                             sparsh_hierarchy_t *out);
+/* New values for level 0 of a hierarchy, same sparsity (d_val[nnz] on the device in the stored order: for a
+ * multicolour-SOR hierarchy the colour-permuted order, as at create; d_diag[nrow] may be NULL).  P_l and R_l are kept.
+ * For every level, A_{l+1} = P_l^T A_l P_l is recomputed on the device, bit for bit what the host setup computes for the
+ * same P.  Coarse diagonals are extracted; each level is then updated as by sparsh_matrix_update_values.  The coarsest
+ * inverse is refactored and cached CUDA graphs are dropped.
+ * The first call builds and keeps a plan: SPARSH_ERR_INVALID, with nothing written, when a stored A_{l+1} does not have
+ * exactly the structure of P_l^T A_l P_l or a product row is longer than the device kernels' lists.  When the coarsest
+ * matrix turns out singular or a CUDA error occurs after writing began, that error is returned and the hierarchy is
+ * stale: V-cycles, solves and coarse solves return SPARSH_ERR_INVALID until a later refresh succeeds. */
+int sparsh_hierarchy_refresh(sparsh_hierarchy_t h, const double *d_val, const double *d_diag);
 int sparsh_hierarchy_destroy(sparsh_hierarchy_t h); /* AMG_GPU1_solver::~AMG_GPU1_solver, src/AMG_gpu_phases_2.cu:265-338 */
 int sparsh_hierarchy_nlevels(sparsh_hierarchy_t h);
 /* borrow the device matrices of one level (for per-op parity tests); P and R are NULL on the coarsest level */

@@ -56,6 +56,8 @@ SIGNATURES = {
     "sparsh_fill": (_i, [_vp, _sz, _d]),
     "sparsh_matrix_create": (_i, [_i, _i, _i, c_int_p, c_int_p, c_dbl_p, c_dbl_p, _vpp]),
     "sparsh_matrix_create_transpose": (_i, [_i, _i, _i, c_int_p, c_int_p, c_dbl_p, _vpp]),
+    "sparsh_matrix_update_values": (_i, [_vp, _vp, _vp]),
+    "sparsh_matrix_fetch": (_i, [_vp, c_int_p, c_int_p, c_dbl_p, c_dbl_p]),
     "sparsh_matrix_destroy": (_i, [_vp]),
     "sparsh_matrix_dims": (_i, [_vp, c_int_p, c_int_p, c_int_p]),
     "sparsh_matrix_kernel": (_i, [_vp, c_int_p, c_int_p, c_int_p]),
@@ -91,6 +93,7 @@ SIGNATURES = {
     "sparsh_params_default": (None, [C.POINTER(Params)]),
     "sparsh_hierarchy_create": (_i, [_i, C.POINTER(LevelDesc), C.POINTER(Params), _vpp]),
     "sparsh_hierarchy_destroy": (_i, [_vp]),
+    "sparsh_hierarchy_refresh": (_i, [_vp, _vp, _vp]),
     "sparsh_hierarchy_nlevels": (_i, [_vp]),
     "sparsh_hierarchy_level": (_i, [_vp, _i, _vpp, _vpp, _vpp]),
     "sparsh_hierarchy_coarse_solve": (_i, [_vp, _vp, _vp]),

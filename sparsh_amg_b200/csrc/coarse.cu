@@ -155,6 +155,52 @@ __global__ void __launch_bounds__(256) dense_gemv_kernel(const double *__restric
     if (lane == 0) x[row] = s;
 }
 
+// Gauss-Jordan of the dense n x n matrix in M, M2 the second buffer of the double-buffered elimination: on success
+// *result is the buffer holding the inverse.  SPARSH_ERR_INVALID for a singular matrix.
+static int gauss_jordan(double *M, double *M2, int n, int *piv, double *d_min, double **result) {
+    Context &c = ctx();
+    // one CTA per SM, all co-resident (cooperative launch): the elimination steps are separated by grid barriers
+    int per_sm = 0;
+    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, gj_coop_kernel, GJ_T, 0);
+    int grid = c.sm_count * (per_sm > 0 ? 1 : 0);
+    if (grid > n) grid = n;
+    if (e == cudaSuccess && (grid < 1 || (n + grid - 1) / grid > GJ_MAX_ROWS)) {
+        set_error("coarse solver: the cooperative Gauss-Jordan kernel does not fit on this device");
+        return SPARSH_ERR_CUDA;
+    }
+    if (e == cudaSuccess) {
+        int nn = n;
+        void *kargs[] = {&M, &M2, &nn, &piv, &d_min};
+        e = cudaLaunchCooperativeKernel((const void *)gj_coop_kernel, dim3(grid), dim3(GJ_T), kargs, 0, c.stream);
+        count_launch();
+    }
+    double *R = (n & 1) ? M2 : M;  // buffer written by the last step
+    static bool attr = false;
+    if (e == cudaSuccess && !attr) {
+        e = cudaFuncSetAttribute(gj_unscramble_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 16384 * 8);
+        attr = true;
+    }
+    if (e == cudaSuccess) {
+        gj_unscramble_kernel<<<n, 256, sizeof(double) * (size_t)n, c.stream>>>(R, n, piv);
+        count_launch();
+        e = cudaGetLastError();
+    }
+    double h_min = 0.0;
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&h_min, d_min, sizeof(double), cudaMemcpyDeviceToHost, c.stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c.stream);
+    if (e != cudaSuccess) {
+        set_error(std::string("coarse solver: ") + cudaGetErrorString(e));
+        return SPARSH_ERR_CUDA;
+    }
+    // the reference aborts on a PARDISO error for a singular coarsest matrix (src/AMG_coarse_level_solver.cpp:52-60)
+    if (!(h_min > 0.0) || !std::isfinite(h_min)) {
+        set_error("coarsest-level matrix is singular (zero pivot in the dense factorisation): e.g. a pure-Neumann problem");
+        return SPARSH_ERR_INVALID;
+    }
+    *result = R;
+    return SPARSH_OK;
+}
+
 int coarse_build_inverse(int n, const int *rp, const int *ci, const double *v, CoarseInverse *out) {
     Context &c = ctx();
     NvtxRange nvtx("sparsh:coarse-inverse");
@@ -182,49 +228,46 @@ int coarse_build_inverse(int n, const int *rp, const int *ci, const double *v, C
         set_error(std::string("coarse solver: ") + cudaGetErrorString(cudaGetLastError()));
         return fail(SPARSH_ERR_CUDA);
     }
-    cudaError_t e = cudaMemcpyAsync(M, dense.data(), sizeof(double) * (size_t)n * n, cudaMemcpyHostToDevice, c.stream);
-    // one CTA per SM, all co-resident (cooperative launch): the elimination steps are separated by grid barriers
-    int per_sm = 0;
-    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, gj_coop_kernel, GJ_T, 0);
-    int grid = c.sm_count * (per_sm > 0 ? 1 : 0);
-    if (grid > n) grid = n;
-    if (e == cudaSuccess && (grid < 1 || (n + grid - 1) / grid > GJ_MAX_ROWS)) {
-        set_error("coarse solver: the cooperative Gauss-Jordan kernel does not fit on this device");
-        return fail(SPARSH_ERR_CUDA);
-    }
-    if (e == cudaSuccess) {
-        int nn = n;
-        void *kargs[] = {&M, &M2, &nn, &piv, &d_min};
-        e = cudaLaunchCooperativeKernel((const void *)gj_coop_kernel, dim3(grid), dim3(GJ_T), kargs, 0, c.stream);
-        count_launch();
-    }
-    double *R = (n & 1) ? M2 : M;  // buffer written by the last step
-    static bool attr = false;
-    if (e == cudaSuccess && !attr) {
-        e = cudaFuncSetAttribute(gj_unscramble_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 16384 * 8);
-        attr = true;
-    }
-    if (e == cudaSuccess) {
-        gj_unscramble_kernel<<<n, 256, sizeof(double) * (size_t)n, c.stream>>>(R, n, piv);
-        count_launch();
-        e = cudaGetLastError();
-    }
-    double h_min = 0.0;
-    if (e == cudaSuccess) e = cudaMemcpyAsync(&h_min, d_min, sizeof(double), cudaMemcpyDeviceToHost, c.stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(c.stream);
+    const cudaError_t e = cudaMemcpyAsync(M, dense.data(), sizeof(double) * (size_t)n * n, cudaMemcpyHostToDevice, c.stream);
     if (e != cudaSuccess) {
         set_error(std::string("coarse solver: ") + cudaGetErrorString(e));
         return fail(SPARSH_ERR_CUDA);
     }
-    // the reference aborts on a PARDISO error for a singular coarsest matrix (src/AMG_coarse_level_solver.cpp:52-60)
-    if (!(h_min > 0.0) || !std::isfinite(h_min)) {
-        set_error("coarsest-level matrix is singular (zero pivot in the dense factorisation): e.g. a pure-Neumann problem");
-        return fail(SPARSH_ERR_INVALID);
-    }
+    double *R = nullptr;
+    const int rc = gauss_jordan(M, M2, n, piv, d_min, &R);
+    if (rc != SPARSH_OK) return fail(rc);
     cudaFree(R == M ? M2 : M);
     cudaFree(d_min);
     cudaFree(piv);
     out->inv = R;
+    return SPARSH_OK;
+}
+
+// dense row i = the stored entries of row i added in stored order onto zeros (coarse_build_inverse's += on the host)
+__global__ void __launch_bounds__(256)
+    csr_to_dense_kernel(int n, const int *__restrict__ rp, const int *__restrict__ ci, const double *__restrict__ v, double *M) {
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= n) return;
+    double *row = M + (size_t)i * n;
+    for (int j = rp[i]; j < rp[i + 1]; j++) row[ci[j]] = __dadd_rn(row[ci[j]], v[j]);
+}
+
+int coarse_refactor(CoarseInverse *ci, const sparsh_matrix_s *A, double **spare, int *piv, double *d_min) {
+    NvtxRange nvtx("sparsh:coarse-refactor");
+    const int n = ci->n;
+    if (n == 0) return SPARSH_OK;
+    cudaStream_t st = ctx().stream;
+    double *M = ci->inv;
+    SP_CUDA(cudaMemsetAsync(M, 0, sizeof(double) * (size_t)n * n, st));
+    csr_to_dense_kernel<<<(n + 255) / 256, 256, 0, st>>>(n, A->rowptr, A->col, A->val, M);
+    count_launch();
+    SP_CUDA(cudaGetLastError());
+    double *R = nullptr;
+    SP_TRY(gauss_jordan(M, *spare, n, piv, d_min, &R));
+    if (R != M) {
+        *spare = M;
+        ci->inv = R;
+    }
     return SPARSH_OK;
 }
 

@@ -283,6 +283,7 @@ int sparsh_hierarchy_destroy(sparsh_hierarchy_t h) {
         dev_free(L.rbuf);
     }
     coarse_free(&h->coarse);
+    refresh_plan_free(h->refresh);
     for (int i = 0; i < 8; i++) cudaFree(h->kv[i]);
     cudaFree(h->d_sc);
     cudaFreeHost(h->h_sc);
@@ -308,11 +309,13 @@ int sparsh_hierarchy_level(sparsh_hierarchy_t h, int level, sparsh_matrix_t *A, 
 
 int sparsh_hierarchy_coarse_solve(sparsh_hierarchy_t h, const double *d_b, double *d_x) {
     SP_REQUIRE(h != nullptr, "hierarchy is NULL");
+    SP_TRY(require_fresh(h));
     return coarse_apply(h->coarse, d_b, d_x);
 }
 
 int sparsh_hierarchy_vcycle(sparsh_hierarchy_t h, const double *d_b, double *d_x, int cycles, int x_is_zero) {
     SP_REQUIRE(h != nullptr && cycles >= 0, "bad arguments");
+    SP_TRY(require_fresh(h));
     for (int k = 0; k < cycles; k++) {
         const bool zero = x_is_zero && k == 0;
         SP_TRY(run_graphed(h, d_b, d_x, zero ? 1 : 0, [&]() { return enqueue_vcycle(h, d_b, d_x, zero); }));
@@ -323,6 +326,7 @@ int sparsh_hierarchy_vcycle(sparsh_hierarchy_t h, const double *d_b, double *d_x
 int sparsh_hierarchy_amg_solve(sparsh_hierarchy_t h, const double *d_b, double *d_x, double tol, int max_cycles,
                                double *h_hist, int *cycles_out) {
     SP_REQUIRE(h != nullptr, "hierarchy is NULL");
+    SP_TRY(require_fresh(h));
     sparsh_matrix_s *A = h->lev[0].A;
     double r1 = 0.0;
     NvtxRange nvtx("sparsh:amg-solve");

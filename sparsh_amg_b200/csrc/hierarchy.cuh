@@ -20,6 +20,9 @@ struct Level {
     std::vector<int> color_count;  // multicolour smoother: prefix offsets per colour (host copy)
 };
 
+struct RefreshPlan;  // refresh.cu: per-level products and workspace of sparsh_hierarchy_refresh
+void refresh_plan_free(RefreshPlan *p);
+
 struct GraphEntry {
     const void *k0 = nullptr, *k1 = nullptr;
     int tag = 0;
@@ -43,10 +46,14 @@ struct sparsh_hierarchy_s {
     double *gm_V = nullptr, *gm_d = nullptr, *gm_h = nullptr;
     int gm_m = 0;
     std::vector<sparsh::GraphEntry> graphs;
+    sparsh::RefreshPlan *refresh = nullptr;  // built by the first sparsh_hierarchy_refresh
+    bool stale = false;  // a refresh failed after writing: solves return SPARSH_ERR_INVALID until one succeeds
 };
 
 namespace sparsh {
 
+// SPARSH_ERR_INVALID (with the error message) when a failed refresh left h's coefficients inconsistent
+int require_fresh(const sparsh_hierarchy_s *h);
 // enqueue one V-cycle on the current stream (no host sync)
 int enqueue_vcycle(sparsh_hierarchy_s *h, const double *b, double *x, bool x_is_zero);
 // run `body` directly, or (params.use_graph) as a cached CUDA graph keyed by (k0,k1,tag)

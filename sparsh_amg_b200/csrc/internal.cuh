@@ -155,6 +155,9 @@ struct sparsh_matrix_s {
     double mean_row = 0.0;
     int win128 = 0, win256 = 0;  // max nnz over any window of 128 / 256 consecutive rows
     int smem_bytes = 0;          // dynamic shared memory of the stream kernel
+    // choose_kernel's result before any twin or sparsh_matrix_force_kernel changed it: sparsh_matrix_update_values
+    // starts its selection from here (the row statistics depend on the sparsity only)
+    int base_kind = sparsh::KIND_VECTOR, base_threads = 256, base_lanes = 8, base_smem_bytes = 0;
     // csr-dict16 twin (present when the dictionaries fit; see DictView)
     unsigned short *code = nullptr;
     double *dict_val = nullptr;
@@ -167,6 +170,7 @@ struct sparsh_matrix_s {
     int *pat_start = nullptr;
     double *pat_diag = nullptr;
     int n_pat = 0, n_pent = 0, n_escape = 0, pat_far = 0;
+    int pat_cap_ent = 0, pat_cap_pat = 0;  // entries / patterns the allocated table arrays hold (reused by value updates)
     bool has_pat = false;
     sparsh::Pat0 pat0;  // len == 0: the lean (speculative-gather) variant does not apply
     // grid-transfer structure, read from the host arrays at upload (HEM: P has both, R = P^T uniform values only)
@@ -315,12 +319,26 @@ void dev_free(void *p);
 void *thread_scratch(size_t bytes);
 void release_thread_scratch();
 
+// ---- Galerkin products with a kept prolongator (rap.cu, refresh.cu) ----------------------------------------------------
+constexpr int RAP_MAX_ROW = 192;  // distinct columns per product row handled by the device kernels' per-thread lists
+// C = A B, structure only: *crp (allocated, arow + 1) and *nnz; *fits = false when a row of C has more than RAP_MAX_ROW
+// entries (nothing allocated then).  Synchronises st.
+int spgemm_structure(int arow, const int *arp, const int *aci, const int *brp, const int *bci, int **crp, int *nnz,
+                     bool *fits, cudaStream_t st);
+// C = A B into a structure from spgemm_structure: first-touch order, unfused multiply / add (the host product's bits)
+int spgemm_values(int arow, const int *arp, const int *aci, const double *av, const int *brp, const int *bci,
+                  const double *bv, const int *crp, int *cci, double *cv, cudaStream_t st);
+
 // ---- dense coarse solve (coarse.cu) ----------------------------------------------------------------------
 struct CoarseInverse {
     int n = 0;
     double *inv = nullptr;  // n x n row-major
 };
 int coarse_build_inverse(int n, const int *h_rowptr, const int *h_col, const double *h_val, CoarseInverse *out);
+// the inverse of the device CSR A (n x n, n == ci->n) in place of ci->inv: dense scatter in stored order, then the same
+// Gauss-Jordan as coarse_build_inverse.  spare (n x n), piv (n) and d_min (1) are caller workspace; the buffer that does
+// not end up holding the inverse is handed back through *spare.  SPARSH_ERR_INVALID when A is singular.
+int coarse_refactor(CoarseInverse *ci, const sparsh_matrix_s *A, double **spare, int *piv, double *d_min);
 int coarse_apply(const CoarseInverse &ci, const double *b, double *x);
 void coarse_free(CoarseInverse *ci);
 

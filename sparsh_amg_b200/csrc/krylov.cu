@@ -313,18 +313,21 @@ extern "C" {
 int sparsh_hierarchy_pcg(sparsh_hierarchy_t h, const double *d_b, double *d_x, double tol, int max_iter, double *h_hist,
                          int *iters) {
     SP_REQUIRE(h != nullptr, "hierarchy is NULL");
+    SP_TRY(require_fresh(h));
     return cg_impl(h, true, d_b, d_x, tol, max_iter, h_hist, iters);
 }
 
 int sparsh_hierarchy_pbicgstab(sparsh_hierarchy_t h, const double *d_b, double *d_x, double tol, int max_iter,
                                double *h_hist, int *iters) {
     SP_REQUIRE(h != nullptr, "hierarchy is NULL");
+    SP_TRY(require_fresh(h));
     return bicg_impl(h, true, d_b, d_x, tol, max_iter, h_hist, iters);
 }
 
 int sparsh_hierarchy_pgmres(sparsh_hierarchy_t h, const double *d_b, double *d_x, double tol, int restart,
                             int max_iter, double *h_hist, int *iters) {
     SP_REQUIRE(h != nullptr, "hierarchy is NULL");
+    SP_TRY(require_fresh(h));
     return gmres_impl(h, true, d_b, d_x, tol, restart, max_iter, h_hist, iters);
 }
 

@@ -47,6 +47,10 @@ void choose_kernel(sparsh_matrix_s *A, const int *rp) {
     } else {
         A->kind = KIND_VECTOR;
     }
+    A->base_kind = A->kind;
+    A->base_threads = A->threads;
+    A->base_lanes = A->lanes;
+    A->base_smem_bytes = A->smem_bytes;
 }
 
 // Aggregation operators (HEM: P has one 1.0 per row, R = P^T rows of one or two 1.0) are recognised from the host
@@ -311,9 +315,10 @@ bool build_dict(sparsh_matrix_s *A, const int *rp, const int *ci, const double *
     if (!dict_encode(n, rp, ci, v, code.data(), dv, dof)) return false;
     const size_t pad = ((nnz + 7) & ~(size_t)7) + 16;  // bulk copies round the slice outwards to multiples of 8 codes
     cudaStream_t st = up().stream;
-    if (dev_alloc(&A->code, sizeof(unsigned short) * pad) != cudaSuccess) return false;
-    dev_alloc(&A->dict_val, sizeof(double) * 256);
-    dev_alloc(&A->dict_off, sizeof(int) * 256);
+    // a value update reuses the arrays of an earlier twin: their sizes depend on nnz only
+    if (!A->code && dev_alloc(&A->code, sizeof(unsigned short) * pad) != cudaSuccess) return false;
+    if (!A->dict_val) dev_alloc(&A->dict_val, sizeof(double) * 256);
+    if (!A->dict_off) dev_alloc(&A->dict_off, sizeof(int) * 256);
     cudaMemsetAsync(A->code, 0, sizeof(unsigned short) * pad, st);
     cudaMemcpyAsync(A->code, code.data(), sizeof(unsigned short) * nnz, cudaMemcpyHostToDevice, st);
     cudaMemcpyAsync(A->dict_val, dv.data(), sizeof(double) * dv.size(), cudaMemcpyHostToDevice, st);
@@ -561,9 +566,29 @@ int pattern_mode() {
     return env ? atoi(env) : 1;
 }
 
-// encodes (on the device, see above) and keeps the twin; false (nothing kept) when the rows do not repeat enough.  rp,
-// ci, v are the HOST arrays (the table is built from the representatives' rows), the device copies are A->rowptr/col/val.
-bool build_pattern(sparsh_matrix_s *A, const int *rp, const int *ci, const double *v, const double *h_diag) {
+// lengths (dst == nullptr) or entries (col - row, value) of the rows reps[0..k): the representative rows a pattern table
+// is built from when the matrix' host arrays are gone (sparsh_matrix_update_values)
+__global__ void __launch_bounds__(256)
+    pat_gather_kernel(int k, const int *__restrict__ reps, const int *__restrict__ rp, const int *__restrict__ ci,
+                      const double *__restrict__ v, const int *__restrict__ dst, int *len, int *off, double *val) {
+    const int t = blockIdx.x * 256 + threadIdx.x;
+    if (t >= k) return;
+    const int r = reps[t], lo = rp[r], l = rp[r + 1] - lo;
+    if (!dst) {
+        len[t] = l;
+        return;
+    }
+    for (int q = 0; q < l; q++) {
+        off[dst[t] + q] = ci[lo + q] - r;
+        val[dst[t] + q] = v[lo + q];
+    }
+}
+
+// encodes (on the device, see above) and keeps the twin; false (nothing kept) when the rows do not repeat enough.  The
+// table is built from the representatives' rows: read from the HOST arrays rp, ci, v when given (the upload), else
+// gathered from the device copies A->rowptr/col/val (a value update).  check_diag: A->diag is the caller's smoothing
+// diagonal, and rows where it differs from the tabulated one become escapes.
+bool build_pattern(sparsh_matrix_s *A, const int *rp, const int *ci, const double *v, bool check_diag) {
     const int n = A->nrow;
     if (n == 0 || A->nnz == 0) return false;
     cudaStream_t st = up().stream;
@@ -578,13 +603,18 @@ bool build_pattern(sparsh_matrix_s *A, const int *rp, const int *ci, const doubl
             A->pat_ent = nullptr;
             A->pat_start = nullptr;
             A->pat_diag = nullptr;
+            A->pat_cap_ent = A->pat_cap_pat = 0;
         }
         cudaGetLastError();
     };
-    // temporaries: [table | id_of | slot_of | counts | overflow], each 256-byte aligned, in one scratch block
+    // temporaries: [table | id_of | slot_of | counts | overflow | gather: reps, lengths, destinations, offsets, values],
+    // each 256-byte aligned, in one scratch block
     auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
     const size_t o_table = 0, o_id = o_table + al(sizeof(PatSlot) * PAT_SLOTS), o_slot = o_id + al(sizeof(int) * PAT_SLOTS),
-                 o_counts = o_slot + al(sizeof(int) * (size_t)n), o_over = o_counts + 256, scratch_bytes = o_over + 256;
+                 o_counts = o_slot + al(sizeof(int) * (size_t)n), o_over = o_counts + 256, o_reps = o_over + 256,
+                 o_len = o_reps + al(sizeof(int) * PAT_MAX_CAND), o_dst = o_len + al(sizeof(int) * PAT_MAX_CAND),
+                 o_goff = o_dst + al(sizeof(int) * PAT_ESCAPE), o_gval = o_goff + al(sizeof(int) * PAT_MAX_ENT),
+                 scratch_bytes = o_gval + al(sizeof(double) * PAT_MAX_ENT);
     char *scratch = static_cast<char *>(thread_scratch(scratch_bytes));
     if (!scratch) return false;
     PatSlot *d_table = reinterpret_cast<PatSlot *>(scratch + o_table);
@@ -604,7 +634,8 @@ bool build_pattern(sparsh_matrix_s *A, const int *rp, const int *ci, const doubl
         cleanup();
         return false;
     }
-    if (cudaMemcpy(table.data(), d_table, sizeof(PatSlot) * PAT_SLOTS, cudaMemcpyDeviceToHost) != cudaSuccess) {
+    if (cudaMemcpyAsync(table.data(), d_table, sizeof(PatSlot) * PAT_SLOTS, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+        cudaStreamSynchronize(st) != cudaSuccess) {
         cleanup();
         return false;
     }
@@ -620,31 +651,71 @@ bool build_pattern(sparsh_matrix_s *A, const int *rp, const int *ci, const doubl
         return false;
     }
     std::sort(cand.begin(), cand.end(), [](const Cand &a, const Cand &b) { return a.count != b.count ? a.count > b.count : a.rep < b.rep; });
+    // row lengths of the candidates, then the ones that enter the table (a row that would overflow it is skipped)
+    const int n_cand = (int)cand.size();
+    std::vector<int> len((size_t)n_cand), reps((size_t)n_cand);
+    for (int k = 0; k < n_cand; k++) reps[k] = cand[k].rep;
+    int *d_reps = reinterpret_cast<int *>(scratch + o_reps), *d_len = reinterpret_cast<int *>(scratch + o_len);
+    if (rp) {
+        for (int k = 0; k < n_cand; k++) len[k] = rp[reps[k] + 1] - rp[reps[k]];
+    } else {
+        cudaMemcpyAsync(d_reps, reps.data(), sizeof(int) * (size_t)n_cand, cudaMemcpyHostToDevice, st);
+        pat_gather_kernel<<<(n_cand + 255) / 256, 256, 0, st>>>(n_cand, d_reps, A->rowptr, A->col, A->val, nullptr, d_len, nullptr, nullptr);
+        cudaMemcpyAsync(len.data(), d_len, sizeof(int) * (size_t)n_cand, cudaMemcpyDeviceToHost, st);
+        if (cudaStreamSynchronize(st) != cudaSuccess) {
+            cleanup();
+            return false;
+        }
+    }
     PatternTable T;
     T.start.push_back(0);
-    std::vector<int> id_of(PAT_SLOTS, -1);
-    for (const Cand &c : cand) {
-        const int r = c.rep, len = rp[r + 1] - rp[r];
-        if ((int)T.diag.size() == PAT_ESCAPE) break;
-        if ((int)T.val.size() + len > PAT_MAX_ENT) continue;
-        id_of[c.slot] = (int)T.diag.size();
+    std::vector<int> id_of(PAT_SLOTS, -1), sel;
+    for (int k = 0; k < n_cand; k++) {
+        if ((int)T.start.size() - 1 == PAT_ESCAPE) break;
+        if (T.start.back() + len[k] > PAT_MAX_ENT) continue;
+        id_of[cand[k].slot] = (int)T.start.size() - 1;
+        sel.push_back(k);
+        T.start.push_back(T.start.back() + len[k]);
+    }
+    const int n_pat = (int)sel.size(), n_ent = T.start.back();
+    if (n_pat == 0) {
+        cleanup();
+        return false;
+    }
+    std::vector<int> g_off;
+    std::vector<double> g_val;
+    if (!rp) {  // the selected rows' entries, in table order
+        std::vector<int> sreps((size_t)n_pat);
+        for (int p = 0; p < n_pat; p++) sreps[p] = reps[sel[p]];
+        g_off.resize((size_t)std::max(n_ent, 1));
+        g_val.resize((size_t)std::max(n_ent, 1));
+        int *d_dst = reinterpret_cast<int *>(scratch + o_dst), *d_goff = reinterpret_cast<int *>(scratch + o_goff);
+        double *d_gval = reinterpret_cast<double *>(scratch + o_gval);
+        cudaMemcpyAsync(d_reps, sreps.data(), sizeof(int) * (size_t)n_pat, cudaMemcpyHostToDevice, st);
+        cudaMemcpyAsync(d_dst, T.start.data(), sizeof(int) * (size_t)n_pat, cudaMemcpyHostToDevice, st);
+        pat_gather_kernel<<<(n_pat + 255) / 256, 256, 0, st>>>(n_pat, d_reps, A->rowptr, A->col, A->val, d_dst, nullptr, d_goff, d_gval);
+        cudaMemcpyAsync(g_off.data(), d_goff, sizeof(int) * (size_t)n_ent, cudaMemcpyDeviceToHost, st);
+        cudaMemcpyAsync(g_val.data(), d_gval, sizeof(double) * (size_t)n_ent, cudaMemcpyDeviceToHost, st);
+        if (cudaStreamSynchronize(st) != cudaSuccess) {
+            cleanup();
+            return false;
+        }
+    }
+    for (int p = 0; p < n_pat; p++) {
+        const int r = reps[sel[p]];
         double d = 0.0;
         bool found = false;
-        for (int k = rp[r]; k < rp[r + 1]; k++) {
-            T.val.push_back(v[k]);
-            T.off.push_back(ci[k] - r);
-            if (!found && ci[k] == r) {
-                d = v[k];
+        for (int q = 0; q < len[sel[p]]; q++) {
+            const int off = rp ? ci[rp[r] + q] - r : g_off[T.start[p] + q];
+            const double x = rp ? v[rp[r] + q] : g_val[T.start[p] + q];
+            T.val.push_back(x);
+            T.off.push_back(off);
+            if (!found && off == 0) {
+                d = x;
                 found = true;
             }
         }
         T.diag.push_back(d);
-        T.start.push_back((int)T.val.size());
-    }
-    const int n_pat = (int)T.diag.size(), n_ent = (int)T.val.size();
-    if (n_pat == 0) {
-        cleanup();
-        return false;
     }
     std::vector<PatEntry> ent((size_t)n_ent + 8, PatEntry{0.0, 0, 0});
     for (int k = 0; k < n_ent; k++) ent[k] = PatEntry{T.val[k], T.off[k], 0};
@@ -663,9 +734,23 @@ bool build_pattern(sparsh_matrix_s *A, const int *rp, const int *ci, const doubl
         }
         pattern_masks(T, z.mask);
     }
-    ok = dev_alloc(&A->pat, (size_t)n + 16) == cudaSuccess && dev_alloc(&A->pat_ent, sizeof(PatEntry) * ent.size()) == cudaSuccess &&
-         dev_alloc(&A->pat_start, sizeof(int) * ((size_t)n_pat + 1)) == cudaSuccess &&
-         dev_alloc(&A->pat_diag, sizeof(double) * (size_t)n_pat) == cudaSuccess;
+    // a value update reuses the arrays of an earlier twin when the new table fits them
+    if (!A->pat) ok = dev_alloc(&A->pat, (size_t)n + 16) == cudaSuccess;
+    if (ok && A->pat_cap_ent < (int)ent.size()) {
+        dev_free(A->pat_ent);
+        A->pat_ent = nullptr;
+        ok = dev_alloc(&A->pat_ent, sizeof(PatEntry) * ent.size()) == cudaSuccess;
+        A->pat_cap_ent = ok ? (int)ent.size() : 0;
+    }
+    if (ok && A->pat_cap_pat < n_pat) {
+        dev_free(A->pat_start);
+        dev_free(A->pat_diag);
+        A->pat_start = nullptr;
+        A->pat_diag = nullptr;
+        ok = dev_alloc(&A->pat_start, sizeof(int) * ((size_t)n_pat + 1)) == cudaSuccess &&
+             dev_alloc(&A->pat_diag, sizeof(double) * (size_t)n_pat) == cudaSuccess;
+        A->pat_cap_pat = ok ? n_pat : 0;
+    }
     unsigned long long counts[3] = {0ull, 0ull, 0ull};
     if (ok) {
         cudaMemsetAsync(A->pat, PAT_ESCAPE, (size_t)n + 16, st);
@@ -673,9 +758,9 @@ bool build_pattern(sparsh_matrix_s *A, const int *rp, const int *ci, const doubl
         cudaMemcpyAsync(A->pat_start, T.start.data(), sizeof(int) * ((size_t)n_pat + 1), cudaMemcpyHostToDevice, st);
         cudaMemcpyAsync(A->pat_diag, T.diag.data(), sizeof(double) * (size_t)n_pat, cudaMemcpyHostToDevice, st);
         cudaMemcpyAsync(d_id_of, id_of.data(), sizeof(int) * PAT_SLOTS, cudaMemcpyHostToDevice, st);
-        // rows whose smoothing diagonal (A->diag, uploaded from h_diag) differs from the tabulated one become escapes
-        pat_assign_kernel<<<grid, 256, 0, st>>>(n, A->rowptr, A->col, A->val, h_diag ? A->diag : nullptr, d_slot_of, d_id_of, A->pat_ent,
-                                                A->pat_start, A->pat_diag, z, A->pat, d_counts);
+        // rows whose smoothing diagonal (A->diag, the caller's) differs from the tabulated one become escapes
+        pat_assign_kernel<<<grid, 256, 0, st>>>(n, A->rowptr, A->col, A->val, check_diag ? A->diag : nullptr, d_slot_of, d_id_of,
+                                                A->pat_ent, A->pat_start, A->pat_diag, z, A->pat, d_counts);
         cudaMemcpyAsync(counts, d_counts, sizeof counts, cudaMemcpyDeviceToHost, st);
         ok = cudaStreamSynchronize(st) == cudaSuccess;
     }
@@ -697,6 +782,117 @@ bool build_pattern(sparsh_matrix_s *A, const int *rp, const int *ci, const doubl
     kept = true;
     cleanup();
     return true;
+}
+
+// ---- value updates on the device (sparsh_matrix_update_values) ----------------------------------------------------
+// differs[0] = 1 when some stored value's bits differ from v[0]'s (transfer_structure's scan)
+__global__ void __launch_bounds__(256) uniform_bits_kernel(size_t nnz, const double *__restrict__ v, int *differs) {
+    const long long u0 = __double_as_longlong(v[0]);
+    for (size_t k = (size_t)blockIdx.x * 256 + threadIdx.x; k < nnz; k += (size_t)gridDim.x * 256)
+        if (__double_as_longlong(v[k]) != u0) {
+            *differs = 1;
+            return;
+        }
+}
+
+// sp_matrix_fill_diagonal: the first stored entry with col == row, else 0
+__global__ void __launch_bounds__(256)
+    diag_extract_kernel(int n, const int *__restrict__ rp, const int *__restrict__ ci, const double *__restrict__ v, double *d) {
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= n) return;
+    double x = 0.0;
+    for (int j = rp[i]; j < rp[i + 1]; j++)
+        if (ci[j] == i) {
+            x = v[j];
+            break;
+        }
+    d[i] = x;
+}
+
+// Can the csr-dict16 twin exist?  Distinct value bit patterns and distinct (col - row) offsets are registered in two
+// small open-addressing sets; count[0] / count[1] receive their sizes, over[0] = 1 as soon as either passes 256 (every
+// thread then stops).  An empty slot holds ~0; a value with exactly those bits is recorded in count[2] instead.
+constexpr int DICT_SLOTS = 1024;
+constexpr unsigned long long DICT_EMPTY = ~0ull;
+__device__ __forceinline__ void dict_insert(unsigned long long *set, unsigned long long key, int *count, int *over) {
+    unsigned int s = (unsigned int)((key * 0x9E3779B97F4A7C15ull) >> 54);
+    for (int probe = 0; probe < DICT_SLOTS; probe++, s = (s + 1) & (DICT_SLOTS - 1)) {
+        unsigned long long seen = *reinterpret_cast<volatile unsigned long long *>(set + s);
+        if (seen == DICT_EMPTY) seen = atomicCAS(set + s, DICT_EMPTY, key);
+        if (seen == DICT_EMPTY) {
+            if (atomicAdd(count, 1) >= 256) atomicExch(over, 1);
+            return;
+        }
+        if (seen == key) return;
+    }
+    atomicExch(over, 1);
+}
+__global__ void __launch_bounds__(256)
+    dict_fits_kernel(int n, const int *__restrict__ rp, const int *__restrict__ ci, const double *__restrict__ v,
+                     unsigned long long *vset, unsigned long long *oset, int *count, int *over) {
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= n || *reinterpret_cast<volatile int *>(over)) return;
+    for (int j = rp[i]; j < rp[i + 1]; j++) {
+        const unsigned long long bits = (unsigned long long)__double_as_longlong(v[j]);
+        if (bits == DICT_EMPTY)
+            atomicExch(count + 2, 1);
+        else
+            dict_insert(vset, bits, count, over);
+        dict_insert(oset, (unsigned long long)(unsigned int)(ci[j] - i), count + 1, over);
+    }
+}
+
+// build_dict from the device arrays: the host encoder runs only when the device found the twin possible
+bool build_dict_device(sparsh_matrix_s *A) {
+    const int n = A->nrow, nnz = A->nnz;
+    if (nnz == 0) return false;
+    cudaStream_t st = up().stream;
+    char *scratch = static_cast<char *>(thread_scratch(2 * sizeof(unsigned long long) * DICT_SLOTS + 256));
+    if (!scratch) return false;
+    unsigned long long *vset = reinterpret_cast<unsigned long long *>(scratch), *oset = vset + DICT_SLOTS;
+    int *d_count = reinterpret_cast<int *>(oset + DICT_SLOTS), *d_over = d_count + 3;
+    int h[4] = {0, 0, 0, 0};
+    cudaMemsetAsync(vset, 0xff, 2 * sizeof(unsigned long long) * DICT_SLOTS, st);
+    cudaMemsetAsync(d_count, 0, sizeof(int) * 4, st);
+    dict_fits_kernel<<<(n + 255) / 256, 256, 0, st>>>(n, A->rowptr, A->col, A->val, vset, oset, d_count, d_over);
+    cudaMemcpyAsync(h, d_count, sizeof h, cudaMemcpyDeviceToHost, st);
+    if (cudaStreamSynchronize(st) != cudaSuccess) {
+        cudaGetLastError();
+        return false;
+    }
+    if (h[3] || h[0] + h[2] > 256 || h[1] > 256) return false;
+    std::vector<int> rp((size_t)n + 1), ci((size_t)nnz);
+    std::vector<double> v((size_t)nnz);
+    if (staged_d2h(rp.data(), A->rowptr, sizeof(int) * ((size_t)n + 1), st) != SPARSH_OK ||
+        staged_d2h(ci.data(), A->col, sizeof(int) * (size_t)nnz, st) != SPARSH_OK ||
+        staged_d2h(v.data(), A->val, sizeof(double) * (size_t)nnz, st) != SPARSH_OK) {
+        cudaGetLastError();
+        return false;
+    }
+    return build_dict(A, rp.data(), ci.data(), v.data());
+}
+
+// The compressed twins and the kernel family, from A's kind as choose_kernel left it.  rp, ci, v: the host arrays of
+// the upload, or nullptr to work from the device arrays (a value update).  check_diag: A->diag is the caller's.
+void choose_twins(sparsh_matrix_s *A, const int *rp, const int *ci, const double *v, bool check_diag) {
+    // Matrices that would run the stream kernel get a lossless compressed twin when they are stencil-like.
+    // csr-pattern8 first (1 B per row, encoded on the device): when the rows repeat it wins, and the csr-dict16 twin
+    // (2 B per entry, encoded by the host: 0.5 s per 10^8 entries) is not even built unless SPARSH_DICT=2 asks for both.
+    const int pmode = pattern_mode();
+    const char *denv = getenv("SPARSH_DICT");
+    const int dmode = denv ? atoi(denv) : 1;  // 0: never, 1: when csr-pattern8 is not selected, 2: always (tests, A/B runs)
+    // (rectangular operators qualify too: the multi-GPU local blocks are nrow x (owned + halo) with a diagonal)
+    bool pattern_selected = false;
+    if (pmode > 0 && A->kind == KIND_STREAM && build_pattern(A, rp, ci, v, check_diag)) pattern_selected = pmode == 1;
+    if (A->kind == KIND_STREAM && dmode > 0 && (!pattern_selected || dmode == 2) &&
+        (rp ? build_dict(A, rp, ci, v) : build_dict_device(A))) {
+        A->kind = KIND_DICT;
+        A->threads = 128;  // measured on B200 (256^3 Jacobi): 128-thread CTAs x 4 rows per thread 0.180 ms, 256 x 4 0.199 ms
+    }
+    if (pattern_selected) {
+        A->kind = KIND_PATTERN;
+        A->threads = 128;
+    }
 }
 
 int validate(int nrow, int ncol, int nnz, const int *rp, const int *ci) {
@@ -764,26 +960,85 @@ int sparsh_matrix_create(int nrow, int ncol, int nnz, const int *h_rowptr, const
         return rc;
     }
     lap("CSR copied");
-    // Matrices that would run the stream kernel get a lossless compressed twin when they are stencil-like.
-    // csr-pattern8 first (1 B per row, encoded on the device): when the rows repeat it wins, and the csr-dict16 twin
-    // (2 B per entry, encoded by the host: 0.5 s per 10^8 entries) is not even built unless SPARSH_DICT=2 asks for both.
-    const int pmode = pattern_mode();
-    const char *denv = getenv("SPARSH_DICT");
-    const int dmode = denv ? atoi(denv) : 1;  // 0: never, 1: when csr-pattern8 is not selected, 2: always (tests, A/B runs)
-    // (rectangular operators qualify too: the multi-GPU local blocks are nrow x (owned + halo) with a diagonal)
-    bool pattern_selected = false;
-    if (pmode > 0 && A->kind == KIND_STREAM && build_pattern(A, h_rowptr, h_colindex, h_val, h_diag)) pattern_selected = pmode == 1;
-    if (A->kind == KIND_STREAM && dmode > 0 && (!pattern_selected || dmode == 2) && build_dict(A, h_rowptr, h_colindex, h_val)) {
-        A->kind = KIND_DICT;
-        A->threads = 128;  // measured on B200 (256^3 Jacobi): 128-thread CTAs x 4 rows per thread 0.180 ms, 256 x 4 0.199 ms
-    }
-    if (pattern_selected) {
-        A->kind = KIND_PATTERN;
-        A->threads = 128;
-    }
+    choose_twins(A, h_rowptr, h_colindex, h_val, h_diag != nullptr);
     lap("twins built");
     if (!slab_bound()) release_thread_scratch();  // a hierarchy build keeps the encoder's scratch until its thread ends
     *out = A;
+    return SPARSH_OK;
+}
+
+int sparsh_matrix_update_values(sparsh_matrix_t A, const double *d_val, const double *d_diag) {
+    SP_TRY(ensure_init());
+    SP_REQUIRE(A != nullptr, "matrix is NULL");
+    SP_REQUIRE(d_val != nullptr || A->nnz == 0, "values are NULL");
+    NvtxRange nvtx("sparsh:update-values");
+    cudaStream_t st = up().stream;
+    const int n = A->nrow;
+    const size_t nnz = (size_t)A->nnz;
+    if (nnz > 0 && d_val != A->val) SP_CUDA(cudaMemcpyAsync(A->val, d_val, sizeof(double) * nnz, cudaMemcpyDeviceToDevice, st));
+    // the selection starts again from the row statistics; a forced kernel is forgotten
+    A->kind = A->base_kind;
+    A->threads = A->base_threads;
+    A->lanes = A->base_lanes;
+    A->smem_bytes = A->base_smem_bytes;
+    A->threads_forced = false;
+    // transfer_structure's value scan (one entry per row depends on the sparsity only and is kept)
+    if (nnz > 0) {
+        struct {
+            int differs;
+            int pad;
+            double v0;
+        } h = {0, 0, 0.0};
+        int *d_flag = static_cast<int *>(thread_scratch(256));
+        SP_REQUIRE(d_flag != nullptr, "value update: no device scratch");
+        SP_CUDA(cudaMemsetAsync(d_flag, 0, sizeof(int), st));
+        const int grid = (int)std::min<size_t>((nnz + 255) / 256, (size_t)ctx().sm_count * 8);
+        uniform_bits_kernel<<<grid, 256, 0, st>>>(nnz, A->val, d_flag);
+        count_launch();
+        SP_CUDA(cudaMemcpyAsync(&h.differs, d_flag, sizeof(int), cudaMemcpyDeviceToHost, st));
+        SP_CUDA(cudaMemcpyAsync(&h.v0, A->val, sizeof(double), cudaMemcpyDeviceToHost, st));
+        SP_CUDA(cudaStreamSynchronize(st));
+        A->uniform_val = h.differs == 0;
+        A->uval = h.v0;
+    } else {
+        A->uniform_val = false;
+        A->uval = 0.0;
+    }
+    A->agg = A->one_per_row && A->kind == KIND_SCALAR;
+    // the smoothing diagonal: the caller's, or extracted as sparsh_matrix_create extracts it
+    if (d_diag || n == A->ncol) {
+        if (!A->diag) SP_CUDA(dev_alloc(&A->diag, sizeof(double) * ((size_t)n + 1)));
+        if (d_diag && d_diag != A->diag && n > 0)
+            SP_CUDA(cudaMemcpyAsync(A->diag, d_diag, sizeof(double) * (size_t)n, cudaMemcpyDeviceToDevice, st));
+        if (!d_diag && n > 0) {
+            diag_extract_kernel<<<(n + 255) / 256, 256, 0, st>>>(n, A->rowptr, A->col, A->val, A->diag);
+            count_launch();
+            SP_CUDA(cudaGetLastError());
+        }
+    } else {
+        dev_free(A->diag);  // a rectangular matrix has a diagonal only when one is given
+        A->diag = nullptr;
+    }
+    A->has_pat = A->has_dict = false;
+    A->n_pat = A->n_pent = A->n_escape = A->pat_far = 0;
+    A->n_dval = A->n_doff = 0;
+    A->pat0 = Pat0();
+    // the encoders' device scratch stays with this thread (grow-only): later updates of the same sizes allocate nothing
+    choose_twins(A, nullptr, nullptr, nullptr, d_diag != nullptr);
+    SP_CUDA(cudaStreamSynchronize(st));
+    SP_CUDA(cudaGetLastError());
+    return SPARSH_OK;
+}
+
+int sparsh_matrix_fetch(sparsh_matrix_t A, int *h_rowptr, int *h_colindex, double *h_val, double *h_diag) {
+    SP_REQUIRE(A != nullptr, "matrix is NULL");
+    SP_REQUIRE(!h_diag || A->diag, "matrix has no diagonal");
+    cudaStream_t st = ctx().stream;
+    SP_CUDA(cudaStreamSynchronize(st));
+    if (h_rowptr) SP_TRY(staged_d2h(h_rowptr, A->rowptr, sizeof(int) * ((size_t)A->nrow + 1), st));
+    if (h_colindex && A->nnz > 0) SP_TRY(staged_d2h(h_colindex, A->col, sizeof(int) * (size_t)A->nnz, st));
+    if (h_val && A->nnz > 0) SP_TRY(staged_d2h(h_val, A->val, sizeof(double) * (size_t)A->nnz, st));
+    if (h_diag && A->nrow > 0) SP_TRY(staged_d2h(h_diag, A->diag, sizeof(double) * (size_t)A->nrow, st));
     return SPARSH_OK;
 }
 

@@ -27,7 +27,6 @@ namespace sparsh {
 
 namespace {
 
-constexpr int RAP_MAX_ROW = 192;  // distinct columns per product row handled by the per-thread list
 constexpr int SCAN_T = 1024, SCAN_ITEMS = 4;
 
 struct DevCsr {
@@ -370,6 +369,38 @@ void upload_jobs(const DevCsr &M, const int *rp, const int *ci, const double *v,
 }
 
 }  // namespace
+
+int spgemm_structure(int arow, const int *arp, const int *aci, const int *brp, const int *bci, int **crp, int *nnz,
+                     bool *fits, cudaStream_t st) {
+    *crp = nullptr;
+    *nnz = 0;
+    *fits = true;
+    Scratch<int> count, flag;
+    SP_CUDA(count.alloc((size_t)arow));
+    SP_CUDA(flag.alloc(1));
+    SP_CUDA(cudaMemsetAsync(flag.p, 0, sizeof(int), st));
+    if (arow > 0) spgemm_count_kernel<<<(arow + 127) / 128, 128, 0, st>>>(arow, arp, aci, brp, bci, count.p, flag.p);
+    int h_flag = 0;
+    SP_CUDA(cudaMemcpyAsync(&h_flag, flag.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+    SP_CUDA(cudaStreamSynchronize(st));
+    if (h_flag) {
+        *fits = false;
+        return SPARSH_OK;
+    }
+    SP_CUDA(cudaMalloc(crp, sizeof(int) * ((size_t)arow + 1)));
+    SP_TRY(exclusive_scan(count.p, arow, *crp, st));
+    SP_CUDA(cudaMemcpyAsync(nnz, *crp + arow, sizeof(int), cudaMemcpyDeviceToHost, st));
+    SP_CUDA(cudaStreamSynchronize(st));
+    return SPARSH_OK;
+}
+
+int spgemm_values(int arow, const int *arp, const int *aci, const double *av, const int *brp, const int *bci,
+                  const double *bv, const int *crp, int *cci, double *cv, cudaStream_t st) {
+    if (arow > 0) spgemm_fill_kernel<<<(arow + 127) / 128, 128, 0, st>>>(arow, arp, aci, av, brp, bci, bv, crp, cci, cv);
+    count_launch();
+    SP_CUDA(cudaGetLastError());
+    return SPARSH_OK;
+}
 
 }  // namespace sparsh
 

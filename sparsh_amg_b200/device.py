@@ -140,6 +140,26 @@ class DeviceMatrix:
         check(self.lib.sparsh_matrix_force_kernel(self.h, kind, threads_or_lanes))
         return self
 
+    def update_values(self, val, diag=None):
+        """new values (nnz, stored order) for the same sparsity; diag None: extracted.  numpy arrays or DeviceVectors.
+        Twins, kernel family and transfer flags are chosen again as at upload (a forced kernel is forgotten)."""
+        v, d = _on_device(val, self.nnz), _on_device(diag, self.nrow)
+        check(self.lib.sparsh_matrix_update_values(self.h, v.ptr, d.ptr if d is not None else None))
+        return self
+
+    def fetch(self):
+        """(rowptr, colindex, val, diag) copied back from the device; diag is None for a matrix without one"""
+        rp = np.zeros(self.nrow + 1, dtype=np.int32)
+        ci = np.zeros(max(self.nnz, 1), dtype=np.int32)
+        v = np.zeros(max(self.nnz, 1))
+        d = np.zeros(max(self.nrow, 1))
+        try:
+            check(self.lib.sparsh_matrix_fetch(self.h, ip(rp), ip(ci), dp(v), dp(d)))
+        except capi.SparshError:  # no diagonal (rectangular operator)
+            d = None
+            check(self.lib.sparsh_matrix_fetch(self.h, ip(rp), ip(ci), dp(v), None))
+        return rp, ci[: self.nnz], v[: self.nnz], (d[: self.nrow] if d is not None else None)
+
     # ---- per-op (device vectors in, device vectors out) ----
     def spmv(self, x, y=None):
         y = y or DeviceVector(self.nrow)
@@ -213,6 +233,16 @@ class DeviceMatrix:
             self.free()
         except Exception:
             pass
+
+
+def _on_device(a, n):
+    """a DeviceVector as given, a numpy array uploaded (None stays None)"""
+    if a is None or isinstance(a, DeviceVector):
+        assert a is None or a.n == n, (a.n, n)
+        return a
+    a = np.ascontiguousarray(a, dtype=np.float64)
+    assert a.size == n, (a.size, n)
+    return DeviceVector(data=a)
 
 
 def galerkin_rap(A, P):
@@ -322,6 +352,14 @@ class DeviceHierarchy:
         check(self.lib.sparsh_hierarchy_level(self.h, k, C.byref(a), C.byref(p), C.byref(r)))
         wrap = lambda hd: DeviceMatrix(handle=hd, owned=False) if hd else None  # noqa: E731
         return wrap(a.value), wrap(p.value), wrap(r.value)
+
+    def refresh(self, val, diag=None):
+        """new level-0 values (nnz, stored order; numpy array or DeviceVector) for the same sparsity: every coarse operator
+        is recomputed on the device with the kept prolongators, twins and the coarse inverse are rebuilt"""
+        A0 = self.level(0)[0]
+        v, d = _on_device(val, A0.nnz), _on_device(diag, A0.nrow)
+        check(self.lib.sparsh_hierarchy_refresh(self.h, v.ptr, d.ptr if d is not None else None))
+        return self
 
     def coarse_solve(self, b, x=None):
         x = x or DeviceVector(b.n)
