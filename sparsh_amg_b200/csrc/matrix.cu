@@ -363,16 +363,18 @@ inline uint64_t row_pattern_hash(const int *rp, const int *ci, const double *v, 
     return h;
 }
 
+// distinct rows beyond which a matrix is declared not stencil-like, by both encoders
+constexpr int PAT_MAX_CAND = 1 << 15;
+
 // Host-only encoder.  pat[i] receives the pattern id of row i (PAT_ESCAPE for rows left to the CSR arrays).  Patterns
 // are numbered by decreasing row count (ties: first occurrence).  h_diag, when given, is the diagonal the caller will
 // smooth with: rows where it differs from the tabulated one become escapes.  Returns false when the matrix is not
-// stencil-like (too many distinct rows, or fewer than min_cover of the rows tabulated).
+// stencil-like (more than PAT_MAX_CAND distinct rows, or fewer than min_cover of the rows tabulated).
 bool pattern_encode(int n, const int *rp, const int *ci, const double *v, const double *h_diag, unsigned char *pat,
                     PatternTable &T, double min_cover) {
     struct Cand {
         int rep, count;
     };
-    constexpr size_t MAX_CAND = 1u << 16;
     std::vector<Cand> cand;
     std::unordered_map<uint64_t, int> by_hash;
     std::vector<int> cand_of((size_t)n, -1);
@@ -389,7 +391,7 @@ bool pattern_encode(int n, const int *rp, const int *ci, const double *v, const 
             const uint64_t h = row_pattern_hash(rp, ci, v, i);
             auto it = by_hash.find(h);
             if (it == by_hash.end()) {
-                if (cand.size() >= MAX_CAND) return false;  // not stencil-like: stop before the map grows with n
+                if (cand.size() >= (size_t)PAT_MAX_CAND) return false;  // not stencil-like: stop before the map grows with n
                 c = (int)cand.size();
                 cand.push_back(Cand{i, 0});
                 by_hash.emplace(h, c);
@@ -470,9 +472,9 @@ void pattern_masks(const PatternTable &T, unsigned char mask[256]) {
 // host), count —; (2) the host reads the few candidates back, orders them exactly like the host encoder (count
 // descending, first occurrence ascending) and builds the table from the representatives' rows; (3) a second kernel
 // gives every row its pattern id after comparing it ENTRY BY ENTRY with the tabulated pattern (a hash collision or a
-// differing smoothing diagonal makes the row an escape).  The result equals the host encoder's.
-constexpr int PAT_SLOTS = 1 << 17;   // open addressing
-constexpr int PAT_MAX_CAND = 1 << 15;  // distinct rows beyond which the matrix is declared not stencil-like
+// differing smoothing diagonal makes the row an escape).  The result equals the host encoder's, including the decision:
+// both give up past PAT_MAX_CAND distinct rows.
+constexpr int PAT_SLOTS = 1 << 17;  // open addressing: load factor <= 1/4 at PAT_MAX_CAND keys
 struct PatSlot {
     unsigned long long key;  // 0 = empty
     int rep, count;
@@ -773,10 +775,10 @@ bool build_pattern(sparsh_matrix_s *A, const int *rp, const int *ci, const doubl
     A->n_escape = n - (int)counts[0];
     A->pat_far = 0;
     for (int k = 0; k < n_ent; k++) A->pat_far = std::max(A->pat_far, T.off[k]);
-    if (z.len > 0) {
-        z.cover = (double)counts[1] / (double)n;
-        z.cover_masked = (double)counts[2] / (double)n;
-    }
+    // the shares are statistics of the table (sparsh_matrix_pattern_stats), also when pattern 0 is too long to travel
+    // by value (z.len == 0: the lean kernel does not apply whatever they are)
+    z.cover = (double)counts[1] / (double)n;
+    z.cover_masked = (double)counts[2] / (double)n;
     A->pat0 = z;
     A->has_pat = true;
     kept = true;
