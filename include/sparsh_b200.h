@@ -47,6 +47,8 @@ int sparsh_device_name(char *buf, size_t len, int *sm_count);
 /* number of kernels this library has launched since the last reset (graph replays count their kernel nodes) */
 long long sparsh_launch_count(void);
 void sparsh_launch_count_reset(void);
+/* adds kernels run that the library could not count without a host read: the loop of an enqueued solve (d_status[2]) */
+void sparsh_launch_count_add(long long kernels);
 
 /* ------------------------------------------------------------------ memory ----- */
 /* replace cudaMalloc / cudaMemcpy / thrust::fill of src/AMG_gpu_phases_2.cu:17-29,127,245-246,259 */
@@ -239,7 +241,12 @@ int sparsh_hierarchy_create(int nlevels, const sparsh_level_desc *levels, const 
  * multicolour-SOR hierarchy the colour-permuted order, as at create; d_diag[nrow] may be NULL).  P_l and R_l are kept.
  * For every level, A_{l+1} = P_l^T A_l P_l is recomputed on the device, bit for bit what the host setup computes for the
  * same P.  Coarse diagonals are extracted; each level is then updated as by sparsh_matrix_update_values.  The coarsest
- * inverse is refactored and cached CUDA graphs are dropped.
+ * inverse is refactored (in place: it keeps its device address) and the library's cached CUDA graphs are dropped.
+ * A CUDA graph of the CALLER's that holds an enqueued solve (sparsh_hierarchy_*_enqueue) or a V-cycle must be captured
+ * again after a refresh, successful or not: kernel choices, by-value launch arguments and twin arrays change, and a
+ * replay of the old graph computes with stale ones (wrong results, no error code).  A captured
+ * sparsh_hierarchy_coarse_solve stays valid.  After a refresh each enqueued method needs one call outside a capture
+ * again before it may be captured.
  * The first call builds and keeps a plan: SPARSH_ERR_INVALID, with nothing written, when a stored A_{l+1} does not have
  * exactly the structure of P_l^T A_l P_l or a product row is longer than the device kernels' lists.  When the coarsest
  * matrix turns out singular or a CUDA error occurs after writing began, that error is returned and the hierarchy is
@@ -292,6 +299,34 @@ int sparsh_hierarchy_solve_host(sparsh_hierarchy_t h, int method, const double *
                                 int max_iter, double *h_hist, int *iters);
 /* bytes moved by one V-cycle according to the algorithmic model of SURVEY §8d (for roofline reports) */
 double sparsh_hierarchy_vcycle_bytes(sparsh_hierarchy_t h, int x_is_zero);
+
+/* ---------------------------------------------------- device-driven hierarchy solvers -- */
+/* Device-driven twins of sparsh_hierarchy_pcg / _pbicgstab / _amg_solve: the same kernels in the same order, so x and
+ * the residual history are bit-identical to theirs.  The iteration loop and its stopping test run on the device (a
+ * conditional WHILE node of a CUDA graph).  The call only enqueues work on the library's current stream: it never
+ * synchronises, allocates or copies to the host once the hierarchy has run the same method once.  If that stream is
+ * being captured by the caller, the solve is recorded into the caller's graph.
+ * Results are in DEVICE memory: d_hist[max_iter+1] (may be NULL) as h_hist of the synchronous call;
+ * d_status[0] = iterations (cycles), d_status[1] = SPARSH_OK or SPARSH_ERR_NOT_CONVERGED, d_status[2] = kernels the
+ * loop ran (d_status has 3 slots).
+ * The return code covers what the host can see: bad arguments, a stale hierarchy, CUDA errors, and SPARSH_ERR_INVALID
+ * for a call under stream capture before the method has run once on this hierarchy outside a capture (that first call
+ * allocates workspace and builds the solve graph, which a capture forbids).  One instantiated graph is cached per
+ * (method, d_b, d_x) address pair and kept until sparsh_hierarchy_refresh or _destroy: a caller that solves every step
+ * reuses its b and x buffers (new addresses each step would build and keep a graph per call).
+ * A graph of the caller's into which a solve was captured is valid until the next sparsh_hierarchy_refresh of h,
+ * successful or not: after it, capture the solve again (see sparsh_hierarchy_refresh), and run the method once outside
+ * a capture first.  b, x, the workspace and the device scalars are read when the work runs, not when it is enqueued:
+ * do not start another solve on the same hierarchy on a different stream before this one has finished.
+ * sparsh_launch_count: the kernels outside the loop count when the call enqueues them (under a caller's capture: once,
+ * when captured); the loop's kernels, unknown to the host, count when the caller adds d_status[2] with
+ * sparsh_launch_count_add (PendingSolve.result() in the Python package does). */
+int sparsh_hierarchy_pcg_enqueue(sparsh_hierarchy_t h, const double *d_b, double *d_x, double tol, int max_iter,
+                                 double *d_hist, int *d_status);
+int sparsh_hierarchy_pbicgstab_enqueue(sparsh_hierarchy_t h, const double *d_b, double *d_x, double tol, int max_iter,
+                                       double *d_hist, int *d_status);
+int sparsh_hierarchy_amg_solve_enqueue(sparsh_hierarchy_t h, const double *d_b, double *d_x, double tol, int max_cycles,
+                                       double *d_hist, int *d_status);
 
 /* ------------------------------------------------------------------ multi-GPU -- */
 /* One process per GPU, NCCL over NVLink 5 / NVSwitch (the reference has no distributed path at all: SURVEY §2.1 last

@@ -11,5 +11,5 @@ There is no CPU fallback: importing is cheap, but every compute call needs lib/l
 """
 from . import capi  # noqa: F401
 from .capi import SparshError  # noqa: F401
-from .device import (DeviceHierarchy, DeviceMatrix, DeviceVector, axpby, axpbypcz, axpy, dot, galerkin_rap,  # noqa: F401
-                     init, launch_count, nrm2, set_stream, sync)
+from .device import (DeviceHierarchy, DeviceMatrix, DeviceVector, PendingSolve, axpby, axpbypcz, axpy, dot,  # noqa: F401
+                     galerkin_rap, init, launch_count, nrm2, set_stream, sync)

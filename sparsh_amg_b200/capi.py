@@ -46,6 +46,7 @@ SIGNATURES = {
     "sparsh_device_name": (_i, [C.c_char_p, _sz, c_int_p]),
     "sparsh_launch_count": (C.c_longlong, []),
     "sparsh_launch_count_reset": (None, []),
+    "sparsh_launch_count_add": (None, [C.c_longlong]),
     "sparsh_malloc": (_i, [_sz, _vpp]),
     "sparsh_free": (_i, [_vp]),
     "sparsh_host_alloc": (_i, [_sz, _vpp]),
@@ -107,6 +108,9 @@ SIGNATURES = {
     "sparsh_gmres": (_i, [_vp, _vp, _vp, _d, _i, _i, c_dbl_p, c_int_p]),
     "sparsh_hierarchy_solve_host": (_i, [_vp, _i, _vp, _vp, _d, _i, c_dbl_p, c_int_p]),
     "sparsh_hierarchy_vcycle_bytes": (_d, [_vp, _i]),
+    "sparsh_hierarchy_pcg_enqueue": (_i, [_vp, _vp, _vp, _d, _i, _vp, _vp]),
+    "sparsh_hierarchy_pbicgstab_enqueue": (_i, [_vp, _vp, _vp, _d, _i, _vp, _vp]),
+    "sparsh_hierarchy_amg_solve_enqueue": (_i, [_vp, _vp, _vp, _d, _i, _vp, _vp]),
     # multi-GPU
     "sparsh_dist_get_unique_id": (_i, [C.c_char_p]),
     "sparsh_dist_init": (_i, [C.c_char_p, _i, _i]),

@@ -252,7 +252,7 @@ __global__ void __launch_bounds__(256)
     for (int j = rp[i]; j < rp[i + 1]; j++) row[ci[j]] = __dadd_rn(row[ci[j]], v[j]);
 }
 
-int coarse_refactor(CoarseInverse *ci, const sparsh_matrix_s *A, double **spare, int *piv, double *d_min) {
+int coarse_refactor(CoarseInverse *ci, const sparsh_matrix_s *A, double *spare, int *piv, double *d_min) {
     NvtxRange nvtx("sparsh:coarse-refactor");
     const int n = ci->n;
     if (n == 0) return SPARSH_OK;
@@ -263,11 +263,10 @@ int coarse_refactor(CoarseInverse *ci, const sparsh_matrix_s *A, double **spare,
     count_launch();
     SP_CUDA(cudaGetLastError());
     double *R = nullptr;
-    SP_TRY(gauss_jordan(M, *spare, n, piv, d_min, &R));
-    if (R != M) {
-        *spare = M;
-        ci->inv = R;
-    }
+    SP_TRY(gauss_jordan(M, spare, n, piv, d_min, &R));
+    // the inverse stays at its address (odd n ends the elimination in the spare buffer: copied back, n^2 doubles), so a
+    // coarse solve captured into a caller's graph before the refresh reads the new inverse
+    if (R != M) SP_CUDA(cudaMemcpyAsync(M, R, sizeof(double) * (size_t)n * n, cudaMemcpyDeviceToDevice, st));
     return SPARSH_OK;
 }
 

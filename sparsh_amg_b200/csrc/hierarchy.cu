@@ -273,6 +273,10 @@ int sparsh_hierarchy_destroy(sparsh_hierarchy_t h) {
     if (ctx().ready) cudaStreamSynchronize(ctx().stream);
     for (auto &g : h->graphs)
         if (g.exec) cudaGraphExecDestroy(g.exec);
+    drop_solve_graphs(h);
+    for (cudaStream_t s : h->solve_stream)
+        if (s) cudaStreamDestroy(s);
+    cudaFree(h->d_ctl);
     for (auto &L : h->lev) {
         sparsh_matrix_destroy(L.A);
         sparsh_matrix_destroy(L.P);
@@ -333,15 +337,14 @@ int sparsh_hierarchy_amg_solve(sparsh_hierarchy_t h, const double *d_b, double *
     SP_TRY(sparsh_residual_norm(A, d_b, d_x, &r1));  // reference src/AMG_phases.cpp:159
     if (h_hist) h_hist[0] = r1;
     int cycles = 0;
-    while (r1 > tol && cycles < max_cycles) {         // :196 (the reference has no cap: SURVEY F6)
+    while (solve_continues(cycles, max_cycles, r1, tol)) {  // :196 (the reference has no cap: SURVEY F6)
         SP_TRY(sparsh_hierarchy_vcycle(h, d_b, d_x, 1, 0));
         cycles++;
         SP_TRY(sparsh_residual_norm(A, d_b, d_x, &r1));  // :219
         if (h_hist) h_hist[cycles] = r1;
-        if (!std::isfinite(r1)) break;
     }
     if (cycles_out) *cycles_out = cycles;
-    return (r1 <= tol) ? SPARSH_OK : SPARSH_ERR_NOT_CONVERGED;
+    return solve_status(r1, tol);
 }
 
 double sparsh_hierarchy_vcycle_bytes(sparsh_hierarchy_t h, int x_is_zero) {

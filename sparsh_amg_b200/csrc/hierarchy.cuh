@@ -30,6 +30,26 @@ struct GraphEntry {
     long long kernels = 0;
 };
 
+// device-driven solves (sparsh_hierarchy_*_enqueue, krylov.cu)
+enum SolveMethod { SOLVE_PCG = 0, SOLVE_PBICGSTAB = 1, SOLVE_AMG = 2 };
+// the loop state of an enqueued solve, in device memory: written by the argument kernel of each call, read and
+// advanced by the loop's control kernels
+struct SolveCtl {
+    double tol;
+    int cap;    // iteration limit (PCG: min(n, max_iter))
+    int count;  // iterations done
+    double res;  // last residual norm
+    double *hist;
+    int *status;
+};
+// one instantiated solve graph (setup, WHILE loop, epilogue) per (method, b, x)
+struct SolveGraph {
+    int method = 0;
+    const void *b = nullptr, *x = nullptr;
+    cudaGraphExec_t exec = nullptr;
+    long long kernels = 0;  // kernels outside the loop (the loop's own are counted by PendingSolve.result())
+};
+
 }  // namespace sparsh
 
 struct sparsh_hierarchy_s {
@@ -46,6 +66,12 @@ struct sparsh_hierarchy_s {
     double *gm_V = nullptr, *gm_d = nullptr, *gm_h = nullptr;
     int gm_m = 0;
     std::vector<sparsh::GraphEntry> graphs;
+    // device-driven solves: loop state, two internal streams (the solve graph's and its loop body's capture), the
+    // cached solve graphs, and which methods have run once outside a caller's stream capture
+    sparsh::SolveCtl *d_ctl = nullptr;
+    cudaStream_t solve_stream[2] = {nullptr, nullptr};
+    std::vector<sparsh::SolveGraph> solves;
+    bool solve_warm[3] = {false, false, false};
     sparsh::RefreshPlan *refresh = nullptr;  // built by the first sparsh_hierarchy_refresh
     bool stale = false;  // a refresh failed after writing: solves return SPARSH_ERR_INVALID until one succeeds
 };
@@ -60,6 +86,8 @@ int enqueue_vcycle(sparsh_hierarchy_s *h, const double *b, double *x, bool x_is_
 template <class F>
 int run_graphed(sparsh_hierarchy_s *h, const void *k0, const void *k1, int tag, F body);
 int krylov_workspace(sparsh_hierarchy_s *h, int nvec);
+// destroys the cached solve graphs of sparsh_hierarchy_*_enqueue and clears solve_warm (refresh, destroy)
+void drop_solve_graphs(sparsh_hierarchy_s *h);
 
 template <class F>
 int run_graphed(sparsh_hierarchy_s *h, const void *k0, const void *k1, int tag, F body) {

@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <cmath>
 #include <string>
 
 #include <nvtx3/nvToolsExt.h>  // header-only (dlopen's the tools library when a profiler is attached; a no-op otherwise)
@@ -68,6 +69,17 @@ inline void count_launch() {
     else
         c.launches++;
 }
+
+// ---- stopping rule of the solve loops: the host loops and the device loops' control kernels both evaluate these, so
+// the two cannot drift.  Double sqrt is correctly rounded on host and device (the library is built without fast-math),
+// so both sides see the same bits.
+__host__ __device__ inline double solve_residual(double sq) { return sqrt(sq); }
+// go on after `count` iterations with residual norm r?  No while count reaches cap or r <= tol; also no after an
+// iteration that produced a non-finite r (the initial residual only meets `r > tol`: NaN stops, +inf iterates)
+__host__ __device__ inline bool solve_continues(int count, int cap, double r, double tol) {
+    return (count == 0 || isfinite(r)) && count < cap && r > tol;
+}
+__host__ __device__ inline int solve_status(double r, double tol) { return r <= tol ? SPARSH_OK : SPARSH_ERR_NOT_CONVERGED; }
 
 constexpr int RED_MAX_BLOCKS = 1 << 20;  // partial sums per reduced value (2^28 rows at 256 rows per block)
 constexpr int RED_MAX_VALUES = 4;
@@ -336,9 +348,9 @@ struct CoarseInverse {
 };
 int coarse_build_inverse(int n, const int *h_rowptr, const int *h_col, const double *h_val, CoarseInverse *out);
 // the inverse of the device CSR A (n x n, n == ci->n) in place of ci->inv: dense scatter in stored order, then the same
-// Gauss-Jordan as coarse_build_inverse.  spare (n x n), piv (n) and d_min (1) are caller workspace; the buffer that does
-// not end up holding the inverse is handed back through *spare.  SPARSH_ERR_INVALID when A is singular.
-int coarse_refactor(CoarseInverse *ci, const sparsh_matrix_s *A, double **spare, int *piv, double *d_min);
+// Gauss-Jordan as coarse_build_inverse.  spare (n x n), piv (n) and d_min (1) are caller workspace; ci->inv keeps its
+// address.  SPARSH_ERR_INVALID when A is singular.
+int coarse_refactor(CoarseInverse *ci, const sparsh_matrix_s *A, double *spare, int *piv, double *d_min);
 int coarse_apply(const CoarseInverse &ci, const double *b, double *x);
 void coarse_free(CoarseInverse *ci);
 

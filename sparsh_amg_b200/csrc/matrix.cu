@@ -1285,7 +1285,7 @@ int sparsh_residual_norm(sparsh_matrix_t A, const double *d_b, const double *d_x
     SP_TRY(launch_csr(A, EPI_RESNORM, d_x, nullptr, a, 0, A->nrow));
     SP_CUDA(cudaMemcpyAsync(c.h_scalar, c.d_scalar, sizeof(double), cudaMemcpyDeviceToHost, c.stream));
     SP_CUDA(cudaStreamSynchronize(c.stream));
-    *h_norm = std::sqrt(c.h_scalar[0]);
+    *h_norm = solve_residual(c.h_scalar[0]);
     return SPARSH_OK;
 }
 

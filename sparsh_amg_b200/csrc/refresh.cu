@@ -316,6 +316,7 @@ int sparsh_hierarchy_refresh(sparsh_hierarchy_t h, const double *d_val, const do
     for (auto &g : h->graphs)
         if (g.exec) cudaGraphExecDestroy(g.exec);
     h->graphs.clear();
+    drop_solve_graphs(h);
     auto t0 = now();
     SP_TRY(sparsh_matrix_update_values(h->lev[0].A, d_val, d_diag));
     if (timing) std::fprintf(stderr, "[refresh] level 0: twins %.6f s\n", secs(t0, now()));
@@ -333,7 +334,7 @@ int sparsh_hierarchy_refresh(sparsh_hierarchy_t h, const double *d_val, const do
                          p->lev[l].agg ? "aggregation" : "general", secs(tb, now()));
     }
     const auto tc = now();
-    SP_TRY(coarse_refactor(&h->coarse, h->lev[L].A, &p->spare, p->piv, p->d_min));
+    SP_TRY(coarse_refactor(&h->coarse, h->lev[L].A, p->spare, p->piv, p->d_min));
     SP_CUDA(cudaStreamSynchronize(st));
     if (timing) std::fprintf(stderr, "[refresh] coarse inverse (n = %d): %.6f s\n", h->coarse.n, secs(tc, now()));
     h->stale = false;

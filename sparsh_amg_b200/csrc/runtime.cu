@@ -194,6 +194,7 @@ int sparsh_device_name(char *buf, size_t len, int *sm_count) {
 }
 long long sparsh_launch_count(void) { return ctx().launches; }
 void sparsh_launch_count_reset(void) { ctx().launches = 0; }
+void sparsh_launch_count_add(long long kernels) { ctx().launches += kernels; }
 
 int sparsh_malloc(size_t bytes, void **d_ptr) {
     SP_TRY(ensure_init());

@@ -245,6 +245,54 @@ def _on_device(a, n):
     return DeviceVector(data=a)
 
 
+def _current_stream():
+    s = C.c_void_p()
+    check(capi.load().sparsh_get_stream(C.byref(s)))
+    return s.value
+
+
+def _device_ptr(v, n):
+    """the device address of a DeviceVector or of a contiguous CUDA float64 tensor of n entries"""
+    if isinstance(v, DeviceVector):
+        assert v.n == n, (v.n, n)
+        return v.ptr
+    assert v.is_cuda and v.dtype.itemsize == 8 and v.dtype.is_floating_point and v.is_contiguous() and v.numel() == n
+    return v.data_ptr()
+
+
+class PendingSolve:
+    """A solve enqueued by DeviceHierarchy.pcg_enqueue / pbicgstab_enqueue / amg_solve_enqueue: its history and status
+    in device memory.  Nothing waits for the solve until result().  Pass it as `pending=` to a later enqueue to reuse
+    its buffers: no allocation, which a call under stream capture requires."""
+
+    def __init__(self, max_iter):
+        self.max_iter = int(max_iter)
+        self.hist = DeviceVector(self.max_iter + 1)
+        self.status = DeviceVector(2)  # 16 bytes: the 3 int32 of d_status
+        self.counted = True
+        self.stream = None  # the library stream the last solve was enqueued on
+
+    def result(self):
+        """Synchronises the stream the last solve was enqueued on, whichever stream is current now, and returns
+        (iterations, hist, converged) as pcg() etc. do.  The first call after an enqueue adds the loop's kernels to the
+        launch counter.  (A solve captured into a graph of the caller's: replay it and synchronise first.)"""
+        lib = capi.load()
+        current = _current_stream()
+        check(lib.sparsh_set_stream(self.stream))
+        try:
+            st = np.zeros(3, dtype=np.int32)
+            check(lib.sparsh_memcpy_d2h(st.ctypes.data, self.status.ptr, st.nbytes))  # synchronises that stream first
+            it, rc, kernels = int(st[0]), int(st[1]), int(st[2])
+            hist = np.zeros(it + 1)
+            check(lib.sparsh_memcpy_d2h(hist.ctypes.data, self.hist.ptr, hist.nbytes))
+        finally:
+            check(lib.sparsh_set_stream(current))
+        if not self.counted:
+            lib.sparsh_launch_count_add(kernels)
+            self.counted = True
+        return it, hist, rc == capi.SPARSH_OK
+
+
 def galerkin_rap(A, P):
     """A_c = P^T (A P) computed on the device (sparsh_galerkin_rap) -> (rowptr, colindex, val) numpy arrays, or None when
     the device kernel does not apply (a product row longer than its per-thread list)"""
@@ -382,6 +430,26 @@ class DeviceHierarchy:
     def pgmres(self, b, x, tol, restart=30, max_iter=500):
         """V-cycle-preconditioned GMRES(restart) (addition: SURVEY §8f.2)"""
         return _gmres(self.lib.sparsh_hierarchy_pgmres, self.h, b, x, tol, restart, max_iter)
+
+    # ---- device-driven solves: enqueue on the library's current stream, never wait (see PendingSolve) ----
+    def pcg_enqueue(self, b, x, tol, max_iter=500, pending=None):
+        return self._enqueue(self.lib.sparsh_hierarchy_pcg_enqueue, b, x, tol, max_iter, pending)
+
+    def pbicgstab_enqueue(self, b, x, tol, max_iter=500, pending=None):
+        return self._enqueue(self.lib.sparsh_hierarchy_pbicgstab_enqueue, b, x, tol, max_iter, pending)
+
+    def amg_solve_enqueue(self, b, x, tol, max_cycles=500, pending=None):
+        return self._enqueue(self.lib.sparsh_hierarchy_amg_solve_enqueue, b, x, tol, max_cycles, pending)
+
+    def _enqueue(self, fn, b, x, tol, max_iter, pending):
+        """b, x: DeviceVectors or CUDA tensors of n float64"""
+        p = pending if pending is not None else PendingSolve(max_iter)
+        assert p.max_iter >= max_iter, (p.max_iter, max_iter)
+        check(fn(self.h, _device_ptr(b, self.n), _device_ptr(x, self.n), float(tol), int(max_iter), p.hist.ptr,
+                 p.status.ptr))
+        p.stream = _current_stream()
+        p.counted = False
+        return p
 
     def solve_host(self, method, b_host, x_host, tol, max_iter=500):
         """method: 'amg' | 'pcg' | 'pbicgstab'; b_host/x_host are numpy arrays (x in/out)"""
